@@ -259,30 +259,24 @@ static int lev_prepare(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     return B200LEV_OK;
 }
 
-// Unit costs, short references, sequence-first tensors: the bit-vector path (lev_bitvec.cu)
-// takes the whole call -- lengths, warnings and DP -- straight from the raw tokens.
-// Returns 0 if it does not apply, 1 if it ran unconditionally (forced mode: the call is
-// Device-selected mode forks: once the uid pre-pass has finished the veto is final, so the
-// wavefront path's stand-by chain (seven launches that exit at once when the bit-vector
-// kernels took the call) runs on a side stream NEXT TO the bit-vector DP kernel instead of
-// behind it, and the caller's stream joins at the end.  In the vetoed case the DP kernel
-// exits at once and the chain does the work.  Nothing the chain touches before its kernels
-// have checked the veto overlaps what the DP kernel reads (lev_group.cu clears its tables in
-// a kernel that stands by too).  One side stream and two events per device, made once.
-// (the side stream and its events are shared by every caller on the device: calls that fork
-// are enqueued one at a time)
+// Device-selected mode forks: once the probe has finished the veto is final, so the wavefront
+// path's stand-by chain (seven launches that exit at once when the bit-vector kernel took the
+// call) runs on a side stream NEXT TO the bit-vector kernel instead of behind it, and the
+// caller's stream joins at the end.  In the vetoed case the bit-vector kernel exits at once and
+// the chain does the work.  Nothing the chain touches before its kernels have checked the veto
+// overlaps what the bit-vector kernel reads.  One side stream and two events per device, made
+// once.  (the side stream and its events are shared by every caller on the device: calls that
+// fork are enqueued one at a time)
 static std::mutex g_fork_mu;
 struct LevFork {
     cudaStream_t side;
-    void* after_uid;
+    void* after_probe;
     void* joined;
 };
 #ifndef B200LEV_EMU
 static bool lev_fork_get(LevFork* f) {
     static LevFork cache[64];
     static bool have[64];
-    if (const char* e = getenv("B200LEV_FORK"))
-        if (atoi(e) == 0) return false;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return false;
     if (!have[dev]) {
@@ -295,17 +289,17 @@ static bool lev_fork_get(LevFork* f) {
             return false;
         }
         cache[dev].side = s2;
-        cache[dev].after_uid = (void*)a;
+        cache[dev].after_probe = (void*)a;
         cache[dev].joined = (void*)b;
         have[dev] = true;
     }
     *f = cache[dev];
     return true;
 }
-// the chain goes to the side stream once the uid kernel is done; returns the stream to use
+// the chain goes to the side stream once the probe is done; returns the stream to use
 static cudaStream_t lev_fork_begin(const LevFork& f, bool on) {
     if (!on) return nullptr;
-    if (cudaStreamWaitEvent(f.side, (cudaEvent_t)f.after_uid, 0) != cudaSuccess) return nullptr;
+    if (cudaStreamWaitEvent(f.side, (cudaEvent_t)f.after_probe, 0) != cudaSuccess) return nullptr;
     return f.side;
 }
 static int lev_fork_join(const LevFork& f, cudaStream_t st) {
@@ -320,6 +314,9 @@ static cudaStream_t lev_fork_begin(const LevFork&, bool) { return nullptr; }
 static int lev_fork_join(const LevFork&, cudaStream_t) { return B200LEV_OK; }
 #endif
 
+// Unit costs, short references, sequence-first tensors: the bit-vector path (lev_bitvec.cu)
+// takes the whole call -- lengths, warnings and DP -- straight from the raw tokens.
+// Returns 0 if it does not apply, 1 if it ran unconditionally (forced mode: the call is
 // done), 2 if its kernels were enqueued in device-selected mode (the caller goes on to
 // enqueue the wavefront path with bv_check set; the state words are already cleared),
 // < 0 on error.
@@ -329,7 +326,7 @@ static int lev_try_bitvec(const b200lev_tokens_t* ref, const b200lev_tokens_t* h
                           int Hout, LevFork* fork, bool* forked, double* acc = nullptr,
                           bool* sums_done = nullptr) {
     *forked = false;
-    if (!L.off_bv_ref) return 0;
+    if (mode == LEV_MODE_MASK || L.R > 128) return 0;  // (lev_layout has no block counter for these)
     LevParams tmp;
     memset(&tmp, 0, sizeof(tmp));
     bool cm, fp;
@@ -352,13 +349,11 @@ static int lev_try_bitvec(const b200lev_tokens_t* ref, const b200lev_tokens_t* h
     }
     *forked = !forced && lev_fork_get(fork);
     const int rc = lev_bitvec_launch(ref, hyp, o, mode, tmp.mult, (int32_t*)(ws + L.off_ref_len),
-                                     (int32_t*)(ws + L.off_hyp_len), ws + L.off_bv_ref,
-                                     ws + L.off_hyp_tok, ws + L.off_slots, forced ? nullptr : state,
-                                     flags, out, out_si, Hout, st, *forked ? fork->after_uid : nullptr,
-                                     short_form, acc);
+                                     (int32_t*)(ws + L.off_hyp_len), (int*)(ws + L.off_bv_counter),
+                                     forced ? nullptr : state, flags, out, out_si, Hout, st,
+                                     *forked ? fork->after_probe : nullptr, short_form, acc);
     if (rc) return rc;
-    if (sums_done != nullptr)
-        *sums_done = short_form && mode == LEV_MODE_FINAL && acc != nullptr && !(getenv("B200LEV_BVS_SUMS") && atoi(getenv("B200LEV_BVS_SUMS")) == 0);
+    if (sums_done != nullptr) *sums_done = short_form && mode == LEV_MODE_FINAL && acc != nullptr;
     return forced ? 1 : 2;
 }
 

@@ -1,4 +1,4 @@
-// lev_bitvec.cu -- unit-cost fast path: bit-parallel Levenshtein, one LANE per pair.
+// lev_bitvec.cu -- unit-cost fast path: which bit-parallel kernel, if any, takes a call.
 //
 // When ins == del == sub (SM:168-174 reduces that case to unit costs and a multiplier) the
 // DP row of SM:286-350 is determined by its +1/0/-1 differences, and Myers' bit-vector
@@ -7,508 +7,24 @@
 // instructions per CELL in the packed wavefront kernel (lev_group.cu).  The value the
 // reference reads off each row -- column r, the distance between the full reference and a
 // hypothesis prefix (SM:352-358, 386-405) -- is the running score of the recurrence, so
-// the final and the prefix modes both fall out of one pass over the hypothesis.
-//
-// Two kernels, both with lane = pair and no transposition anywhere: a sequence-first token
-// tensor (T, N) is already "position-major, pair-minor", so lane l of a warp reading
-// tok[t][n0 + l] is one coalesced row, and the (H', N) output row of 32 neighbouring pairs is
-// one 128-byte store.  K0 (lev_pack.cu) is not needed on this path.
-//
-//   lev_bv_uid_kernel   per warp (32 consecutive pairs): one coalesced pass over the reference
-//       columns finds the RUNS of identical references (an n-best batch repeats every
-//       reference nbest times), their lengths (SM:137-143, 195-228) and the warnings.  The
-//       lanes of a run build ONE hash table for it together (buckets of 4 ways in shared
-//       memory, a way is claimed with a CAS on its key word, a build with an overflowing
-//       bucket is retried under another multiplier); then every lane looks its own
-//       hypothesis tokens up with one 128-bit read of the keys and one 32-bit read of the
-//       position bytes -- no probe loop.  Emits 1 uid byte per token (the table row of the
-//       token; 0xff: not in the reference), 16 per 128-bit store.  Reads the raw tokens once.
-//   lev_bv_dp_kernel    per run one table of match masks Peq[uid] in shared memory, per lane
-//       one Myers step per hypothesis token.  The reference is RIGHT-aligned in the 32*W-bit
-//       vector: the o = 32W - r low bits start with Pv = 0 and never match, which makes each
-//       of them a copy of the boundary row D[0][i] = i, so the boundary enters the first real
-//       bit through the ordinary shift and the score is always read at the top bit of the
-//       last word.
+// the final and the prefix modes both fall out of one pass over the hypothesis.  Both kernels
+// work with lane = pair straight from the raw sequence-first tokens; K0 (lev_pack.cu) is not
+// needed on this path.
 //
 // Eligibility (lev_bitvec_eligible): unit costs after SM:168-174, final or prefix mode, at most
-// 128 reference positions, unit stride along the batch axis of both token tensors and of
-// the prefix output.  The kernels are enqueued AHEAD of the wavefront path and decide on the
-// device (lev_bv_took, lev_common.cuh): a block of 32 pairs with more than 4 distinct
-// references, or a reference token the 32-bit keys cannot hold, vetoes, and the wavefront
-// kernels -- which otherwise exit at once -- do the work.
+// 128 reference positions, unit stride along the batch axis of both token tensors and of the
+// prefix output.  Then, per call:
+//
+//   Ks  lev_bv_short_kernel (lev_bvshort.cu), R <= 64: the reference in registers, no tables --
+//       any batch, taken unconditionally.
+//   Kb  lev_bv_fused_kernel (lev_bvfused.cu), R <= 128: per-run hash tables and match masks in
+//       shared memory, built for n-best batches (<= 4 distinct references per 32 pairs).  A call
+//       that declares its references shared (ref_group >= 8) takes it unconditionally; any other
+//       batch of at least B200LEV_BITVEC_MIN_PAIRS pairs is enqueued AHEAD of the wavefront path
+//       and decided on the device: lev_bv_probe_kernel vetoes through state[3] (lev_bv_took,
+//       lev_common.cuh) when a sampled block holds more references than that, and the wavefront
+//       kernels -- which otherwise exit at once -- do the work.
 #include "lev_bitvec.cuh"
-
-// ---------------------------------------------------------------------------------------
-// uid pre-pass
-// ---------------------------------------------------------------------------------------
-// One block of 32 consecutive pairs, one warp.  Returns false if the warp should stop (it
-// vetoed the path for the whole batch).
-template <typename TT>
-__device__ __forceinline__ bool lev_bv_uid_block(const LevBvArgs& a, int4* keys4, unsigned* posw,
-                                                 const int nb, const int64_t block, const int lane) {
-    constexpr int NT = LEV_BV_NT;
-    const int64_t pair = block * 32 + lane;
-    const bool valid = pair < a.P;
-    const int64_t pc = valid ? pair : (int64_t)a.P - 1;  // lanes past the batch shadow the last pair
-    const int64_t rcol = pc / a.ref_group;
-    const TT* __restrict__ rsrc = reinterpret_cast<const TT*>(a.ref) + rcol;
-    const TT* __restrict__ hsrc = reinterpret_cast<const TT*>(a.hyp) + pc;
-    const int rst = (int)a.ref_st, hst = (int)a.hyp_st;  // (lev_bitvec_eligible: strides fit int32)
-
-    // ---- one coalesced pass over my reference column: is it the same as my left neighbour's
-    // (runs), where is its first eos (SM:137-143, 198-218), does it hold a token the 32-bit
-    // keys cannot represent -----------------------------------------------------------------
-    for (int k = 0; k < 48 && k < a.H; ++k) lev_prefetch_l2(hsrc + (int64_t)k * hst);
-    // Both streaming passes work on 16 positions as two halves of 8 whose loads ping-pong:
-    // one half's 8 loads are in flight while the other half is processed.
-    int first_eos = a.R, exact0 = 0;
-    bool diff;
-    {
-        const int prev_col = __shfl_up_sync(LEV_FULL_MASK, (int)rcol, 1);
-        const bool other = prev_col != (int)rcol;
-        const int eos_lo = (int)a.eos, eos_hi = (int)(a.eos >> 32);
-        int dacc = 0, wacc = 0;  // differences to the left neighbour / to a sign extension
-        // (this pass needs no table yet, so its registers go into deeper batches: halves of 16)
-        constexpr int DH = 16;
-        auto observe = [&](const TT (&buf)[DH], int t0) {
-            unsigned eos_bits = 0, empty_bits = 0;
-#pragma unroll
-            for (int k = 0; k < DH; ++k) {
-                const int64_t x = (int64_t)buf[k];
-                const int lo = (int)x, hi = (int)(x >> 32);
-                dacc |= lo ^ __shfl_up_sync(LEV_FULL_MASK, lo, 1);
-                if (sizeof(TT) == 8) {
-                    dacc |= hi ^ __shfl_up_sync(LEV_FULL_MASK, hi, 1);
-                    wacc |= hi ^ (lo >> 31);
-                }
-                eos_bits |= (lo == eos_lo && hi == eos_hi) ? (1u << k) : 0u;
-                empty_bits |= lo == LEV_BV_EMPTY ? 1u : 0u;
-            }
-            // positions past R were loaded as 0 (= what the neighbour loaded): mask them out
-            const int live = a.R - t0;
-            if (live < DH) eos_bits &= live > 0 ? (1u << live) - 1u : 0u;
-            if (a.has_eos && eos_bits != 0 && first_eos == a.R) first_eos = t0 + __ffs((int)eos_bits) - 1;
-            if (empty_bits) exact0 = 1;
-        };
-        const TT* rp = rsrc;
-        TT bufA[DH], bufB[DH];
-#pragma unroll
-        for (int k = 0; k < DH; ++k) bufA[k] = (k < a.R) ? rp[(int64_t)k * rst] : (TT)0;
-#pragma unroll 1
-        for (int t0 = 0; t0 < a.R; t0 += 2 * DH) {
-            LEV_OPAQUE_PTR(rp);
-#pragma unroll
-            for (int k = 0; k < DH; ++k)
-                bufB[k] = (t0 + DH + k < a.R) ? rp[(int64_t)(DH + k) * rst] : (TT)0;
-            observe(bufA, t0);
-            if (a.check_state && t0 == 0) {
-                // unrelated references differ within their first tokens: such a batch is
-                // handed back to the wavefront path after one group of loads per warp
-                const unsigned same = __ballot_sync(LEV_FULL_MASK, lane > 0 && !(dacc != 0 && other));
-                if (32 - __popc(same) > LEV_BV_NT) {
-                    if (lane == 0) atomicExch(a.state + 3, 1);
-                    return false;
-                }
-            }
-            rp += 2 * DH * (int64_t)rst;
-            LEV_OPAQUE_PTR(rp);
-#pragma unroll
-            for (int k = 0; k < DH; ++k)
-                bufA[k] = (t0 + 2 * DH + k < a.R) ? rp[(int64_t)k * rst] : (TT)0;
-            observe(bufB, t0 + DH);
-        }
-        diff = dacc != 0 && other;
-        if (wacc != 0) exact0 = 1;
-    }
-    const LevBvRuns runs = lev_bv_runs(!diff, lane);
-    // device-selected mode: more runs than tables, or reference tokens the 32-bit keys cannot
-    // hold (the exact path below is correct but slow: leave those to the wavefront kernels)
-    if (a.check_state && (runs.count > LEV_BV_NT || __any_sync(LEV_FULL_MASK, exact0 != 0))) {
-        if (lane == 0) atomicExch(a.state + 3, 1);
-        return false;
-    }
-    if (valid) a.lead[pair] = (unsigned char)runs.lead;
-
-    int myflags = 0;
-    int rlen = a.R, hlen = a.H;
-#pragma unroll 1
-    for (int base = 0; base < runs.count; base += NT) {
-        const bool active = runs.index >= base && runs.index < base + NT;
-        const int tb = active ? runs.index - base : 0;
-        const bool leader = active && runs.lead == lane;
-        // ---- reference: the lanes of a run build its table together ------------------------
-        // Lane i of a run of n lanes takes positions i, i + n, ...: it claims a free way of the
-        // token's bucket with a CAS on the key word (an equal key already there = duplicate),
-        // then writes its position byte.  Which occurrence ends up representing a token is a
-        // race, and does not matter: a uid only has to be the SAME row for every occurrence
-        // and for the hypothesis look-ups, which all read the finished table.  Positions past
-        // the eos may get in too: their rows receive no bits, so matching them is no match.
-        const int run_pos = lane - runs.lead;
-        int seed = 0;
-        int exact = exact0;  // no usable table: compare tokens one by one (rare)
-        bool need = active && !exact;
-#pragma unroll 1
-        for (int attempt = 0; attempt < LEV_BV_TRIES; ++attempt) {
-            unsigned clear = 0;  // tables (of this pass) being (re)built
-#pragma unroll
-            for (int t = 0; t < NT; ++t)
-                if (__any_sync(LEV_FULL_MASK, need && tb == t)) clear |= 1u << t;
-            if (clear == 0) break;
-            __syncwarp();
-            for (int i = lane; i < nb * NT; i += 32)
-                if ((clear >> (i % NT)) & 1u) {
-                    keys4[i] = make_int4(LEV_BV_EMPTY, LEV_BV_EMPTY, LEV_BV_EMPTY, LEV_BV_EMPTY);
-                    posw[i] = ~0u;
-                }
-            __syncwarp();
-            bool overflow = false;
-            if (need) {
-                seed = attempt;
-                const unsigned hmul = lev_bv_mult(seed);
-                for (int t0 = run_pos; t0 < a.R; t0 += 8 * runs.len) {
-                    int vv[8];  // 8 of my positions at a time: the loads overlap
-#pragma unroll
-                    for (int k = 0; k < 8; ++k)
-                        vv[k] = (t0 + k * runs.len < a.R) ? (int)rsrc[(int64_t)(t0 + k * runs.len) * rst] : 0;
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        const int t = t0 + k * runs.len;
-                        if (t >= a.R) break;
-                        const int v = vv[k];
-                        const int idx = (int)lev_bv_hash(v, hmul, a.slots_log2) * NT + tb;
-                        int* kk = reinterpret_cast<int*>(&keys4[idx]);
-                        int w = 0;
-                        for (; w < 4; ++w) {
-                            const int old = atomicCAS(&kk[w], LEV_BV_EMPTY, v);
-                            if (old == LEV_BV_EMPTY) {
-                                reinterpret_cast<unsigned char*>(&posw[idx])[w] = (unsigned char)t;
-                                break;
-                            }
-                            if (old == v) break;
-                        }
-                        overflow |= w == 4;
-                    }
-                }
-            }
-            // the run retries (next multiplier) if any of its lanes met a full bucket
-            const bool run_bad = (__ballot_sync(LEV_FULL_MASK, overflow) & runs.mask) != 0;
-            need = need && run_bad;
-            if (need && attempt == LEV_BV_TRIES - 1) {
-                need = false;
-                exact = 1;
-            }
-        }
-        __syncwarp();
-        if (active) {
-            rlen = a.R;
-            if (a.has_eos && first_eos < a.R) rlen = first_eos + (a.include_eos ? 1 : 0);
-            if (a.has_eos && a.include_eos && first_eos == a.R) myflags |= B200LEV_FLAG_REF_NO_EOS;
-        }
-        if (active && !exact) {
-            // each lane looks its own positions up and drops the byte into the leader's chunks
-            const unsigned hmul = lev_bv_mult(seed);
-            unsigned char* bytes = reinterpret_cast<unsigned char*>(a.ref_uid);
-            const int64_t lead_pair = pair - run_pos;  // (the leader of a run is always inside the batch)
-            for (int t0 = run_pos; t0 < rlen; t0 += 8 * runs.len) {
-                int vv[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    vv[k] = (t0 + k * runs.len < rlen) ? (int)rsrc[(int64_t)(t0 + k * runs.len) * rst] : 0;
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    const int t = t0 + k * runs.len;
-                    if (t >= rlen) break;
-                    const int v = vv[k];
-                    const int idx = (int)lev_bv_hash(v, hmul, a.slots_log2) * NT + tb;
-                    const int4 kk = keys4[idx];
-                    const unsigned pw = posw[idx];
-                    int way = 4;  // first matching way, the rule the hypothesis look-ups use too
-                    if (kk.w == v) way = 3;
-                    if (kk.z == v) way = 2;
-                    if (kk.y == v) way = 1;
-                    if (kk.x == v) way = 0;
-                    bytes[((int64_t)(t >> 4) * a.P + lead_pair) * 16 + (t & 15)] =
-                        (unsigned char)__byte_perm(pw, LEV_BV_NOMATCH, way);
-                }
-            }
-        }
-        if (leader && exact && valid) {
-            // rare: a reference token outside int32 (equal low words prove nothing) or no
-            // overflow-free table -- this run's uids by exact comparison, O(r^2) cached loads
-            for (int c = 0; c * 16 < a.R; ++c) {
-                unsigned q[4] = {~0u, ~0u, ~0u, ~0u};
-                for (int k = 0; k < 16; ++k) {
-                    const int j = c * 16 + k;
-                    if (j >= rlen) break;
-                    const TT x = rsrc[(int64_t)j * rst];
-                    int u = j;
-                    for (int e = 0; e < j; ++e)
-                        if (rsrc[(int64_t)e * rst] == x) {
-                            u = e;
-                            break;
-                        }
-                    q[k >> 2] = lev_bv_set_byte(q[k >> 2], (unsigned)u, k & 3);
-                }
-                a.ref_uid[(int64_t)c * a.P + pair] = make_uint4(q[0], q[1], q[2], q[3]);
-            }
-        }
-        __syncwarp();
-        // ---- hypothesis: hyp_uid[i] = the row of hyp[i]'s token (0xff: not in the reference).
-        // Every position is looked up, also those past the eos: the DP never reads their bytes,
-        // and the loop stays free of control flow.
-        if (active) {
-            const unsigned hmul = lev_bv_mult(seed);
-            const int eos_lo = (int)a.eos, eos_hi = (int)(a.eos >> 32);
-            int h_eos = a.H;
-            unsigned q[4];
-            // (kept free of branches: the 8 table reads of a half are independent and overlap)
-            auto lookup = [&](const TT (&buf)[8], int t0, int qbase) {
-                unsigned eos_bits = 0;  // bit k: position t0 + k holds the eos
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    const int64_t x = (int64_t)buf[k];
-                    const int v = (int)x, hi = (int)(x >> 32);
-                    eos_bits |= (v == eos_lo && hi == eos_hi) ? (1u << k) : 0u;
-                    const int idx = (int)lev_bv_hash(v, hmul, a.slots_log2) * NT + tb;
-                    const int4 kk = keys4[idx];
-                    const unsigned pw = posw[idx];
-                    // first matching way; a token outside int32 cannot equal an int32 key
-                    int way = 4;
-                    way = kk.w == v ? 3 : way;
-                    way = kk.z == v ? 2 : way;
-                    way = kk.y == v ? 1 : way;
-                    way = kk.x == v ? 0 : way;
-                    if (sizeof(TT) == 8) way = hi != (v >> 31) ? 4 : way;
-                    const unsigned u = __byte_perm(pw, LEV_BV_NOMATCH, way);
-                    q[qbase + (k >> 2)] = lev_bv_set_byte(q[qbase + (k >> 2)], u, k & 3);
-                }
-                // positions past H were loaded as 0, which may be the eos: mask them out
-                const int live = a.H - t0;
-                if (live < 8) eos_bits &= live > 0 ? (1u << live) - 1u : 0u;
-                if (a.has_eos && eos_bits != 0 && h_eos == a.H) h_eos = t0 + __ffs((int)eos_bits) - 1;
-            };
-            const TT* hp = hsrc;
-            TT bufA[8], bufB[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) bufA[k] = (k < a.H) ? lev_ldg_stream(hp + (int64_t)k * hst) : (TT)0;
-#pragma unroll 1
-            for (int t0 = 0; t0 < a.H; t0 += 16) {
-                LEV_OPAQUE_PTR(hp);
-#pragma unroll
-                for (int k = 0; k < 16; ++k)
-                    if (t0 + 48 + k < a.H) lev_prefetch_l2(hp + (int64_t)(48 + k) * hst);
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    bufB[k] = (t0 + 8 + k < a.H) ? lev_ldg_stream(hp + (int64_t)(8 + k) * hst) : (TT)0;
-                q[0] = q[1] = q[2] = q[3] = ~0u;
-                lookup(bufA, t0, 0);
-                hp += 16 * (int64_t)hst;
-                LEV_OPAQUE_PTR(hp);
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    bufA[k] = (t0 + 16 + k < a.H) ? lev_ldg_stream(hp + (int64_t)k * hst) : (TT)0;
-                lookup(bufB, t0 + 8, 2);
-                if (valid) a.hyp_uid[(int64_t)(t0 >> 4) * a.P + pair] = make_uint4(q[0], q[1], q[2], q[3]);
-            }
-            hlen = a.H;
-            if (a.has_eos && h_eos < a.H) hlen = h_eos + (a.include_eos ? 1 : 0);
-            if (a.has_eos && a.include_eos && h_eos == a.H) myflags |= B200LEV_FLAG_HYP_NO_EOS;
-            if (exact && valid) {
-                // rare (see above): the table of this run is unusable, so what the stream just
-                // wrote for this pair is too -- redo it by exact comparison
-                for (int c = 0; c * 16 < hlen; ++c) {
-                    unsigned qq[4] = {~0u, ~0u, ~0u, ~0u};
-                    for (int k = 0; k < 16 && c * 16 + k < hlen; ++k) {
-                        const int64_t x = (int64_t)hsrc[(int64_t)(c * 16 + k) * hst];
-                        unsigned u = LEV_BV_NOMATCH;
-                        for (int e = 0; e < rlen; ++e)
-                            if ((int64_t)rsrc[(int64_t)e * rst] == x) {
-                                u = (unsigned)e;
-                                break;
-                            }
-                        qq[k >> 2] = lev_bv_set_byte(qq[k >> 2], u, k & 3);
-                    }
-                    a.hyp_uid[(int64_t)c * a.P + pair] = make_uint4(qq[0], qq[1], qq[2], qq[3]);
-                }
-            }
-        }
-    }
-    if (valid) {
-        a.hyp_len[pair] = hlen;
-        if (pair % a.ref_group == 0) a.ref_len[rcol] = rlen;
-        if (a.norm && rlen == 0) myflags |= B200LEV_FLAG_EMPTY_REF;  // SM:360-366, 397-404
-    } else {
-        myflags = 0;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) myflags |= __shfl_xor_sync(LEV_FULL_MASK, myflags, o);
-    if (lane == 0 && myflags != 0 && a.flags != nullptr) atomicOr(a.flags, myflags);
-    __syncwarp();  // the next block of this warp reuses the tables
-    return true;
-}
-
-// Warps are independent and walk the blocks of 32 pairs with a grid stride: the grid stays
-// small (a vetoed launch, or this kernel standing by, drains in a few microseconds).
-// (4 CTAs per SM on purpose: with 128 registers the compiler keeps both load batches and the
-// look-up temporaries in registers -- 118 -> 100 us on cfg2 against 5 CTAs at 96 registers)
-template <typename TT>
-__global__ void __launch_bounds__(32 * LEV_BV_WARPS, 4) lev_bv_uid_kernel(const LevBvArgs a) {
-    LEV_DYN_SMEM(int, smem);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int nb = 1 << a.slots_log2;  // buckets per table
-    // per warp: keys [nb][NT] int4 (4 ways), then posw [nb][NT] words (4 position bytes)
-    int4* keys4 = reinterpret_cast<int4*>(smem + (size_t)warp * (nb * LEV_BV_NT * 5));
-    unsigned* posw = reinterpret_cast<unsigned*>(keys4 + nb * LEV_BV_NT);
-    const int64_t nblocks = ((int64_t)a.P + 31) / 32;
-    for (int64_t block = (int64_t)blockIdx.x * LEV_BV_WARPS + warp; block < nblocks;
-         block += (int64_t)gridDim.x * LEV_BV_WARPS) {
-        if (a.check_state && !lev_bv_took(a.state)) return;  // some warp has vetoed
-        if (!lev_bv_uid_block<TT>(a, keys4, posw, nb, block, lane)) return;
-    }
-}
-
-// ---------------------------------------------------------------------------------------
-// the DP
-// ---------------------------------------------------------------------------------------
-template <int W, int MODE>
-__device__ __forceinline__ void lev_bv_dp_block(const LevBvArgs& a, unsigned* M, const int tab_words,
-                                                const int64_t block, const int lane) {
-    constexpr int NT = LEV_BV_NT;
-    const int64_t pair = block * 32 + lane;
-    const bool valid = pair < a.P;
-    const int64_t pc = valid ? pair : (int64_t)a.P - 1;
-    const int r = a.ref_len[pc / a.ref_group], h = a.hyp_len[pc];
-    const int Z = a.R;
-    const LevBvRuns runs = lev_bv_runs(lane > 0 && (int)a.lead[pc] != lane, lane);
-    // the reference occupies bits [o, 32 W)
-    const int o = 32 * W - r;
-    const int mysteps = a.exclude_last ? (h > 0 ? h - 1 : 0) : h;  // SM:286-288
-    const float rf = (float)r;
-    const float y = r > 0 ? __frcp_rn(rf) : 0.0f;
-    const int first_pad = h + (a.exclude_last ? 0 : 1);
-
-    for (int base = 0; base < runs.count; base += NT) {
-        const bool active = runs.index >= base && runs.index < base + NT;
-        const int tb = active ? runs.index - base : 0;
-        const bool leader = active && runs.lead == lane;
-        __syncwarp();
-        {
-            uint4* mz = reinterpret_cast<uint4*>(M);
-            for (int i = lane; i < tab_words / 4; i += 32) mz[i] = make_uint4(0u, 0u, 0u, 0u);
-        }
-        __syncwarp();
-        if (leader) {  // the run's match masks, from its leader's uid bytes
-            for (int c = 0; c * 16 < r; ++c) {
-                const uint4 q4 = a.ref_uid[(int64_t)c * a.P + pc];
-                const unsigned q[4] = {q4.x, q4.y, q4.z, q4.w};
-#pragma unroll
-                for (int k = 0; k < 16; ++k) {
-                    const int j = c * 16 + k;
-                    if (j < r) {
-                        const unsigned u = (q[k >> 2] >> (8 * (k & 3))) & 0xffu;
-                        const int b = j + o;
-                        M[(u * NT + tb) * W + (b >> 5)] |= 1u << (b & 31);
-                    }
-                }
-            }
-        }
-        __syncwarp();
-        // rows this pass has to run: the longest hypothesis among its pairs
-        int steps = active ? mysteps : 0;
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            const int other = __shfl_xor_sync(LEV_FULL_MASK, steps, d);
-            steps = other > steps ? other : steps;
-        }
-        if (!active) continue;  // (no warp-wide operation below this line in the pass)
-        unsigned pv[W], mv[W];
-#pragma unroll
-        for (int w = 0; w < W; ++w) {
-            const int lo = 32 * w;
-            pv[w] = o <= lo ? ~0u : (o >= lo + 32 ? 0u : (~0u << (o - lo)));
-            mv[w] = 0u;
-        }
-        int score = r;
-        float* __restrict__ orow = a.out + pair;  // prefix: row 0 of this pair
-        auto emit = [&](int i, int rv) {          // SM:352-388: one output row
-            float val = __fmul_rn((float)rv, a.mult);
-            if (a.norm) {
-                if (r == 0) {
-                    val = i > 0 ? 1.0f : 0.0f;
-                } else {  // correctly rounded val / r (Markstein, see lev_group.cu)
-                    const float q0 = __fmul_rn(val, y);
-                    val = __fmaf_rn(__fmaf_rn(-rf, q0, val), y, q0);
-                }
-            }
-            if (valid) *orow = i < first_pad ? val : a.padding;
-            orow += a.out_si;
-        };
-        int fin = r;  // FINAL: hypotheses without rows keep D[r][0] = r
-        if (MODE == LEV_MODE_PREFIX && a.Hout > 0) emit(0, r);
-        int i = 1;
-        uint4 q4 = make_uint4(~0u, ~0u, ~0u, ~0u);
-        if (steps > 0) q4 = a.hyp_uid[pc];
-        for (int c = 0; c * 16 < steps; ++c) {
-            const unsigned q[4] = {q4.x, q4.y, q4.z, q4.w};
-            if ((c + 1) * 16 < steps) q4 = a.hyp_uid[(int64_t)(c + 1) * a.P + pc];  // next chunk
-#pragma unroll
-            for (int k = 0; k < 16; ++k, ++i) {
-                if (i > steps) break;
-                unsigned u = (q[k >> 2] >> (8 * (k & 3))) & 0xffu;
-                u = u < (unsigned)Z ? u : (unsigned)Z;
-                unsigned eq[W];
-                // a row's W words are adjacent: one 128-bit (W = 4) or 64-bit (W = 2) read; the
-                // lanes of a run read the same address (broadcast)
-                const unsigned* row = M + (u * NT + tb) * W;
-                if (W == 4) {
-                    const uint4 e = *reinterpret_cast<const uint4*>(row);
-                    eq[0] = e.x;
-                    eq[W > 1 ? 1 : 0] = e.y;
-                    eq[W > 2 ? 2 : 0] = e.z;
-                    eq[W > 3 ? 3 : 0] = e.w;
-                } else if (W == 2) {
-                    const uint2 e = *reinterpret_cast<const uint2*>(row);
-                    eq[0] = e.x;
-                    eq[W > 1 ? 1 : 0] = e.y;
-                } else {
-#pragma unroll
-                    for (int w = 0; w < W; ++w) eq[w] = row[w];
-                }
-                score += lev_bv_step<W>(eq, pv, mv);
-                if (MODE == LEV_MODE_PREFIX) {
-                    emit(i, score);
-                } else if (i == h) {
-                    fin = score;
-                }
-            }
-        }
-        if (MODE == LEV_MODE_PREFIX) {
-            for (; i < a.Hout; ++i) {  // rows past every hypothesis of this pass
-                if (valid) *orow = a.padding;
-                orow += a.out_si;
-            }
-        } else if (valid) {  // SM:390-405
-            float val = __fmul_rn((float)fin, a.mult);
-            if (a.norm) val = (r == 0) ? (h > 0 ? 1.0f : 0.0f) : val / rf;
-            a.out[pair] = val;
-        }
-    }
-    __syncwarp();  // the next block of this warp reuses the tables
-}
-
-template <int W, int MODE>
-__global__ void __launch_bounds__(32 * LEV_BV_WARPS) lev_bv_dp_kernel(const LevBvArgs a) {
-    if (a.check_state && !lev_bv_took(a.state)) return;
-    LEV_DYN_SMEM(unsigned, smem);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    // per warp: Peq[(R + 1)][NT tables][W]; row R stays zero (no match)
-    const int tab_words = (a.R + 1) * W * LEV_BV_NT;
-    unsigned* M = smem + (size_t)warp * tab_words;
-    const int64_t nblocks = ((int64_t)a.P + 31) / 32;
-    for (int64_t block = (int64_t)blockIdx.x * LEV_BV_WARPS + warp; block < nblocks;
-         block += (int64_t)gridDim.x * LEV_BV_WARPS)
-        lev_bv_dp_block<W, MODE>(a, M, tab_words, block, lane);
-}
 
 // ---------------------------------------------------------------------------------------
 // host side
@@ -547,15 +63,10 @@ bool lev_bitvec_eligible(const b200lev_tokens_t* ref, const b200lev_tokens_t* hy
     if (mode != LEV_MODE_FINAL && mode != LEV_MODE_PREFIX) return false;
     if (count_mode || float_path || ins_i != 1 || del_i != 1 || sub_i != 1) return false;
     if (ref->T > 128 || ref->T < 1 || hyp->T >= (1 << 20)) return false;
+    if (!lev_bvfused_supports(ref->elem_bytes) || ref->elem_bytes != hyp->elem_bytes) return false;
     *short_form = lev_bvshort_supports(ref->elem_bytes, ref->T) && hyp->N >= lev_bvshort_min_pairs();
-    {
-        const char* e = getenv("B200LEV_BV_FUSED");
-        const char* g = getenv("B200LEV_BV_GROUPED");
-        *grouped = !*short_form && ref_group >= 8 && hyp->N >= 128 && !(e != nullptr && atoi(e) == 0) &&
-                   !(g != nullptr && atoi(g) == 0) && lev_bvfused_supports(ref->elem_bytes);
-    }
+    *grouped = !*short_form && ref_group >= 8 && hyp->N >= 128;
     if (!*short_form && !*grouped && hyp->N < lev_bv_min_pairs()) return false;
-    if (ref->elem_bytes != hyp->elem_bytes) return false;
     if (ref->stride_t >= ((int64_t)1 << 31) || hyp->stride_t >= ((int64_t)1 << 31) ||
         ref->stride_t < 0 || hyp->stride_t < 0)
         return false;
@@ -564,47 +75,14 @@ bool lev_bitvec_eligible(const b200lev_tokens_t* ref, const b200lev_tokens_t* hy
     return true;
 }
 
-// CTAs for P pairs: every CTA an equal number of 128-pair blocks, at most `per_sm` x 148 CTAs
-static unsigned lev_bv_grid(int64_t P, int per_sm) {
-    int64_t n = (P + 32 * LEV_BV_WARPS - 1) / (32 * LEV_BV_WARPS);
-    const int64_t cap = (int64_t)148 * per_sm;
-    if (n > cap) {
-        const int64_t each = (n + cap - 1) / cap;
-        n = (n + each - 1) / each;
-    }
-    return (unsigned)n;
-}
-
-template <typename TT>
-static void lev_bv_launch_uid(const LevBvArgs& a, size_t smem, cudaStream_t st) {
-    auto kern = lev_bv_uid_kernel<TT>;
-    if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    lev_launch(kern, dim3(lev_bv_grid(a.P, 10)), dim3(32 * LEV_BV_WARPS), smem, st, a);
-}
-
-template <int W>
-static void lev_bv_launch_dp(const LevBvArgs& a, cudaStream_t st) {
-    const size_t smem = sizeof(unsigned) * (size_t)(a.R + 1) * W * LEV_BV_NT * LEV_BV_WARPS;
-    const dim3 grid(lev_bv_grid(a.P, 16)), block(32 * LEV_BV_WARPS);
-    if (a.mode == LEV_MODE_PREFIX) {
-        auto kern = lev_bv_dp_kernel<W, LEV_MODE_PREFIX>;
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        lev_launch(kern, grid, block, smem, st, a);
-    } else {
-        auto kern = lev_bv_dp_kernel<W, LEV_MODE_FINAL>;
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        lev_launch(kern, grid, block, smem, st, a);
-    }
-}
-
-// The caller has checked lev_bitvec_eligible.  `uid_ref` / `uid_hyp` are workspace regions of
-// P * round_up(R, 16) and P * round_up(H, 16) bytes, `lead` of P bytes.  `state` non-NULL:
-// the kernels run only if K0's state words select this path (lev_bv_selected).
+// The caller has checked lev_bitvec_eligible.  `counter` is one workspace word (Kb's block
+// counter).  `state` non-NULL: device-selected mode, Kb runs only if its probe does not veto;
+// `after_probe` (a cudaEvent_t, may be NULL) is recorded once that decision is final.
 int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                       const b200lev_opts_t* o, int mode, float mult, int32_t* ref_len,
-                      int32_t* hyp_len, void* uid_ref, void* uid_hyp, void* lead,
-                      int32_t* state, int32_t* flags, float* out, int64_t out_si, int Hout,
-                      cudaStream_t st, void* after_uid, bool short_form, double* acc) {
+                      int32_t* hyp_len, int* counter, int32_t* state, int32_t* flags, float* out,
+                      int64_t out_si, int Hout, cudaStream_t st, void* after_probe, bool short_form,
+                      double* acc) {
     LevBvArgs a;
     memset(&a, 0, sizeof(a));
     a.ref = ref->data;
@@ -620,9 +98,7 @@ int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     a.include_eos = o->include_eos;
     a.ref_len = ref_len;
     a.hyp_len = hyp_len;
-    a.ref_uid = (uint4*)uid_ref;
-    a.hyp_uid = (uint4*)uid_hyp;
-    a.lead = (unsigned char*)lead;
+    a.counter = counter;
     a.state = state;
     a.check_state = state != nullptr;
     a.flags = flags;
@@ -636,52 +112,14 @@ int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     a.padding = (float)o->padding;
     a.out = out;
     a.out_si = out_si;
-    a.acc = (short_form && mode == LEV_MODE_FINAL && !(getenv("B200LEV_BVS_SUMS") && atoi(getenv("B200LEV_BVS_SUMS")) == 0)) ? acc : nullptr;
+    a.acc = (short_form && mode == LEV_MODE_FINAL) ? acc : nullptr;
     if (short_form) {  // R <= 64: lane = pair, reference in registers, no tables (lev_bvshort.cu)
         if (getenv("B200LEV_TRACE"))
             fprintf(stderr, "b200lev: short bit-vector kernel, mode %d, R=%d H=%d P=%d\n", mode, a.R, a.H, a.P);
         return lev_bvshort_launch(a, ref->elem_bytes, st);
     }
-    // B200LEV_BV_FUSED=0 keeps the two-kernel form (uid pre-pass + DP) for comparison
-    const char* fe = getenv("B200LEV_BV_FUSED");
-    if ((fe == nullptr || atoi(fe) != 0) && lev_bvfused_supports(ref->elem_bytes)) {
-        if (getenv("B200LEV_TRACE"))
-            fprintf(stderr, "b200lev: fused bit-vector kernel, mode %d, R=%d H=%d P=%d W=%d device-selected=%d\n",
-                    mode, a.R, a.H, a.P, (a.R + 31) / 32, a.check_state);
-        return lev_bvfused_launch(a, ref->elem_bytes, st, after_uid);
-    }
-    const size_t smem_uid = (size_t)(1 << a.slots_log2) * LEV_BV_NT * 20 * LEV_BV_WARPS;
     if (getenv("B200LEV_TRACE"))
-        fprintf(stderr, "b200lev: bit-vector path, mode %d, R=%d H=%d P=%d W=%d device-selected=%d\n",
+        fprintf(stderr, "b200lev: fused bit-vector kernel, mode %d, R=%d H=%d P=%d W=%d device-selected=%d\n",
                 mode, a.R, a.H, a.P, (a.R + 31) / 32, a.check_state);
-    lev_prof_begin(LEV_PROF_BV_UID, st);
-    switch (ref->elem_bytes) {
-        case 8: lev_bv_launch_uid<int64_t>(a, smem_uid, st); break;
-        case 4: lev_bv_launch_uid<int32_t>(a, smem_uid, st); break;
-        case 2: lev_bv_launch_uid<int16_t>(a, smem_uid, st); break;
-        case 1: lev_bv_launch_uid<int8_t>(a, smem_uid, st); break;
-        default:
-            lev_set_error("unsupported token element size %d", (int)ref->elem_bytes);
-            return B200LEV_ERR_ARG;
-    }
-    lev_prof_end(LEV_PROF_BV_UID, st);
-    int rc = lev_check_cuda("lev_bv_uid_kernel");
-    if (rc) return rc;
-#ifndef B200LEV_EMU
-    // the veto is final once this kernel is done: the stand-by chain forks from here
-    if (after_uid != nullptr && cudaEventRecord((cudaEvent_t)after_uid, st) != cudaSuccess)
-        return lev_check_cuda("cudaEventRecord");
-#else
-    (void)after_uid;
-#endif
-    lev_prof_begin(LEV_PROF_BV_DP, st);
-    const int W = (a.R + 31) / 32;
-    switch (W) {
-        case 1: lev_bv_launch_dp<1>(a, st); break;
-        case 2: lev_bv_launch_dp<2>(a, st); break;
-        case 3: lev_bv_launch_dp<3>(a, st); break;
-        default: lev_bv_launch_dp<4>(a, st); break;
-    }
-    lev_prof_end(LEV_PROF_BV_DP, st);
-    return lev_check_cuda("lev_bv_dp_kernel");
+    return lev_bvfused_launch(a, ref->elem_bytes, st, after_probe);
 }

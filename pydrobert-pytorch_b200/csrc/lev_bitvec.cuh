@@ -1,12 +1,11 @@
-// lev_bitvec.cuh -- pieces shared by the unit-cost bit-vector kernels (lev_bitvec.cu: the
-// two-kernel uid + DP form; lev_bvfused.cu: the fused single-kernel form).
+// lev_bitvec.cuh -- pieces shared by the unit-cost bit-vector kernels (lev_bvfused.cu: Kb, the
+// n-best kernel; lev_bvshort.cu: Ks, the short-reference kernel) and their host-side selection
+// (lev_bitvec.cu).
 #pragma once
 #include "lev_common.cuh"
 
-#define LEV_BV_NOMATCH 0xffu
 #define LEV_BV_EMPTY ((int)0x80000000)  // key of a free way (a token with this value: exact path)
-constexpr int LEV_BV_NT = 4;     // tables per warp = runs of identical references per pass
-constexpr int LEV_BV_WARPS = 4;  // warps per CTA (independent: no block barrier anywhere)
+constexpr int LEV_BV_NT = 4;  // tables per warp = runs of identical references per pass
 
 struct LevBvArgs {
     const void* ref;  // raw token tensors, stride 1 along the batch axis
@@ -18,9 +17,7 @@ struct LevBvArgs {
     int include_eos;
     int32_t* ref_len;  // [Nref]  (same workspace slots K0 fills on the other paths)
     int32_t* hyp_len;  // [P]
-    uint4* ref_uid;    // [ceil(R/16)][P]  16 uid bytes per (chunk, pair); run leaders only
-    uint4* hyp_uid;    // [ceil(H/16)][P]
-    unsigned char* lead;  // [P] lane (0..31) of the leader of the pair's run in its 32-block
+    int* counter;      // Kb: the next block of 32 pairs to claim (zeroed by the probe or a memset)
     int32_t* flags;    // caller's warning flags, may be NULL
     int32_t* state;  // workspace state words; [3] != 0 = "not for this path" (lev_bv_took)
     int check_state;   // device-selected mode: veto through state[3] instead of multi-pass
@@ -66,10 +63,6 @@ __device__ __forceinline__ LevBvRuns lev_bv_runs(bool same, int lane) {
     return r;
 }
 
-__device__ __forceinline__ unsigned lev_bv_set_byte(unsigned word, unsigned byte, int k) {
-    return (word & ~(0xffu << (8 * k))) | (byte << (8 * k));
-}
-
 // sum = t + pv over W 32-bit words (carry chain in one asm block)
 template <int W>
 __device__ __forceinline__ void lev_bv_add(const unsigned (&t)[W], const unsigned (&pv)[W],
@@ -104,111 +97,13 @@ __device__ __forceinline__ void lev_bv_add(const unsigned (&t)[W], const unsigne
 #endif
 }
 
-// One row of the recurrence; returns the score change at the top bit (reference column r).
-template <int W>
-__device__ __forceinline__ int lev_bv_step(const unsigned (&eq)[W], unsigned (&pv)[W],
-                                           unsigned (&mv)[W]) {
-    unsigned t[W], sum[W], ph[W], mh[W];
-#pragma unroll
-    for (int w = 0; w < W; ++w) t[w] = eq[w] & pv[w];
-    lev_bv_add<W>(t, pv, sum);
-#pragma unroll
-    for (int w = 0; w < W; ++w) {
-        const unsigned xh = (sum[w] ^ pv[w]) | eq[w];
-        ph[w] = mv[w] | ~(xh | pv[w]);
-        mh[w] = pv[w] & xh;
-    }
-    const int delta = (int)(ph[W - 1] >> 31) - (int)(mh[W - 1] >> 31);
-#pragma unroll
-    for (int w = W - 1; w >= 0; --w) {
-        const unsigned phs = w ? __funnelshift_l(ph[w - 1], ph[w], 1) : ((ph[0] << 1) | 1u);
-        const unsigned mhs = w ? __funnelshift_l(mh[w - 1], mh[w], 1) : (mh[0] << 1);
-        const unsigned xv = eq[w] | mv[w];
-        pv[w] = mhs | ~(xv | phs);
-        mv[w] = phs & xv;
-    }
-    return delta;
-}
-
-
 // ---------------------------------------------------------------------------------------
-// pieces of the fused kernel (lev_bvfused.cu)
+// the two kernels' launchers; the hash-table build of Kb
 // ---------------------------------------------------------------------------------------
 bool lev_bvshort_supports(int elem_bytes, int64_t R);
 int lev_bvshort_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st);
 bool lev_bvfused_supports(int elem_bytes);
 int lev_bvfused_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st, void* after_probe);
-
-struct LevBvRefScan {
-    int first_eos;  // position of the first eos in my reference column (R: none)
-    int exact0;     // the column holds a token the 32-bit keys cannot represent
-    bool diff;      // my column differs from my left neighbour's (a run starts at this lane)
-    bool vetoed;    // (may_veto) more than LEV_BV_NT runs after the first tokens
-};
-
-// One coalesced pass over a lane's reference column, 16 positions per half, the two halves'
-// loads ping-pong: runs of identical references (SM:1426/1439 repeat every reference over its
-// n-best list), first eos (SM:137-143, 198-218), tokens outside int32.
-template <typename TT>
-__device__ __forceinline__ LevBvRefScan lev_bv_ref_scan(const LevBvArgs& a, const TT* __restrict__ rsrc,
-                                                        const int rst, const int64_t rcol,
-                                                        const int lane, const bool may_veto) {
-    LevBvRefScan s;
-    s.first_eos = a.R;
-    s.exact0 = 0;
-    s.vetoed = false;
-    const int prev_col = __shfl_up_sync(LEV_FULL_MASK, (int)rcol, 1);
-    const bool other = prev_col != (int)rcol;
-    const int eos_lo = (int)a.eos, eos_hi = (int)(a.eos >> 32);
-    int dacc = 0, wacc = 0;  // differences to the left neighbour / to a sign extension
-    constexpr int DH = 16;
-    auto observe = [&](const TT (&buf)[DH], int t0) {
-        unsigned eos_bits = 0, empty_bits = 0;
-#pragma unroll
-        for (int k = 0; k < DH; ++k) {
-            const int64_t x = (int64_t)buf[k];
-            const int lo = (int)x, hi = (int)(x >> 32);
-            dacc |= lo ^ __shfl_up_sync(LEV_FULL_MASK, lo, 1);
-            if (sizeof(TT) == 8) {
-                dacc |= hi ^ __shfl_up_sync(LEV_FULL_MASK, hi, 1);
-                wacc |= hi ^ (lo >> 31);
-            }
-            eos_bits |= (lo == eos_lo && hi == eos_hi) ? (1u << k) : 0u;
-            empty_bits |= lo == LEV_BV_EMPTY ? 1u : 0u;
-        }
-        // positions past R were loaded as 0 (= what the neighbour loaded): mask them out
-        const int live = a.R - t0;
-        if (live < DH) eos_bits &= live > 0 ? (1u << live) - 1u : 0u;
-        if (a.has_eos && eos_bits != 0 && s.first_eos == a.R) s.first_eos = t0 + __ffs((int)eos_bits) - 1;
-        if (empty_bits) s.exact0 = 1;
-    };
-    const TT* rp = rsrc;
-    TT bufA[DH], bufB[DH];
-#pragma unroll
-    for (int k = 0; k < DH; ++k) bufA[k] = (k < a.R) ? rp[(int64_t)k * rst] : (TT)0;
-#pragma unroll 1
-    for (int t0 = 0; t0 < a.R; t0 += 2 * DH) {
-        LEV_OPAQUE_PTR(rp);
-#pragma unroll
-        for (int k = 0; k < DH; ++k) bufB[k] = (t0 + DH + k < a.R) ? rp[(int64_t)(DH + k) * rst] : (TT)0;
-        observe(bufA, t0);
-        if (may_veto && t0 == 0) {
-            const unsigned same = __ballot_sync(LEV_FULL_MASK, lane > 0 && !(dacc != 0 && other));
-            if (32 - __popc(same) > LEV_BV_NT) {
-                s.vetoed = true;
-                break;
-            }
-        }
-        rp += 2 * DH * (int64_t)rst;
-        LEV_OPAQUE_PTR(rp);
-#pragma unroll
-        for (int k = 0; k < DH; ++k) bufA[k] = (t0 + 2 * DH + k < a.R) ? rp[(int64_t)k * rst] : (TT)0;
-        observe(bufB, t0 + DH);
-    }
-    s.diff = dacc != 0 && other;
-    if (wacc != 0) s.exact0 = 1;
-    return s;
-}
 
 // The lanes of a run build its hash table together (warp-collective: every lane calls it).
 // Lane i of a run of n lanes takes positions i, i + n, ...: it claims a free way of the token's

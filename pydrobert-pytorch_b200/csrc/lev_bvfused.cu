@@ -1,20 +1,17 @@
-// lev_bvfused.cu -- the unit-cost n-best fast path as ONE kernel: lengths, run detection,
+// lev_bvfused.cu -- Kb, the unit-cost n-best fast path as ONE kernel: lengths, run detection,
 // token -> match-mask tables and Myers' bit-vector recurrence, lane = pair, straight from the
 // raw sequence-first tokens to the (H', N) output rows.
 //
-// lev_bitvec.cu does the same work in two kernels that meet in global memory (1 uid byte per
-// token).  Its uid pre-pass is a latency-bound gather (16 warps/SM behind 40 KB of hash tables
-// per CTA, ~58 instructions per hypothesis token, 0.36 of the HBM peak) that takes longer than
-// the DP it prepares.  Fused, the hash look-up of hypothesis token i feeds the Myers step of row
-// i directly: the look-up's shared-memory latency hides behind the ~45 ALU instructions of the
-// previous row's step, the uid bytes never exist, and one launch replaces two.  Per warp (32
-// consecutive pairs = 4 runs of an 8-best batch):
+// The hash look-up of hypothesis token i feeds the Myers step of row i directly: the look-up's
+// shared-memory latency hides behind the ~45 ALU instructions of the previous row's step, and
+// no per-token intermediate goes through global memory (DESIGN §9).  Per warp (32 consecutive
+// pairs = 4 runs of an 8-best batch):
 //
 //   A  one coalesced pass over the reference columns: runs of identical references (each lane
-//      compares with its left neighbour), first eos, "needs 64-bit compares" (lev_bv_ref_scan)
+//      compares with its left neighbour), first eos, "needs 64-bit compares" (lev_bvf_scan)
 //   B  per run, its lanes build ONE bucketed hash table token -> first-claimed position
-//      (lev_bv_build_table, shared with lev_bitvec.cu), then set, for every reference position,
-//      its bit in the match mask Peq[position byte] of the run (shared-memory atomicOr)
+//      (lev_bv_build_table, lev_bitvec.cuh), then set, for every reference position, its bit in
+//      the match mask Peq[position byte] of the run (shared-memory atomicOr)
 //   C  every lane streams ITS hypothesis column (rows of 32 neighbouring pairs: one coalesced
 //      256-byte load per row, two halves of 8 rows in flight), and per token: hash -> 128-bit
 //      read of the bucket's keys -> position byte -> 128-bit read of Peq -> Myers step ->
@@ -45,23 +42,11 @@ constexpr int LEV_BVF_WARPS = LEV_BVF_WARPS_PER_CTA;
 #ifndef LEV_BVF_CH
 #define LEV_BVF_CH 4  // hypothesis positions per loop trip
 #endif
-#ifndef LEV_BVF_PRED_ST
-#define LEV_BVF_PRED_ST 1  // 1: the row store as one predicated instruction, no branch
-#endif
-#ifndef LEV_BVF_SCAN_PTR
-#define LEV_BVF_SCAN_PTR 1  // 1: the reference scan reads through a running pointer
-#endif
 #ifndef LEV_BVF_PF_AHEAD
 #define LEV_BVF_PF_AHEAD 32  // rows the L2 prefetch runs ahead of the hypothesis stream
 #endif
-#ifndef LEV_BVF_DYNAMIC
-#define LEV_BVF_DYNAMIC 1  // 1: after its first block a warp claims blocks from a global counter
-#endif
 #ifndef LEV_BVF_PROBE_BLOCKS
 #define LEV_BVF_PROBE_BLOCKS 1024  // blocks of 32 pairs the probe samples at most
-#endif
-#ifndef LEV_BVF_LD_PLAIN
-#define LEV_BVF_LD_PLAIN 0  // 1: plain loads instead of evict-first ones in the hypothesis stream
 #endif
 
 // ---- the match-mask table of one pass: M[(R + 1)][NT][W], row R stays zero (no match) ----
@@ -155,7 +140,7 @@ __device__ __forceinline__ LevBvfScan lev_bvf_scan(const LevBvArgs& a, const TT*
     const TT* __restrict__ rp = rsrc;
     int tl = 0;  // first row of the next batch
     auto ld_batch = [&](TT (&buf)[DH]) {
-        if (LEV_BVF_SCAN_PTR && tl + DH <= a.R) {  // (warp-uniform)
+        if (tl + DH <= a.R) {  // (warp-uniform)
 #pragma unroll
             for (int k = 0; k < DH; ++k) buf[k] = rp[(int64_t)k * rst];
             rp += (int64_t)DH * rst;
@@ -367,11 +352,7 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
             if (PREFIX) {
                 // row t is a value iff t <= h (t < h with exclude_last: token t must exist)
                 const int c_m = EXCL ? in_m : prev_m;
-#if LEV_BVF_PRED_ST
                 lev_st_f32_if(t < a.Hout, orow, c_m != 0 ? prev_val : a.padding);
-#else
-                if (t < a.Hout) *orow = c_m != 0 ? prev_val : a.padding;
-#endif
                 orow += a.out_si;
                 prev_m = in_m;
             }
@@ -430,7 +411,7 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
                 if (tl + CH <= H) {  // (warp-uniform)
 #pragma unroll
                     for (int k = 0; k < CH; ++k)
-                        buf[k] = LEV_BVF_LD_PLAIN ? hp[(int64_t)k * hst] : lev_ldg_stream(hp + (int64_t)k * hst);
+                        buf[k] = lev_ldg_stream(hp + (int64_t)k * hst);
                     hp += (int64_t)CH * hst;
                 } else {
 #pragma unroll
@@ -520,8 +501,8 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
 }
 
 // Warps are independent: each takes the block of 32 pairs of its own index, then claims further
-// blocks from a global counter (LEV_BVF_DYNAMIC; a grid stride without it).  Per warp: keys
-// [nb][NT] int4 (4 ways), posw [nb][NT] words (4 position bytes), M [(R + 1)][NT][W] words.
+// blocks from a global counter.  Per warp: keys [nb][NT] int4 (4 ways), posw [nb][NT] words
+// (4 position bytes), M [(R + 1)][NT][W] words.
 template <typename TT, int W, int KIND>
 __global__ void __launch_bounds__(32 * LEV_BVF_WARPS, LEV_BVF_CTAS_PER_SM) lev_bv_fused_kernel(const LevBvArgs a) {
     if (a.check_state && !lev_bv_took(a.state)) return;  // the probe handed the batch back
@@ -536,13 +517,12 @@ __global__ void __launch_bounds__(32 * LEV_BVF_WARPS, LEV_BVF_CTAS_PER_SM) lev_b
     const int64_t nblocks = ((int64_t)a.P + 31) / 32;
     const int64_t stride = (int64_t)gridDim.x * LEV_BVF_WARPS;
     const int64_t first = (int64_t)blockIdx.x * LEV_BVF_WARPS + warp;
-#if LEV_BVF_DYNAMIC
-    // The first block of a warp is its own; further ones are claimed from a counter (the first
-    // word of the uid region, which this form leaves idle; zeroed by the probe or a memset), one
-    // block AHEAD so that the stream of the current block can announce the next one to L2.  A
-    // warp's blocks take different times (ragged hypotheses, table retries): equal shares leave
-    // the last warps of an SM running alone at a third of the occupancy.
-    int* counter = reinterpret_cast<int*>(a.ref_uid);
+    // The first block of a warp is its own; further ones are claimed from a counter (zeroed by
+    // the probe or a memset), one block AHEAD so that the stream of the current block can
+    // announce the next one to L2.  A warp's blocks take different times (ragged hypotheses,
+    // table retries): equal shares leave the last warps of an SM running alone at a third of
+    // the occupancy.
+    int* counter = a.counter;
     auto claim = [&]() -> int64_t {
         int c = 0;
         if (lane == 0) c = atomicAdd(counter, 1);
@@ -558,11 +538,6 @@ __global__ void __launch_bounds__(32 * LEV_BVF_WARPS, LEV_BVF_CTAS_PER_SM) lev_b
         block = next;
         first_block = false;
     }
-#else
-    for (int64_t block = first; block < nblocks; block += stride)
-        lev_bvf_block<TT, W, KIND>(a, keys4, posw, M, nb, tab_words, block,
-                                   block + stride < nblocks ? block + stride : -1, block == first, lane);
-#endif
 }
 
 // ---- the probe: is this an n-best shaped batch? ---------------------------------------------
@@ -573,9 +548,7 @@ __global__ void __launch_bounds__(128) lev_bv_probe_kernel(const LevBvArgs a, co
                                                            const int64_t nsample) {
     const int lane = threadIdx.x & 31;
     const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-#if LEV_BVF_DYNAMIC
-    if (blockIdx.x == 0 && threadIdx.x == 0) *reinterpret_cast<int*>(a.ref_uid) = 0;  // the block counter
-#endif
+    if (blockIdx.x == 0 && threadIdx.x == 0) *a.counter = 0;
     if (s >= nsample) return;
     const int64_t block = s * stride;
     const int64_t pair = block * 32 + lane;
@@ -637,7 +610,9 @@ static void lev_bvf_launch_t(const LevBvArgs& a, cudaStream_t st) {
     }
 }
 
-bool lev_bvfused_supports(int elem_bytes) { return elem_bytes == 8 || elem_bytes == 4 || elem_bytes == 2; }
+bool lev_bvfused_supports(int elem_bytes) {
+    return elem_bytes == 8 || elem_bytes == 4 || elem_bytes == 2 || elem_bytes == 1;
+}
 
 // `a` as lev_bitvec_launch fills it.  With a.check_state the probe runs first and `after_probe`
 // (a cudaEvent_t, may be NULL) is recorded behind it: the veto is final from there on.
@@ -647,19 +622,18 @@ int lev_bvfused_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st, void
         const int64_t stride = (nblocks + LEV_BVF_PROBE_BLOCKS - 1) / LEV_BVF_PROBE_BLOCKS;
         const int64_t nsample = (nblocks + stride - 1) / stride;
         const dim3 grid((unsigned)((nsample + 3) / 4)), block(128);
-        lev_prof_begin(LEV_PROF_BV_UID, st);
+        lev_prof_begin(LEV_PROF_BV_PROBE, st);
         switch (elem_bytes) {
             case 8: lev_launch(lev_bv_probe_kernel<int64_t>, grid, block, 0, st, a, stride, nsample); break;
             case 4: lev_launch(lev_bv_probe_kernel<int32_t>, grid, block, 0, st, a, stride, nsample); break;
-            default: lev_launch(lev_bv_probe_kernel<int16_t>, grid, block, 0, st, a, stride, nsample); break;
+            case 2: lev_launch(lev_bv_probe_kernel<int16_t>, grid, block, 0, st, a, stride, nsample); break;
+            default: lev_launch(lev_bv_probe_kernel<int8_t>, grid, block, 0, st, a, stride, nsample); break;
         }
-        lev_prof_end(LEV_PROF_BV_UID, st);
+        lev_prof_end(LEV_PROF_BV_PROBE, st);
         const int rc = lev_check_cuda("lev_bv_probe_kernel");
         if (rc) return rc;
     }
-#if LEV_BVF_DYNAMIC
-    if (!a.check_state && cudaMemsetAsync(a.ref_uid, 0, sizeof(int), st) != cudaSuccess) return lev_check_cuda("memset");
-#endif
+    if (!a.check_state && cudaMemsetAsync(a.counter, 0, sizeof(int), st) != cudaSuccess) return lev_check_cuda("memset");
 #ifndef B200LEV_EMU
     if (after_probe != nullptr && cudaEventRecord((cudaEvent_t)after_probe, st) != cudaSuccess)
         return lev_check_cuda("cudaEventRecord");
@@ -670,7 +644,8 @@ int lev_bvfused_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st, void
     switch (elem_bytes) {
         case 8: lev_bvf_launch_t<int64_t>(a, st); break;
         case 4: lev_bvf_launch_t<int32_t>(a, st); break;
-        default: lev_bvf_launch_t<int16_t>(a, st); break;
+        case 2: lev_bvf_launch_t<int16_t>(a, st); break;
+        default: lev_bvf_launch_t<int8_t>(a, st); break;
     }
     lev_prof_end(LEV_PROF_BV_DP, st);
     return lev_check_cuda("lev_bv_fused_kernel");

@@ -439,7 +439,7 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
 bool lev_bvshort_supports(int elem_bytes, int64_t R) {
     const char* e = getenv("B200LEV_BV_SHORT");
     if (e != nullptr && atoi(e) == 0) return false;
-    return R >= 1 && R <= 64 && (elem_bytes == 8 || elem_bytes == 4 || elem_bytes == 2);
+    return R >= 1 && R <= 64 && (elem_bytes == 8 || elem_bytes == 4 || elem_bytes == 2 || elem_bytes == 1);
 }
 
 template <typename TT, int W>
@@ -462,7 +462,8 @@ int lev_bvshort_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st) {
     switch (elem_bytes) {
         case 8: two ? lev_bvs_launch_w<int64_t, 2>(a, st) : lev_bvs_launch_w<int64_t, 1>(a, st); break;
         case 4: two ? lev_bvs_launch_w<int32_t, 2>(a, st) : lev_bvs_launch_w<int32_t, 1>(a, st); break;
-        default: two ? lev_bvs_launch_w<int16_t, 2>(a, st) : lev_bvs_launch_w<int16_t, 1>(a, st); break;
+        case 2: two ? lev_bvs_launch_w<int16_t, 2>(a, st) : lev_bvs_launch_w<int16_t, 1>(a, st); break;
+        default: two ? lev_bvs_launch_w<int8_t, 2>(a, st) : lev_bvs_launch_w<int8_t, 1>(a, st); break;
     }
     lev_prof_end(LEV_PROF_BV_DP, st);
     return lev_check_cuda("lev_bv_short_kernel");

@@ -52,9 +52,8 @@ struct LevLayout {
     int64_t Hr, Hr16;
     size_t off_raw;
     size_t off_uid, off_dtok, off_ndist, off_dbits;
-    // bit-vector path (lev_bitvec.cu): 16-byte uid chunks [ceil(R/16)][P]; the hypothesis
-    // chunks [ceil(H/16)][P] reuse the packed-hypothesis region, which that path leaves idle
-    size_t off_bv_ref;
+    // bit-vector path (lev_bitvec.cu; final and prefix modes, R <= 128): Kb's block counter
+    size_t off_bv_counter;
     // pack kernel, few long sequences: [N first-eos words][ceil(N / 32) tickets] per side
     size_t off_split_ref, off_split_hyp;
     size_t bytes;
@@ -96,7 +95,7 @@ static inline LevLayout lev_layout(const b200lev_tokens_t* ref, const b200lev_to
     L.Hr = lev_round_up(L.H + 1, 4);
     L.Hr16 = lev_round_up(L.H + 1, 8);
     L.off_raw = (kind == 2) ? take(sizeof(int32_t) * (size_t)L.P * L.Hr) : 0;
-    L.off_bv_ref = (kind != 1 && L.R <= 128) ? take((size_t)L.P * (size_t)lev_round_up(L.R > 0 ? L.R : 1, 16)) : 0;
+    L.off_bv_counter = (kind != 1 && L.R <= 128) ? take(sizeof(int32_t)) : 0;
     L.off_uid = L.off_dtok = L.off_ndist = L.off_dbits = 0;
     if (for_completion) {
         L.off_uid = take(sizeof(int32_t) * (size_t)L.Nref * L.Rp);
@@ -188,7 +187,7 @@ __device__ __forceinline__ bool lev_mask16_takes(const LevParams& p, int pair) {
 // optional per-kernel timing (b200lev_profile): CUDA events recorded on the launch stream
 // around each phase; slots of b200lev_profile_read()
 enum LevProfSlot { LEV_PROF_PACK_REF = 0, LEV_PROF_PACK_HYP, LEV_PROF_SORT, LEV_PROF_DP,
-                   LEV_PROF_FINALIZE, LEV_PROF_STANDBY, LEV_PROF_BV_UID, LEV_PROF_BV_DP,
+                   LEV_PROF_FINALIZE, LEV_PROF_STANDBY, LEV_PROF_BV_PROBE, LEV_PROF_BV_DP,
                    LEV_PROF_COMP_UID, LEV_PROF_COMP_FILL, LEV_PROF_ERR_SUM, LEV_PROF_MASK16,
                    LEV_PROF_NSLOTS };
 void lev_prof_begin(int slot, cudaStream_t st);
@@ -213,11 +212,11 @@ int lev_launch_cta(const LevParams& p, int mode, bool count_mode, bool float_pat
 // pack time), else 0
 int lev_group_eligible(int64_t R, int64_t H, int64_t P);
 // Device-side choice between the bit-vector path and the wavefront path (no host round trip).
-// When the shapes and costs admit the bit-vector kernels they are enqueued FIRST: the uid
-// kernel finds out whether every block of 32 consecutive pairs holds at most 4 runs of
-// identical references (n-best batches do) and vetoes through state[3] otherwise; every
+// When the shapes and costs admit the n-best bit-vector kernel it is enqueued FIRST: its probe
+// looks at a sample of the blocks of 32 consecutive pairs for more than 4 runs of identical
+// references (n-best batches have at most 4) and vetoes through state[3] if it finds one; every
 // kernel of the wavefront path, enqueued behind, then starts with lev_bv_took() and exits at
-// once if the work is already done (and the bit-vector DP kernel with the opposite test).
+// once if the work is already done (and the bit-vector kernel with the opposite test).
 __device__ __forceinline__ bool lev_bv_took(const int* state) {
     return *reinterpret_cast<const volatile int*>(state + 3) == 0;
 }
@@ -227,9 +226,9 @@ bool lev_bitvec_eligible(const b200lev_tokens_t* ref, const b200lev_tokens_t* hy
                          int64_t out_sn, int ref_group, bool* short_form, bool* grouped);
 int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                       const b200lev_opts_t* o, int mode, float mult, int32_t* ref_len,
-                      int32_t* hyp_len, void* uid_ref, void* uid_hyp, void* lead,
-                      int32_t* state, int32_t* flags, float* out, int64_t out_si, int Hout,
-                      cudaStream_t st, void* after_uid, bool short_form, double* acc);
+                      int32_t* hyp_len, int* counter, int32_t* state, int32_t* flags, float* out,
+                      int64_t out_si, int Hout, cudaStream_t st, void* after_probe, bool short_form,
+                      double* acc);
 // 0: off, 1: forced (tests; runs whatever the references look like), 2: device-selected
 int lev_bitvec_mode();
 int lev_launch_uid(const b200lev_tokens_t* ref, const int32_t* packed, const int* state,

@@ -636,15 +636,14 @@ int lev_launch_group(const LevParams& p, int mode, bool count_mode, cudaStream_t
                    (int64_t)maxc * (p.R + p.H + 2) < LEVG_BIG16)
                       ? 1
                       : 0;
-    if (const char* e = getenv("B200LEV_GROUP_PACKED16")) geo.allow16 = geo.allow16 && atoi(e);
     LevGroupGeom tmp = geo;
     if (levg_geometry(p, false, &tmp) > 200 * 1024) return 0;
     tmp = geo;
     if (geo.allow16 && levg_geometry(p, true, &tmp) > 200 * 1024) geo.allow16 = 0;
     // bucketing: clear the scatter cursors + meta and the slot table, then scan + scatter
     if (p.bv_check) {
-        // stand-by mode: the slot table shares its bytes with the bit-vector path's tables and
-        // this chain may run beside that path's DP kernel, so the clearing stands by as well
+        // stand-by mode: the clearing stands by as well, so a batch the bit-vector kernel took
+        // costs no memsets here
         lev_launch(lev_group_clear_kernel, dim3(148 * 2), dim3(256), 0, st, p,
                    (int64_t)(p.nbins + 16), (int64_t)(p.P + LEVG_NCLS * 32));
     } else if (cudaMemsetAsync(p.gcursor, 0, sizeof(int) * (size_t)(p.nbins + 16), st) != cudaSuccess ||

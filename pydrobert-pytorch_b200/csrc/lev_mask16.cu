@@ -246,8 +246,6 @@ __global__ void __launch_bounds__(256) lev_mask16_kernel(const LevParams p, cons
 // Enqueues the packed kernel if the call's shapes and costs admit it; returns 1 then (the caller
 // sets LevParams::mask16 for the lev_warp_kernel launch behind it), 0 if not, < 0 on errors.
 int lev_launch_mask16(const LevParams& p, bool float_path, cudaStream_t st) {
-    if (const char* e = getenv("B200LEV_MASK16"))
-        if (atoi(e) == 0) return 0;
     // (few pairs: a warp per pair on lev_warp_kernel finishes sooner than half as many warps here)
     int64_t min_pairs = 2048;
     if (const char* e = getenv("B200LEV_MASK16_MIN_PAIRS")) min_pairs = atoll(e);
@@ -263,10 +261,6 @@ int lev_launch_mask16(const LevParams& p, bool float_path, cudaStream_t st) {
     if (per_warp > budget) return 0;
     int wpc = (int)(budget / per_warp);
     if (wpc > 4) wpc = 4;  // small CTAs: a batch is often a single wave, and whole CTAs are what the SMs share out
-    if (const char* e = getenv("B200LEV_MASK16_WPC")) {  // tuning: warps per CTA
-        const int w = atoi(e);
-        if (w >= 1 && w < wpc) wpc = w;
-    }
     const size_t smem = per_warp * wpc;
     const int64_t nduo = ((int64_t)p.P + 1) / 2;
     int64_t blocks = (nduo + wpc - 1) / wpc;

@@ -21,7 +21,7 @@ bench)
 ncu)
   timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 80 --csv \
       --log-file $OUT/launches.csv python bench.py --steps 3 --warmup 3 --no-cpu-baseline > $OUT/ncu_launch.log 2>&1
-  timeout 900 ncu --set full --clock-control none --import-source on -k regex:${NCU_KERNEL:-lev_bv_uid_kernel} -s ${NCU_SKIP:-5} -c 1 \
+  timeout 900 ncu --set full --clock-control none --import-source on -k regex:${NCU_KERNEL:-lev_bv_fused_kernel} -s ${NCU_SKIP:-5} -c 1 \
       -f -o $OUT/prof_dp python bench.py --steps 3 --warmup 3 --no-cpu-baseline > $OUT/ncu_full.log 2>&1
   ls -la $OUT ;;
 esac

@@ -14,7 +14,7 @@ cap fused lev_bv_fused_kernel 3 --config 2
 cap short_cfg4 lev_bv_short_kernel 3 --config 4
 cap short_cfg1 lev_bv_short_kernel 3 --config 1
 cap mask16 lev_mask16_kernel 2 --config 3
-B200LEV_MASK16=0 cap mask lev_warp_kernel 2 --config 3
+B200LEV_MASK16_MIN_PAIRS=2147483648 cap mask lev_warp_kernel 2 --config 3
 cap fill lev_completion_fill 2 --config 3
 cap uid lev_uid_kernel 2 --config 3
 cap cta lev_cta_kernel 2 --config 5

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """minimum_error_rate_loss forward + backward on the cfg2 shapes (64 and 16 384 utterances x 8
-samples, T = 100): ms per call.  B200LEV_BV_GROUPED=0 = the device-selected path of round 2a."""
+samples, T = 100): ms per call.  The call declares its references shared, so the fused
+bit-vector kernel takes it without a probe."""
 import os
 import sys
 

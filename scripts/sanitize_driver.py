@@ -57,8 +57,7 @@ def nbest_case(what):
          O.prefix_error_rates(rx, h, eos=0), what)
 
 
-which = sys.argv[1:] or ["warp", "group", "cta", "bitvec2", "fused", "short", "completion", "mask16", "loss", "seqlp",
-                         "ragged"]
+which = sys.argv[1:] or ["warp", "group", "cta", "fused", "short", "completion", "mask16", "loss", "seqlp", "ragged"]
 if "warp" in which:  # K1: warp per pair (lev_dp.cu), integer and float costs
     run({"B200LEV_BITVEC": "0", "B200LEV_CTA_KERNEL": "0"}, lambda: prefix_case(70, 80, 9, 7, "K1 warp kernel"))
     run({"B200LEV_BITVEC": "0"}, lambda: prefix_case(40, 45, 5, 7, "K1 float costs", ins_cost=0.7, del_cost=1.1, sub_cost=1.3)
@@ -69,10 +68,7 @@ if "cta" in which:  # K2: CTA per pair, TMA-staged tokens, inter-warp progress f
     run({"B200LEV_BITVEC": "0", "B200LEV_CTA_KERNEL": "1"}, lambda: prefix_case(700, 650, 6, 30, "K2 CTA kernel"))
     run({"B200LEV_BITVEC": "0", "B200LEV_CTA_KERNEL": "1"},
         lambda: prefix_case(300, 280, 4, 30, "K2 CTA kernel, costs 3/3/4", ins_cost=3.0, del_cost=3.0, sub_cost=4.0))
-if "bitvec2" in which:  # two-kernel bit-vector form: shared-memory CAS hash tables
-    run({"B200LEV_BITVEC": "1", "B200LEV_BITVEC_MIN_PAIRS": "1", "B200LEV_BV_FUSED": "0"},
-        lambda: nbest_case("bit-vector uid + DP kernels"))
-if "fused" in which:  # fused bit-vector kernel + probe
+if "fused" in which:  # fused bit-vector kernel (shared-memory CAS hash tables) + probe
     run({"B200LEV_BITVEC": "1", "B200LEV_BITVEC_MIN_PAIRS": "1"}, lambda: nbest_case("fused bit-vector kernel"))
     run({"B200LEV_BITVEC_MIN_PAIRS": "1", "B200LEV_GROUP_MIN_PAIRS": "1"},
         lambda: nbest_case("device-selected (probe + fork)"))

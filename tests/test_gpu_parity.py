@@ -345,17 +345,15 @@ def test_group_kernel_vs_oracle(F, dev, shape, costs, monkeypatch):
                                padding=-3, spread=spread, **flags)
 
 
-@pytest.fixture(params=["fused", "two_kernel", "short"])
+@pytest.fixture(params=["fused", "short"])
 def bv_form(request, monkeypatch):
-    """The forms of the unit-cost bit-vector path: the fused kernel (lev_bvfused.cu, the default
-    for R > 64), the uid pre-pass + DP pair it replaced (lev_bitvec.cu, B200LEV_BV_FUSED=0), and
-    the lane-per-pair short-reference kernel (lev_bvshort.cu, R <= 64; larger shapes of a
-    "short" run fall through to the fused kernel)."""
+    """The two kernels of the unit-cost bit-vector path: the fused kernel (lev_bvfused.cu, the
+    default for R > 64, here for every R) and the lane-per-pair short-reference kernel
+    (lev_bvshort.cu, R <= 64; larger shapes of a "short" run fall through to the fused kernel)."""
     if request.param == "short":
         monkeypatch.setenv("B200LEV_BVSHORT_MIN_PAIRS", "1")
     else:
         monkeypatch.setenv("B200LEV_BV_SHORT", "0")
-        monkeypatch.setenv("B200LEV_BV_FUSED", "1" if request.param == "fused" else "0")
     return request.param
 
 
@@ -581,21 +579,21 @@ def test_bench_batch_all_dp_paths_agree(F, dev, monkeypatch):
 
 
 def test_device_selected_fork_ordering(F, dev, monkeypatch):
-    """The stand-by chain runs on a side stream beside the bit-vector DP kernel: back-to-back
+    """The stand-by chain runs on a side stream beside the bit-vector kernel: back-to-back
     calls on a non-default stream, alternating batches the bit-vector kernels take (n-best) and
     veto (unrelated references), no synchronisation in between -- every result equals the
-    single-stream (B200LEV_FORK=0) result of the same batch."""
+    wavefront kernels' (B200LEV_BITVEC=0) result of the same batch on the default stream."""
     import bench
 
     ref_np, hyp_np, _ = bench.make_batch(1024, seed=5)
     hyp = torch.from_numpy(hyp_np).to(dev)
     shared = torch.from_numpy(np.repeat(ref_np, bench.NBEST, axis=1)).to(dev)
     unrelated = torch.from_numpy(bench.make_batch(1024, seed=6)[1]).to(dev)
-    monkeypatch.setenv("B200LEV_FORK", "0")
+    monkeypatch.setenv("B200LEV_BITVEC", "0")
     want = [F.prefix_error_rates(r, hyp, eos=0, warn=False) for r in (shared, unrelated)]
     want_f = [F.error_rate(r, hyp, eos=0, warn=False) for r in (shared, unrelated)]
     torch.cuda.synchronize()
-    monkeypatch.setenv("B200LEV_FORK", "1")
+    monkeypatch.delenv("B200LEV_BITVEC")
     s = torch.cuda.Stream(dev)
     got = []
     with torch.cuda.stream(s):
@@ -678,7 +676,7 @@ def test_completion_packed_mask_kernel(F, dev, costs, monkeypatch):
 
 def test_grouped_references_take_the_fused_kernel(F, dev, monkeypatch):
     PC.check_grouped_references(F, dev)
-    monkeypatch.setenv("B200LEV_BV_GROUPED", "0")  # the same batches through the wavefront kernels
+    monkeypatch.setenv("B200LEV_BITVEC", "0")  # the same batches through the wavefront kernels
     PC.check_grouped_references(F, dev, seed=1)
 
 

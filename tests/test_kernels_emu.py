@@ -91,7 +91,7 @@ def test_n_best_shared_reference(F):
 
 def test_grouped_references_take_the_fused_kernel(F, monkeypatch):
     PC.check_grouped_references(F, DEV)
-    monkeypatch.setenv("B200LEV_BV_GROUPED", "0")  # the same batches through the wavefront kernels
+    monkeypatch.setenv("B200LEV_BITVEC", "0")  # the same batches through the wavefront kernels
     PC.check_grouped_references(F, DEV, seed=1)
 
 
@@ -169,17 +169,15 @@ def test_group_kernel_vs_oracle(F, shape, costs, monkeypatch):
                                padding=-3, spread=spread, **flags)
 
 
-@pytest.fixture(params=["fused", "two_kernel", "short"])
+@pytest.fixture(params=["fused", "short"])
 def bv_form(request, monkeypatch):
-    """The forms of the unit-cost bit-vector path: the fused kernel (lev_bvfused.cu, the default
-    for R > 64), the uid pre-pass + DP pair it replaced (lev_bitvec.cu, B200LEV_BV_FUSED=0), and
-    the lane-per-pair short-reference kernel (lev_bvshort.cu, R <= 64; larger shapes of a
-    "short" run fall through to the fused kernel)."""
+    """The two kernels of the unit-cost bit-vector path: the fused kernel (lev_bvfused.cu, the
+    default for R > 64, here for every R) and the lane-per-pair short-reference kernel
+    (lev_bvshort.cu, R <= 64; larger shapes of a "short" run fall through to the fused kernel)."""
     if request.param == "short":
         monkeypatch.setenv("B200LEV_BVSHORT_MIN_PAIRS", "1")
     else:
         monkeypatch.setenv("B200LEV_BV_SHORT", "0")
-        monkeypatch.setenv("B200LEV_BV_FUSED", "1" if request.param == "fused" else "0")
     return request.param
 
 
