@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define B200LEV_ABI_VERSION 1
+#define B200LEV_ABI_VERSION 2
 
 #define B200LEV_OK 0
 #define B200LEV_ERR_ARG (-1)       /* bad argument (shape, stride, dtype, NULL) */
@@ -82,9 +82,8 @@ int b200lev_device_count(void);
 
 /* Scratch bytes needed by the calls below for these shapes (packed tokens, lengths,
  * bucketing tables).  kind: B200LEV_WS_FINAL for b200lev_final*, B200LEV_WS_PREFIX for
- * b200lev_prefix* (adds the raw prefix rows), B200LEV_WS_COMPLETION for the completion
- * calls (adds the distinct-token tables and bitmaps).  b200lev_pack may be given the
- * largest of the kinds that will follow it. */
+ * b200lev_prefix (adds the raw prefix rows), B200LEV_WS_COMPLETION for the completion
+ * calls (adds the distinct-token tables and bitmaps). */
 #define B200LEV_WS_FINAL 0
 #define B200LEV_WS_COMPLETION 1
 #define B200LEV_WS_PREFIX 2
@@ -108,26 +107,6 @@ int b200lev_prefix(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                    const b200lev_opts_t *opts, float *out, int64_t out_stride_i,
                    int64_t out_stride_n, void *workspace, size_t workspace_bytes,
                    int32_t *flags, void *stream);
-
-/*
- * The two halves of b200lev_final / b200lev_prefix, exposed separately so that a caller
- * can keep tokens packed across calls or time the DP kernel on its own (bench.py):
- *   b200lev_pack            K0 only: lengths (SM:137-143, 195-228) + pair-major int32
- *                           token tables into the workspace;
- *   b200lev_prefix_packed   the DP + prefix epilogue on a workspace b200lev_pack filled
- *                           (ref/hyp are read for their shapes only);
- *   b200lev_final_packed    likewise for the final value.
- */
-int b200lev_pack(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
-                 const b200lev_opts_t *opts, void *workspace, size_t workspace_bytes,
-                 int32_t *flags, void *stream);
-int b200lev_prefix_packed(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
-                          const b200lev_opts_t *opts, float *out, int64_t out_stride_i,
-                          int64_t out_stride_n, void *workspace, size_t workspace_bytes,
-                          int32_t *flags, void *stream);
-int b200lev_final_packed(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
-                         const b200lev_opts_t *opts, float *out, void *workspace,
-                         size_t workspace_bytes, int32_t *flags, void *stream);
 
 /*
  * optimal_completion (SM:464-517), two phases around the one host read the
@@ -196,28 +175,14 @@ int b200lev_mwer_backward(const float *er, const void *log_probs, int32_t dtype,
                           int64_t M, int64_t lp_sn, int64_t lp_sm, int32_t sub_avg,
                           int32_t reduction, const void *grad_out, void *grad, void *stream);
 
-/*
- * Bulk scoring accumulators (command_line.py:1135-1147 pattern): acc[0] += sum(er),
- * acc[1] += sum(ref_lens), acc[2] += number of pairs; double precision on device so
- * one all-reduce(sum) of 24 bytes finishes a multi-GPU job.  `ref_lens` is the int32
- * length table the workspace of the last b200lev_final call holds (see
- * b200lev_workspace_ref_lens).
- */
-int b200lev_err_sum(const float *er, const int32_t *ref_lens, int64_t P, int32_t ref_group,
-                    double *acc, void *stream);
-
-/* b200lev_final followed by b200lev_err_sum in one call: `out` as b200lev_final, and
- * acc[0] += sum(out), acc[1] += sum over pairs of the reference length, acc[2] += #pairs (fp64,
- * device).  Where the short-reference kernel serves the call the sums are accumulated inside it
- * (no second kernel): the per-batch body of command_line.py:1124-1147. */
+/* b200lev_final and the bulk-scoring totals in one call: `out` as b200lev_final, and
+ * acc[0] += sum(out), acc[1] += sum over pairs of the reference length, acc[2] += #pairs (fp64
+ * on the device, so one all-reduce(sum) of 24 bytes finishes a multi-GPU job).  Where the
+ * short-reference kernel serves the call the sums are accumulated inside it (no second kernel):
+ * the per-batch body of command_line.py:1124-1147. */
 int b200lev_final_sums(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                        const b200lev_opts_t *opts, float *out, void *workspace,
                        size_t workspace_bytes, int32_t *flags, double *acc, void *stream);
-/* pointers into a workspace laid out by b200lev_final/prefix/completion_count */
-const int32_t *b200lev_workspace_ref_lens(const b200lev_tokens_t *ref,
-                                          const b200lev_tokens_t *hyp, const void *workspace);
-const int32_t *b200lev_workspace_hyp_lens(const b200lev_tokens_t *ref,
-                                          const b200lev_tokens_t *hyp, const void *workspace);
 
 /* fill_after_eos (SM:30-42), the scan: tokens is a contiguous int64 (outer, T, inner)
  * view; mask[o, t, i] = 1 iff an eos occurs at some t' < t.  The broadcasted fill of

@@ -49,10 +49,6 @@ SIGNATURES = {
     "b200lev_workspace_bytes": (c_sz, [_PT, _PT, c_i32, c_i32]),
     "b200lev_final": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_prefix": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_i64, c_i64, c_vp, c_sz, c_vp, c_vp]),
-    "b200lev_pack": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_sz, c_vp, c_vp]),
-    "b200lev_prefix_packed": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_i64, c_i64, c_vp, c_sz, c_vp,
-                                             c_vp]),
-    "b200lev_final_packed": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_completion_count": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_sz, c_vp, c_vp, c_vp]),
     "b200lev_completion_fill": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_sz, c_i64, c_vp, c_i64,
                                                c_i64, c_vp]),
@@ -67,9 +63,6 @@ SIGNATURES = {
     "b200lev_mwer_backward": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_i32,
                                              c_i32, c_vp, c_vp, c_vp]),
     "b200lev_final_sums": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp, c_vp]),
-    "b200lev_err_sum": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp]),
-    "b200lev_workspace_ref_lens": (c_vp, [_PT, _PT, c_vp]),
-    "b200lev_workspace_hyp_lens": (c_vp, [_PT, _PT, c_vp]),
     "b200lev_after_eos_mask": (ctypes.c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp]),
     "b200lev_ragged_to_padded": (ctypes.c_int, [c_vp, c_i32, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64,
                                                 c_vp, c_vp]),
@@ -116,7 +109,7 @@ def lib() -> ctypes.CDLL:
                 "b200lev has no CPU fallback."
             )
         _lib = _bind(ctypes.CDLL(LIB_PATH))
-        if _lib.b200lev_abi_version() != 1:
+        if _lib.b200lev_abi_version() != 2:
             raise B200LevError("libb200lev.so ABI version mismatch")
     return _lib
 

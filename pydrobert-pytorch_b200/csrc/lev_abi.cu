@@ -147,15 +147,29 @@ static inline char* lev_ws_base(const void* ws) {
     return (char*)(((uintptr_t)ws + 127) & ~(uintptr_t)127);
 }
 
-extern "C" const int32_t* b200lev_workspace_ref_lens(const b200lev_tokens_t* ref,
-                                                     const b200lev_tokens_t* hyp, const void* ws) {
-    LevLayout L = lev_layout(ref, hyp, 0, 0);
-    return (const int32_t*)(lev_ws_base(ws) + L.off_ref_len);
-}
-extern "C" const int32_t* b200lev_workspace_hyp_lens(const b200lev_tokens_t* ref,
-                                                     const b200lev_tokens_t* hyp, const void* ws) {
-    LevLayout L = lev_layout(ref, hyp, 0, 0);
-    return (const int32_t*)(lev_ws_base(ws) + L.off_hyp_len);
+// The argument prologue of the string-matching entry points: checks the token views and the
+// options, lays out the workspace for `kind` and checks the caller's buffers.  Returns LEV_EMPTY
+// when the call has nothing to write (no pairs, no output rows, or `inner` <= 0), and NULL
+// buffers are then fine; else B200LEV_OK with *L filled, or an error status (`null_status` for a
+// NULL `out` or `ws`).
+static constexpr int LEV_EMPTY = 1;
+static int lev_begin(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                     const b200lev_opts_t* o, int kind, const void* out, const void* ws,
+                     size_t ws_bytes, LevLayout* L, int64_t inner = 1,
+                     int null_status = B200LEV_ERR_ARG) {
+    const int rc = lev_check_tokens(ref, hyp, o);
+    if (rc) return rc;
+    *L = lev_layout(ref, hyp, kind, kind == B200LEV_WS_FINAL ? 0 : o->exclude_last);
+    if (hyp->N == 0 || L->Hout <= 0 || inner <= 0) return LEV_EMPTY;
+    if (!out || !ws) {
+        lev_set_error("NULL output or workspace");
+        return null_status;
+    }
+    if (ws_bytes < L->bytes + 128) {
+        lev_set_error("workspace too small: %zu < %zu", ws_bytes, L->bytes + 128);
+        return B200LEV_ERR_WORKSPACE;
+    }
+    return B200LEV_OK;
 }
 
 // Fills the cost fields of `p`.  Returns count_mode / float_path through the out-params.
@@ -185,47 +199,17 @@ static void lev_classify_costs(const b200lev_opts_t* o, int64_t R, int64_t H, Le
     *float_path = !integral;
 }
 
-// pack both token tensors into the workspace and fill the common fields of `p`
-static int lev_prepare(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+// the fields of `p` every mode shares: workspace tables, the caller's tensors, options, costs
+static void lev_params(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                        const b200lev_opts_t* o, const LevLayout& L, char* ws, int32_t* flags,
-                       cudaStream_t st, LevParams* p, bool do_pack = true, int bv_check = 0) {
-    int32_t* ref_tok = (int32_t*)(ws + L.off_ref_tok);
-    int32_t* hyp_tok = (int32_t*)(ws + L.off_hyp_tok);
-    int32_t* ref_len = (int32_t*)(ws + L.off_ref_len);
-    int32_t* hyp_len = (int32_t*)(ws + L.off_hyp_len);
-    // K0 leaves what the DP kernels need to know about the tokens (wider than int32?
-    // value range) in 4 state words of the workspace; the caller's flags get the same
-    // warning bits
-    int32_t* state = (int32_t*)(ws + L.off_flags);
-    if (do_pack) {
-        // the group kernel's (class, length) histogram is built by the hypothesis pass
-        // whenever the shapes make that kernel eligible (lev_group.cu decides later)
-        const int G = lev_group_eligible(L.R, L.H, L.P);
-        const size_t clear = sizeof(int32_t) * (size_t)(4 + (G ? L.nbins : 0));
-        // (with bv_check the bit-vector launcher cleared them before its kernels ran)
-        if (!bv_check && cudaMemsetAsync(state, 0, clear, st) != cudaSuccess) return lev_check_cuda("memset");
-        lev_prof_begin(LEV_PROF_PACK_REF, st);
-        int rc = lev_launch_pack(ref, o->has_eos, o->eos, o->include_eos, ref_tok, L.Rp, nullptr, 0,
-                                 ref_len, flags, state, B200LEV_FLAG_REF_NO_EOS, nullptr, 1, 0,
-                                 nullptr, bv_check, st, (int32_t*)(ws + L.off_split_ref));
-        lev_prof_end(LEV_PROF_PACK_REF, st);
-        if (rc) return rc;
-        lev_prof_begin(LEV_PROF_PACK_HYP, st);
-        rc = lev_launch_pack(hyp, o->has_eos, o->eos, o->include_eos, hyp_tok, L.Hp,
-                             (uint16_t*)(ws + L.off_hyp_tok16), L.Hp16, hyp_len, flags, state,
-                             B200LEV_FLAG_HYP_NO_EOS, ref_len, o->ref_group, G,
-                             G ? (int*)(ws + L.off_ghist) : nullptr, bv_check, st,
-                             (int32_t*)(ws + L.off_split_hyp));
-        lev_prof_end(LEV_PROF_PACK_HYP, st);
-        if (rc) return rc;
-    }
+                       LevParams* p, bool* count_mode, bool* float_path) {
     memset(p, 0, sizeof(*p));
-    p->ref_tok = ref_tok;
-    p->hyp_tok = hyp_tok;
+    p->ref_tok = (const int32_t*)(ws + L.off_ref_tok);
+    p->hyp_tok = (const int32_t*)(ws + L.off_hyp_tok);
     p->hyp_tok16 = (const uint16_t*)(ws + L.off_hyp_tok16);
     p->Hp16 = L.Hp16;
-    p->ref_len = ref_len;
-    p->hyp_len = hyp_len;
+    p->ref_len = (const int32_t*)(ws + L.off_ref_len);
+    p->hyp_len = (const int32_t*)(ws + L.off_hyp_len);
     p->Rp = L.Rp;
     p->Hp = L.Hp;
     p->R = (int)L.R;
@@ -236,8 +220,7 @@ static int lev_prepare(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     p->exclude_last = o->exclude_last;
     p->padding = (float)o->padding;
     p->flags = flags;
-    p->wide_flag = state;
-    p->bv_check = bv_check;
+    p->wide_flag = (const int*)(ws + L.off_flags);
     p->ref_raw = ref->data;
     p->hyp_raw = hyp->data;
     p->ref_st = ref->stride_t;
@@ -256,7 +239,37 @@ static int lev_prepare(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     p->raw16 = (unsigned short*)p->raw32;
     p->Hr = L.Hr;
     p->Hr16 = L.Hr16;
-    return B200LEV_OK;
+    lev_classify_costs(o, L.R, L.H, p, count_mode, float_path);
+}
+
+// K0: pack both token tensors into the workspace.  It leaves what the DP kernels need to know
+// about the tokens (wider than int32? value range) in 4 state words of the workspace; the
+// caller's flags get the same warning bits.  With bv_check the bit-vector launcher has cleared
+// the state words before its kernels ran.
+static int lev_pack_tokens(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                           const b200lev_opts_t* o, const LevLayout& L, char* ws, int32_t* flags,
+                           int bv_check, cudaStream_t st) {
+    int32_t* ref_len = (int32_t*)(ws + L.off_ref_len);
+    int32_t* state = (int32_t*)(ws + L.off_flags);
+    // the group kernel's (class, length) histogram is built by the hypothesis pass whenever the
+    // shapes make that kernel eligible (lev_group.cu decides later)
+    const int G = lev_group_eligible(L.R, L.H, L.P);
+    const size_t clear = sizeof(int32_t) * (size_t)(4 + (G ? L.nbins : 0));
+    if (!bv_check && cudaMemsetAsync(state, 0, clear, st) != cudaSuccess) return lev_check_cuda("memset");
+    lev_prof_begin(LEV_PROF_PACK_REF, st);
+    int rc = lev_launch_pack(ref, o->has_eos, o->eos, o->include_eos, (int32_t*)(ws + L.off_ref_tok),
+                             L.Rp, nullptr, 0, ref_len, flags, state, B200LEV_FLAG_REF_NO_EOS, nullptr,
+                             1, 0, nullptr, bv_check, st, (int32_t*)(ws + L.off_split_ref));
+    lev_prof_end(LEV_PROF_PACK_REF, st);
+    if (rc) return rc;
+    lev_prof_begin(LEV_PROF_PACK_HYP, st);
+    rc = lev_launch_pack(hyp, o->has_eos, o->eos, o->include_eos, (int32_t*)(ws + L.off_hyp_tok), L.Hp,
+                         (uint16_t*)(ws + L.off_hyp_tok16), L.Hp16, (int32_t*)(ws + L.off_hyp_len),
+                         flags, state, B200LEV_FLAG_HYP_NO_EOS, ref_len, o->ref_group, G,
+                         G ? (int*)(ws + L.off_ghist) : nullptr, bv_check, st,
+                         (int32_t*)(ws + L.off_split_hyp));
+    lev_prof_end(LEV_PROF_PACK_HYP, st);
+    return rc;
 }
 
 // Device-selected mode forks: once the probe has finished the veto is final, so the wavefront
@@ -314,105 +327,62 @@ static cudaStream_t lev_fork_begin(const LevFork&, bool) { return nullptr; }
 static int lev_fork_join(const LevFork&, cudaStream_t) { return B200LEV_OK; }
 #endif
 
-// Unit costs, short references, sequence-first tensors: the bit-vector path (lev_bitvec.cu)
-// takes the whole call -- lengths, warnings and DP -- straight from the raw tokens.
-// Returns 0 if it does not apply, 1 if it ran unconditionally (forced mode: the call is
-// done), 2 if its kernels were enqueued in device-selected mode (the caller goes on to
-// enqueue the wavefront path with bv_check set; the state words are already cleared),
-// < 0 on error.
-static int lev_try_bitvec(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                          const b200lev_opts_t* o, const LevLayout& L, char* ws, int32_t* flags,
-                          cudaStream_t st, int mode, float* out, int64_t out_si, int64_t out_sn,
-                          int Hout, LevFork* fork, bool* forked, double* acc = nullptr,
-                          bool* sums_done = nullptr) {
-    *forked = false;
-    if (mode == LEV_MODE_MASK || L.R > 128) return 0;  // (lev_layout has no block counter for these)
-    LevParams tmp;
-    memset(&tmp, 0, sizeof(tmp));
-    bool cm, fp;
-    lev_classify_costs(o, L.R, L.H, &tmp, &cm, &fp);
-    bool short_form = false, grouped = false;
-    if (!lev_bitvec_eligible(ref, hyp, mode, cm, fp, tmp.ins_i, tmp.del_i, tmp.sub_i, out_sn, o->ref_group,
-                             &short_form, &grouped))
-        return 0;
-    // the short-reference kernel takes any batch, the fused kernel any batch whose references the
-    // caller declared shared: nothing to select on the device, no chain behind them
-    const bool forced = lev_bitvec_mode() == 1 || short_form || grouped;
-    int32_t* state = (int32_t*)(ws + L.off_flags);
-    if (!forced) {
-        // device-selected: only where the wavefront fallback is the group path, whose kernels
-        // know how to stand by; the state words are cleared here, once, for both paths
-        const int G = lev_group_eligible(L.R, L.H, L.P);
-        if (G == 0) return 0;
-        const size_t clear = sizeof(int32_t) * (size_t)(4 + L.nbins);
-        if (cudaMemsetAsync(state, 0, clear, st) != cudaSuccess) return lev_check_cuda("memset");
-    }
-    *forked = !forced && lev_fork_get(fork);
-    const int rc = lev_bitvec_launch(ref, hyp, o, mode, tmp.mult, (int32_t*)(ws + L.off_ref_len),
-                                     (int32_t*)(ws + L.off_hyp_len), (int*)(ws + L.off_bv_counter),
-                                     forced ? nullptr : state, flags, out, out_si, Hout, st,
-                                     *forked ? fork->after_probe : nullptr, short_form, acc);
-    if (rc) return rc;
-    if (sums_done != nullptr) *sums_done = short_form && mode == LEV_MODE_FINAL && acc != nullptr;
-    return forced ? 1 : 2;
-}
-
-extern "C" int b200lev_err_sum(const float* er, const int32_t* ref_lens, int64_t P, int32_t ref_group,
-                               double* acc, void* stream);
-
-static int lev_final_impl(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                          const b200lev_opts_t* opts, float* out, void* workspace,
-                          size_t workspace_bytes, int32_t* flags, void* stream, bool do_pack,
-                          double* acc = nullptr) {
-    int rc = lev_check_tokens(ref, hyp, opts);
-    if (rc) return rc;
-    if (hyp->N == 0) return B200LEV_OK;
-    if (!out || !workspace) {
-        lev_set_error("NULL output/workspace");
-        return B200LEV_ERR_ARG;
-    }
-    const LevLayout L = lev_layout(ref, hyp, 0, 0);
-    if (workspace_bytes < L.bytes + 128) {
-        lev_set_error("workspace too small: %zu < %zu", workspace_bytes, L.bytes + 128);
-        return B200LEV_ERR_WORKSPACE;
-    }
+// b200lev_final / b200lev_final_sums (FINAL; `acc` NULL or the sums) and b200lev_prefix (PREFIX,
+// output strides).  Unit costs, short references, sequence-first tensors: the bit-vector path
+// (lev_bitvec.cu) takes the whole call -- lengths, warnings and DP -- straight from the raw
+// tokens.  Otherwise, or behind its probe when the device selects, K0 and the wavefront DP run.
+static int lev_string_match(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                            const b200lev_opts_t* opts, int mode, float* out, int64_t out_si,
+                            int64_t out_sn, void* workspace, size_t workspace_bytes,
+                            int32_t* flags, double* acc, void* stream) {
+    const bool final = mode == LEV_MODE_FINAL;
+    LevLayout L;
+    int rc = lev_begin(ref, hyp, opts, final ? B200LEV_WS_FINAL : B200LEV_WS_PREFIX, out, workspace,
+                       workspace_bytes, &L);
+    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
     cudaStream_t st = (cudaStream_t)stream;
-    LevParams p;
+    char* ws = lev_ws_base(workspace);
     b200lev_opts_t o = *opts;
-    o.exclude_last = 0;  // SM:165
-    int bv = 0;
-    LevFork fork;
-    bool forked = false;
+    if (final) o.exclude_last = 0;  // SM:165
+    LevParams p;
+    bool cm, fp;
+    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
+    p.out = out;
+    if (!final) {
+        p.out_si = out_si;
+        p.out_sn = out_sn;
+        p.Hout = (int)L.Hout;
+    }
     std::lock_guard<std::mutex> fork_lock(g_fork_mu);
-    if (do_pack) {
-        bool sums_done = false;
-        bv = lev_try_bitvec(ref, hyp, &o, L, lev_ws_base(workspace), flags, st, LEV_MODE_FINAL, out,
-                            0, 1, 0, &fork, &forked, acc, &sums_done);
-        if (bv < 0) return bv;
-        if (bv == 1) {
-            if (acc != nullptr && !sums_done)
-                return b200lev_err_sum(out, (const int32_t*)(lev_ws_base(workspace) + L.off_ref_len), hyp->N,
-                                       o.ref_group, acc, stream);
-            return B200LEV_OK;
+    const LevBvRoute bv = lev_bitvec_route(ref, hyp, mode, p, cm, fp);
+    LevFork fork;
+    const bool forked = bv == LEV_BV_SELECTED && lev_fork_get(&fork);
+    if (bv != LEV_BV_NONE) {
+        rc = lev_bitvec_launch(bv, ref, hyp, &o, mode, L, ws, p, st, forked ? fork.after_probe : nullptr, acc);
+        if (rc) return rc;
+    }
+    if (bv == LEV_BV_NONE || bv == LEV_BV_SELECTED) {
+        cudaStream_t side = lev_fork_begin(fork, forked);
+        cudaStream_t cs = side ? side : st;  // the wavefront chain's stream
+        p.bv_check = bv == LEV_BV_SELECTED;
+        rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, p.bv_check, cs);
+        if (rc == B200LEV_OK) rc = lev_launch_dp(p, mode, cm, fp, cs);
+        if (side) {
+            const int jr = lev_fork_join(fork, st);
+            if (rc == B200LEV_OK) rc = jr;
         }
     }
-    cudaStream_t side = lev_fork_begin(fork, forked && bv == 2);
-    cudaStream_t cs = side ? side : st;  // the wavefront chain's stream
-    rc = lev_prepare(ref, hyp, &o, L, lev_ws_base(workspace), flags, cs, &p, do_pack, bv == 2);
-    if (rc == B200LEV_OK) {
-        bool cm, fp;
-        lev_classify_costs(&o, L.R, L.H, &p, &cm, &fp);
-        p.out = out;
-        rc = lev_launch_dp(p, LEV_MODE_FINAL, cm, fp, cs);
-    }
-    if (side) {
-        const int jr = lev_fork_join(fork, st);
-        if (rc == B200LEV_OK) rc = jr;
-    }
-    if (rc == B200LEV_OK && acc != nullptr)
-        rc = b200lev_err_sum(out, (const int32_t*)(lev_ws_base(workspace) + L.off_ref_len), hyp->N,
-                             o.ref_group, acc, stream);
+    // (Ks accumulates the sums itself)
+    if (rc == B200LEV_OK && acc != nullptr && bv != LEV_BV_SHORT)
+        rc = lev_launch_err_sum(out, p.ref_len, hyp->N, o.ref_group, acc, st);
     return rc;
+}
+
+extern "C" int b200lev_final(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                             const b200lev_opts_t* opts, float* out, void* workspace,
+                             size_t workspace_bytes, int32_t* flags, void* stream) {
+    return lev_string_match(ref, hyp, opts, LEV_MODE_FINAL, out, 0, 0, workspace, workspace_bytes,
+                            flags, nullptr, stream);
 }
 
 extern "C" int b200lev_final_sums(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
@@ -423,130 +393,41 @@ extern "C" int b200lev_final_sums(const b200lev_tokens_t* ref, const b200lev_tok
         return B200LEV_ERR_ARG;
     }
     if (hyp && hyp->N == 0) return B200LEV_OK;
-    return lev_final_impl(ref, hyp, opts, out, workspace, workspace_bytes, flags, stream, true, acc);
-}
-
-extern "C" int b200lev_final(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                             const b200lev_opts_t* opts, float* out, void* workspace,
-                             size_t workspace_bytes, int32_t* flags, void* stream) {
-    return lev_final_impl(ref, hyp, opts, out, workspace, workspace_bytes, flags, stream, true);
-}
-
-extern "C" int b200lev_final_packed(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                                    const b200lev_opts_t* opts, float* out, void* workspace,
-                                    size_t workspace_bytes, int32_t* flags, void* stream) {
-    return lev_final_impl(ref, hyp, opts, out, workspace, workspace_bytes, flags, stream, false);
-}
-
-extern "C" int b200lev_pack(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                            const b200lev_opts_t* opts, void* workspace, size_t workspace_bytes,
-                            int32_t* flags, void* stream) {
-    int rc = lev_check_tokens(ref, hyp, opts);
-    if (rc) return rc;
-    if (hyp->N == 0) return B200LEV_OK;
-    const LevLayout L = lev_layout(ref, hyp, 0, 0);
-    if (!workspace || workspace_bytes < L.bytes + 128) {
-        lev_set_error("workspace too small: %zu < %zu", workspace_bytes, L.bytes + 128);
-        return B200LEV_ERR_WORKSPACE;
-    }
-    LevParams p;
-    return lev_prepare(ref, hyp, opts, L, lev_ws_base(workspace), flags, (cudaStream_t)stream, &p, true);
-}
-
-static int lev_prefix_impl(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                           const b200lev_opts_t* opts, float* out, int64_t out_stride_i,
-                           int64_t out_stride_n, void* workspace, size_t workspace_bytes,
-                           int32_t* flags, void* stream, bool do_pack) {
-    int rc = lev_check_tokens(ref, hyp, opts);
-    if (rc) return rc;
-    const LevLayout L = lev_layout(ref, hyp, 2, opts->exclude_last);
-    if (hyp->N == 0 || L.Hout <= 0) return B200LEV_OK;
-    if (!out || !workspace) {
-        lev_set_error("NULL output/workspace");
-        return B200LEV_ERR_ARG;
-    }
-    if (workspace_bytes < L.bytes + 128) {
-        lev_set_error("workspace too small: %zu < %zu", workspace_bytes, L.bytes + 128);
-        return B200LEV_ERR_WORKSPACE;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    LevParams p;
-    int bv = 0;
-    LevFork fork;
-    bool forked = false;
-    std::lock_guard<std::mutex> fork_lock(g_fork_mu);
-    if (do_pack) {
-        bv = lev_try_bitvec(ref, hyp, opts, L, lev_ws_base(workspace), flags, st, LEV_MODE_PREFIX,
-                            out, out_stride_i, out_stride_n, (int)L.Hout, &fork, &forked);
-        if (bv < 0) return bv;
-        if (bv == 1) return B200LEV_OK;
-    }
-    cudaStream_t side = lev_fork_begin(fork, forked && bv == 2);
-    cudaStream_t cs = side ? side : st;  // the wavefront chain's stream
-    rc = lev_prepare(ref, hyp, opts, L, lev_ws_base(workspace), flags, cs, &p, do_pack, bv == 2);
-    if (rc == B200LEV_OK) {
-        bool cm, fp;
-        lev_classify_costs(opts, L.R, L.H, &p, &cm, &fp);
-        p.out = out;
-        p.out_si = out_stride_i;
-        p.out_sn = out_stride_n;
-        p.Hout = (int)L.Hout;
-        rc = lev_launch_dp(p, LEV_MODE_PREFIX, cm, fp, cs);
-    }
-    if (side) {
-        const int jr = lev_fork_join(fork, st);
-        if (rc == B200LEV_OK) rc = jr;
-    }
-    return rc;
+    return lev_string_match(ref, hyp, opts, LEV_MODE_FINAL, out, 0, 0, workspace, workspace_bytes,
+                            flags, acc, stream);
 }
 
 extern "C" int b200lev_prefix(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                               const b200lev_opts_t* opts, float* out, int64_t out_stride_i,
                               int64_t out_stride_n, void* workspace, size_t workspace_bytes,
                               int32_t* flags, void* stream) {
-    return lev_prefix_impl(ref, hyp, opts, out, out_stride_i, out_stride_n, workspace,
-                           workspace_bytes, flags, stream, true);
-}
-
-extern "C" int b200lev_prefix_packed(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                                     const b200lev_opts_t* opts, float* out, int64_t out_stride_i,
-                                     int64_t out_stride_n, void* workspace, size_t workspace_bytes,
-                                     int32_t* flags, void* stream) {
-    return lev_prefix_impl(ref, hyp, opts, out, out_stride_i, out_stride_n, workspace,
-                           workspace_bytes, flags, stream, false);
+    return lev_string_match(ref, hyp, opts, LEV_MODE_PREFIX, out, out_stride_i, out_stride_n,
+                            workspace, workspace_bytes, flags, nullptr, stream);
 }
 
 extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                                         const b200lev_opts_t* opts, void* workspace,
                                         size_t workspace_bytes, int32_t* umax, int32_t* flags,
                                         void* stream) {
-    int rc = lev_check_tokens(ref, hyp, opts);
-    if (rc) return rc;
-    if (!umax) {
+    LevLayout L;
+    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_COMPLETION, umax, workspace, workspace_bytes, &L);
+    if (rc < 0) return rc;
+    if (!umax) {  // (an empty batch still writes U = 0)
         lev_set_error("NULL umax");
         return B200LEV_ERR_ARG;
     }
     cudaStream_t st = (cudaStream_t)stream;
     if (cudaMemsetAsync(umax, 0, sizeof(int32_t), st) != cudaSuccess) return lev_check_cuda("memset");
-    if (hyp->N == 0) return B200LEV_OK;
-    if (!workspace) {
-        lev_set_error("NULL workspace");
-        return B200LEV_ERR_ARG;
-    }
-    const LevLayout L = lev_layout(ref, hyp, 1, opts->exclude_last);
-    if (workspace_bytes < L.bytes + 128) {
-        lev_set_error("workspace too small: %zu < %zu", workspace_bytes, L.bytes + 128);
-        return B200LEV_ERR_WORKSPACE;
-    }
+    if (rc == LEV_EMPTY) return B200LEV_OK;
     char* ws = lev_ws_base(workspace);
-    LevParams p;
     b200lev_opts_t o = *opts;
     o.return_mistakes = 0;  // SM:479-491: the mask is always taken on the cost row
     o.norm = 0;
-    rc = lev_prepare(ref, hyp, &o, L, ws, flags, st, &p);
-    if (rc) return rc;
+    LevParams p;
     bool cm, fp;
-    lev_classify_costs(&o, L.R, L.H, &p, &cm, &fp);
+    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
+    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
+    if (rc) return rc;
     int32_t* uid = (int32_t*)(ws + L.off_uid);
     int64_t* dtok = (int64_t*)(ws + L.off_dtok);
     int32_t* ndist = (int32_t*)(ws + L.off_ndist);
@@ -568,14 +449,11 @@ extern "C" int b200lev_completion_fill(const b200lev_tokens_t* ref, const b200le
                                        const b200lev_opts_t* opts, const void* workspace,
                                        size_t workspace_bytes, int64_t U, int64_t* out,
                                        int64_t out_stride_i, int64_t out_stride_n, void* stream) {
-    int rc = lev_check_tokens(ref, hyp, opts);
-    if (rc) return rc;
-    if (hyp->N == 0 || U <= 0) return B200LEV_OK;
-    const LevLayout L = lev_layout(ref, hyp, 1, opts->exclude_last);
-    if (!workspace || !out || workspace_bytes < L.bytes + 128) {
-        lev_set_error("bad workspace/output");
-        return B200LEV_ERR_WORKSPACE;
-    }
+    // (a NULL output counts as a bad workspace here)
+    LevLayout L;
+    const int rc = lev_begin(ref, hyp, opts, B200LEV_WS_COMPLETION, out, workspace, workspace_bytes,
+                             &L, U, B200LEV_ERR_WORKSPACE);
+    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
     const char* ws = lev_ws_base(workspace);
     return lev_launch_completion_fill((const uint32_t*)(ws + L.off_dbits),
                                       (const int64_t*)(ws + L.off_dtok), (const int*)(ws + L.off_flags), L.Rp,

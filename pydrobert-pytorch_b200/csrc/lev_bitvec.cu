@@ -11,7 +11,7 @@
 // work with lane = pair straight from the raw sequence-first tokens; K0 (lev_pack.cu) is not
 // needed on this path.
 //
-// Eligibility (lev_bitvec_eligible): unit costs after SM:168-174, final or prefix mode, at most
+// Eligibility (lev_bitvec_route): unit costs after SM:168-174, final or prefix mode, at most
 // 128 reference positions, unit stride along the batch axis of both token tensors and of the
 // prefix output.  Then, per call:
 //
@@ -20,10 +20,10 @@
 //   Kb  lev_bv_fused_kernel (lev_bvfused.cu), R <= 128: per-run hash tables and match masks in
 //       shared memory, built for n-best batches (<= 4 distinct references per 32 pairs).  A call
 //       that declares its references shared (ref_group >= 8) takes it unconditionally; any other
-//       batch of at least B200LEV_BITVEC_MIN_PAIRS pairs is enqueued AHEAD of the wavefront path
-//       and decided on the device: lev_bv_probe_kernel vetoes through state[3] (lev_bv_took,
-//       lev_common.cuh) when a sampled block holds more references than that, and the wavefront
-//       kernels -- which otherwise exit at once -- do the work.
+//       batch of at least B200LEV_BITVEC_MIN_PAIRS pairs whose wavefront path is the group kernel
+//       is enqueued AHEAD of that path and decided on the device: lev_bv_probe_kernel vetoes
+//       through state[3] (lev_bv_took, lev_common.cuh) when a sampled block holds more references
+//       than that, and the wavefront kernels -- which otherwise exit at once -- do the work.
 #include "lev_bitvec.cuh"
 
 // ---------------------------------------------------------------------------------------
@@ -32,7 +32,7 @@
 // B200LEV_BITVEC: 0 = never, 1 = forced (tests: whatever the references look like, multi-pass
 // where a block of 32 pairs holds more than 4 distinct references), default 2 = enqueued ahead
 // of the wavefront path, which it pre-empts on the device when the batch is n-best shaped.
-int lev_bitvec_mode() {
+static int lev_bitvec_mode() {
     const char* e = getenv("B200LEV_BITVEC");
     return e != nullptr ? atoi(e) : 2;
 }
@@ -54,35 +54,34 @@ static int64_t lev_bvshort_min_pairs() {
 // _string.py:1426/1439 -- minimum_error_rate_loss): with 8 or more a block of 32 pairs holds at
 // most 4 - 5 references, which is what the fused kernel's tables are built for, so there is
 // nothing to probe and no stand-by chain to enqueue; such a call is worth it from a few warps on.
-bool lev_bitvec_eligible(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int mode,
-                         bool count_mode, bool float_path, int ins_i, int del_i, int sub_i,
-                         int64_t out_sn, int ref_group, bool* short_form, bool* grouped) {
-    *short_form = false;
-    *grouped = false;
-    if (lev_bitvec_mode() == 0) return false;
-    if (mode != LEV_MODE_FINAL && mode != LEV_MODE_PREFIX) return false;
-    if (count_mode || float_path || ins_i != 1 || del_i != 1 || sub_i != 1) return false;
-    if (ref->T > 128 || ref->T < 1 || hyp->T >= (1 << 20)) return false;
-    if (!lev_bvfused_supports(ref->elem_bytes) || ref->elem_bytes != hyp->elem_bytes) return false;
-    *short_form = lev_bvshort_supports(ref->elem_bytes, ref->T) && hyp->N >= lev_bvshort_min_pairs();
-    *grouped = !*short_form && ref_group >= 8 && hyp->N >= 128;
-    if (!*short_form && !*grouped && hyp->N < lev_bv_min_pairs()) return false;
+LevBvRoute lev_bitvec_route(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int mode,
+                            const LevParams& p, bool count_mode, bool float_path) {
+    const int bv = lev_bitvec_mode();
+    if (bv == 0 || mode == LEV_MODE_MASK) return LEV_BV_NONE;
+    if (count_mode || float_path || p.ins_i != 1 || p.del_i != 1 || p.sub_i != 1) return LEV_BV_NONE;
+    // (lev_layout has a block counter for R <= 128 only)
+    if (ref->T > 128 || ref->T < 1 || hyp->T >= (1 << 20)) return LEV_BV_NONE;
+    if (!lev_bvfused_supports(ref->elem_bytes) || ref->elem_bytes != hyp->elem_bytes) return LEV_BV_NONE;
+    const bool short_form = lev_bvshort_supports(ref->elem_bytes, ref->T) && hyp->N >= lev_bvshort_min_pairs();
+    const bool grouped = !short_form && p.ref_group >= 8 && hyp->N >= 128;
+    if (!short_form && !grouped && hyp->N < lev_bv_min_pairs()) return LEV_BV_NONE;
     if (ref->stride_t >= ((int64_t)1 << 31) || hyp->stride_t >= ((int64_t)1 << 31) ||
         ref->stride_t < 0 || hyp->stride_t < 0)
-        return false;
-    if ((ref->N > 1 && ref->stride_n != 1) || (hyp->N > 1 && hyp->stride_n != 1)) return false;
-    if (mode == LEV_MODE_PREFIX && out_sn != 1) return false;
-    return true;
+        return LEV_BV_NONE;
+    if ((ref->N > 1 && ref->stride_n != 1) || (hyp->N > 1 && hyp->stride_n != 1)) return LEV_BV_NONE;
+    if (mode == LEV_MODE_PREFIX && p.out_sn != 1) return LEV_BV_NONE;
+    // the short-reference kernel takes any batch, the fused kernel any batch whose references the
+    // caller declared shared: nothing to select on the device, no chain behind them
+    if (short_form) return LEV_BV_SHORT;
+    if (grouped || bv == 1) return LEV_BV_FUSED;
+    // device-selected: only where the wavefront fallback is the group path, whose kernels know how
+    // to stand by
+    return lev_group_eligible(p.R, p.H, p.P) ? LEV_BV_SELECTED : LEV_BV_NONE;
 }
 
-// The caller has checked lev_bitvec_eligible.  `counter` is one workspace word (Kb's block
-// counter).  `state` non-NULL: device-selected mode, Kb runs only if its probe does not veto;
-// `after_probe` (a cudaEvent_t, may be NULL) is recorded once that decision is final.
-int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                      const b200lev_opts_t* o, int mode, float mult, int32_t* ref_len,
-                      int32_t* hyp_len, int* counter, int32_t* state, int32_t* flags, float* out,
-                      int64_t out_si, int Hout, cudaStream_t st, void* after_probe, bool short_form,
-                      double* acc) {
+int lev_bitvec_launch(LevBvRoute route, const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                      const b200lev_opts_t* o, int mode, const LevLayout& L, char* ws,
+                      const LevParams& p, cudaStream_t st, void* after_probe, double* acc) {
     LevBvArgs a;
     memset(&a, 0, sizeof(a));
     a.ref = ref->data;
@@ -96,27 +95,33 @@ int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     a.has_eos = o->has_eos;
     a.eos = o->eos;
     a.include_eos = o->include_eos;
-    a.ref_len = ref_len;
-    a.hyp_len = hyp_len;
-    a.counter = counter;
-    a.state = state;
-    a.check_state = state != nullptr;
-    a.flags = flags;
+    a.ref_len = (int32_t*)(ws + L.off_ref_len);
+    a.hyp_len = (int32_t*)(ws + L.off_hyp_len);
+    a.counter = (int*)(ws + L.off_bv_counter);
+    a.flags = p.flags;
     a.slots_log2 = 4;  // buckets of 4 ways: on average at most one token per bucket
     while ((1 << a.slots_log2) < a.R) ++a.slots_log2;
     a.mode = mode;
     a.norm = o->norm;
     a.exclude_last = mode == LEV_MODE_PREFIX ? o->exclude_last : 0;
-    a.Hout = Hout;
-    a.mult = mult;
+    a.Hout = p.Hout;
+    a.mult = p.mult;
     a.padding = (float)o->padding;
-    a.out = out;
-    a.out_si = out_si;
-    a.acc = (short_form && mode == LEV_MODE_FINAL) ? acc : nullptr;
-    if (short_form) {  // R <= 64: lane = pair, reference in registers, no tables (lev_bvshort.cu)
+    a.out = p.out;
+    a.out_si = p.out_si;
+    if (route == LEV_BV_SHORT) {  // R <= 64: lane = pair, reference in registers, no tables (lev_bvshort.cu)
+        a.acc = mode == LEV_MODE_FINAL ? acc : nullptr;
         if (getenv("B200LEV_TRACE"))
             fprintf(stderr, "b200lev: short bit-vector kernel, mode %d, R=%d H=%d P=%d\n", mode, a.R, a.H, a.P);
         return lev_bvshort_launch(a, ref->elem_bytes, st);
+    }
+    if (route == LEV_BV_SELECTED) {
+        // Kb runs only if its probe does not veto.  The state words are cleared here, once, for
+        // both paths: the wavefront chain's pack kernels find them cleared.
+        a.state = (int32_t*)(ws + L.off_flags);
+        a.check_state = 1;
+        if (cudaMemsetAsync(a.state, 0, sizeof(int32_t) * (size_t)(4 + L.nbins), st) != cudaSuccess)
+            return lev_check_cuda("memset");
     }
     if (getenv("B200LEV_TRACE"))
         fprintf(stderr, "b200lev: fused bit-vector kernel, mode %d, R=%d H=%d P=%d W=%d device-selected=%d\n",

@@ -25,7 +25,7 @@
 //
 // Per DP cell that is about one ALU-pipe instruction (the packed wavefront kernel issues 1.5
 // and half an FMA-pipe one), and it is the WHOLE call.  Taken unconditionally (no probe, no
-// stand-by chain) whenever lev_bitvec_eligible holds and R <= 64.
+// stand-by chain) wherever lev_bitvec_route admits the bit-vector path and R <= 64.
 #include "lev_bitvec.cuh"
 
 constexpr int LEV_BVS_WARPS = 4;

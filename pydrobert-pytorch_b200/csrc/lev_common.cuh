@@ -220,17 +220,25 @@ int lev_group_eligible(int64_t R, int64_t H, int64_t P);
 __device__ __forceinline__ bool lev_bv_took(const int* state) {
     return *reinterpret_cast<const volatile int*>(state + 3) == 0;
 }
-// unit-cost bit-vector path (lev_bitvec.cu)
-bool lev_bitvec_eligible(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int mode,
-                         bool count_mode, bool float_path, int ins_i, int del_i, int sub_i,
-                         int64_t out_sn, int ref_group, bool* short_form, bool* grouped);
-int lev_bitvec_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                      const b200lev_opts_t* o, int mode, float mult, int32_t* ref_len,
-                      int32_t* hyp_len, int* counter, int32_t* state, int32_t* flags, float* out,
-                      int64_t out_si, int Hout, cudaStream_t st, void* after_probe, bool short_form,
-                      double* acc);
-// 0: off, 1: forced (tests; runs whatever the references look like), 2: device-selected
-int lev_bitvec_mode();
+// unit-cost bit-vector path (lev_bitvec.cu): which kernel takes a final / prefix call
+enum LevBvRoute {
+    LEV_BV_NONE,      // the wavefront path alone
+    LEV_BV_SHORT,     // Ks takes the call (and, in final mode, the error sums)
+    LEV_BV_FUSED,     // Kb takes the call
+    LEV_BV_SELECTED,  // probe + Kb ahead of the wavefront path's stand-by chain (lev_bv_took)
+};
+// `p` as lev_abi.cu fills it for the call: costs, shapes, ref_group, out_sn
+LevBvRoute lev_bitvec_route(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int mode,
+                            const LevParams& p, bool count_mode, bool float_path);
+// `ws` is the aligned workspace laid out as `L`; `acc` (final mode, may be NULL) goes to Ks.
+// With LEV_BV_SELECTED `after_probe` (a cudaEvent_t, may be NULL) is recorded once the veto is final.
+int lev_bitvec_launch(LevBvRoute route, const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                      const b200lev_opts_t* o, int mode, const LevLayout& L, char* ws,
+                      const LevParams& p, cudaStream_t st, void* after_probe, double* acc);
+// K7 (lev_loss.cu): acc[0] += sum(er), acc[1] += sum of the pairs' reference lengths, acc[2] += P
+// (P >= 1, ref_group >= 1)
+int lev_launch_err_sum(const float* er, const int32_t* ref_lens, int64_t P, int ref_group,
+                       double* acc, cudaStream_t st);
 int lev_launch_uid(const b200lev_tokens_t* ref, const int32_t* packed, const int* state,
                    const int32_t* ref_len, int32_t* uid,
                    int64_t* dtok, int32_t* ndist, int64_t Rp, cudaStream_t st);

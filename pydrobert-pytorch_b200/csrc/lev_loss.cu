@@ -460,16 +460,14 @@ lev_err_sum_kernel(const float* __restrict__ er, const int32_t* __restrict__ ref
     }
 }
 
-extern "C" int b200lev_err_sum(const float* er, const int32_t* ref_lens, int64_t P,
-                               int32_t ref_group, double* acc, void* stream) {
-    if (P <= 0) return B200LEV_OK;
-    if (ref_group < 1) ref_group = 1;
+int lev_launch_err_sum(const float* er, const int32_t* ref_lens, int64_t P, int ref_group,
+                       double* acc, cudaStream_t st) {
     int64_t blocks = (P + 255) / 256;
     if (blocks > 148 * 8) blocks = 148 * 8;
-    lev_prof_begin(LEV_PROF_ERR_SUM, (cudaStream_t)stream);
-    lev_launch(lev_err_sum_kernel, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, er,
-               ref_lens, P, (int)ref_group, acc);
-    lev_prof_end(LEV_PROF_ERR_SUM, (cudaStream_t)stream);
+    lev_prof_begin(LEV_PROF_ERR_SUM, st);
+    lev_launch(lev_err_sum_kernel, dim3((unsigned)blocks), dim3(256), 0, st, er, ref_lens, P,
+               ref_group, acc);
+    lev_prof_end(LEV_PROF_ERR_SUM, st);
     return lev_check_cuda("lev_err_sum_kernel");
 }
 

@@ -18,7 +18,7 @@ def wall(fn, n=2000):
     torch.cuda.synchronize(); return (time.perf_counter() - t0) / n * 1e6
 print("functional.prefix_error_rates        %.1f us" % wall(lambda: F.prefix_error_rates(ref, hyp, eos=0, warn=False)))
 args = (ref, hyp, 0, True, False, 1.0, 1.0, 1.0, True, True, False, -100, True, 1)
-print("_ops.string_matching_fast            %.1f us" % wall(lambda: _ops.string_matching_fast(*args)))
+print("_ops.string_matching_impl            %.1f us" % wall(lambda: _ops.string_matching_impl(*args)))
 L = _abi.lib()
 rt, ht = _ops._tok_struct(ref, False), _ops._tok_struct(hyp, False)
 o = _ops._opts(0, True, 1.0, 1.0, 1.0, True, False, -100, True, 1)

@@ -241,7 +241,7 @@ def check_nbest_batch(F, dev, seed, R, H, n_utts, nbest, V=30, shared=True, wide
 def check_grouped_references(F, dev, seed=0):
     """minimum_error_rate_loss on batches whose group size (samples per reference) is 8 or more:
     the call declares its references shared, so the fused bit-vector kernel takes it without a
-    probe (lev_bitvec_eligible: grouped) -- group sizes that divide 32, that do not (a block of 32
+    probe (lev_bitvec_route: grouped) -- group sizes that divide 32, that do not (a block of 32
     pairs then holds 5 references: two table passes), references of 65 .. 128 tokens (longer or
     shorter ones go elsewhere), sub_avg on and off, and the error rates themselves through the
     registered op."""

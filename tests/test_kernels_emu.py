@@ -185,7 +185,7 @@ def bv_form(request, monkeypatch):
 @pytest.mark.parametrize("group", [1, 3])
 def test_final_sums_every_kernel_form(F, bv_form, costs, group, monkeypatch):
     """b200lev_final_sums (the bulk-scoring step, command_line.py:1124-1147): the fp64 totals are
-    the same whether the short-reference kernel accumulates them itself or b200lev_err_sum follows
+    the same whether the short-reference kernel accumulates them itself or lev_err_sum_kernel follows
     the fused / wavefront kernels -- odd pair counts (lanes shadowing the last pair), references
     shared by `group` hypotheses, normalised and raw values."""
     from b200lev import _ops
