@@ -109,6 +109,20 @@ int b200lev_prefix(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                    int32_t *flags, void *stream);
 
 /*
+ * Per pair the correct / substitution / deletion / insertion counts (sclite's C/S/D/I) along
+ * the path the count mode of error_rate takes (SM:292-314: sub over ins over del on ties), also
+ * for uniform costs.  S + D + I equals error_rate(norm=False) for the same eos and costs,
+ * C + S + D the reference length and C + S + I the hypothesis length.
+ * out: device int64, element (n, k) at out[n*4 + k], k = 0 correct, 1 substitutions,
+ * 2 deletions, 3 insertions.  opts: has_eos, eos, include_eos and the costs as for
+ * b200lev_final; ref_group must be 1; norm, exclude_last, padding, return_mistakes are
+ * ignored.  Workspace: b200lev_workspace_bytes(ref, hyp, B200LEV_WS_FINAL, 0).
+ */
+int b200lev_error_counts(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
+                         const b200lev_opts_t *opts, int64_t *out, void *workspace,
+                         size_t workspace_bytes, int32_t *flags, void *stream);
+
+/*
  * optimal_completion (SM:464-517), two phases around the one host read the
  * reference also needs (SM:511: U = counts.max().item()).
  *   phase 1 runs the DP in mask mode (SM:271-278, 319-339, 347-355), leaves the

@@ -187,6 +187,43 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, nor
 
 
 # ---------------------------------------------------------------------------------------
+# error counts: (C, S, D, I) per pair
+# ---------------------------------------------------------------------------------------
+def error_counts_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
+                      batch_first: bool, ins_cost: float, del_cost: float, sub_cost: float
+                      ) -> Tuple[Tensor, Tensor]:
+    """Per pair the correct, substitution, deletion and insertion counts along the path the
+    count mode of ``error_rate`` takes (_string.py:292-314), ``(out, flags)``: int64 ``(N, 4)``
+    and the int32[1] warning flags, on the device of ``ref``.  One C call
+    (``b200lev_error_counts``)."""
+    _, _, n = _shapes(ref, hyp, batch_first, 1)
+    ref, hyp = _as_tokens(ref), _as_tokens(hyp)
+    pl = _host.Placement(ref, hyp)
+    ref, hyp, dev = pl.to_dev(ref), pl.to_dev(hyp), pl.dev
+    L = _abi.lib()
+    with _DeviceGuard(dev):
+        rt, ht = _tok_struct(ref, batch_first), _tok_struct(hyp, batch_first)
+        o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, False, False, 0, True, 1)
+        flags = torch.zeros(1, dtype=torch.int32, device=dev)
+        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 0, 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        out = torch.empty((n, 4), dtype=torch.long, device=dev)
+        _abi.check(L.b200lev_error_counts(ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o),
+                                          out.data_ptr(), ws.data_ptr(), nbytes, flags.data_ptr(),
+                                          _stream(dev)))
+    return pl.back(out), pl.back(flags)
+
+
+error_counts = torch.library.custom_op("b200lev::error_counts", error_counts_impl, mutates_args=())
+
+
+@error_counts.register_fake
+def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
+    n = hyp.shape[0] if batch_first else hyp.shape[1]
+    return ref.new_empty((n, 4), dtype=torch.long), ref.new_empty((1,), dtype=torch.int32)
+
+
+# ---------------------------------------------------------------------------------------
 # optimal completion
 # ---------------------------------------------------------------------------------------
 def optimal_completion_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,

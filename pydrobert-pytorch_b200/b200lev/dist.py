@@ -91,6 +91,31 @@ def bulk_error_rate(ref: torch.Tensor, hyp: torch.Tensor, eos: Optional[int] = N
     return er, acc
 
 
+def bulk_error_counts(ref: torch.Tensor, hyp: torch.Tensor, eos: Optional[int] = None,
+                      include_eos: bool = False, batch_first: bool = False, ins_cost: float = 1.0,
+                      del_cost: float = 1.0, sub_cost: float = 1.0, process_group=None,
+                      warn: bool = False):
+    """:func:`bulk_error_rate` with the breakdown: score this rank's pairs and reduce the
+    counts over the process group.
+
+    Returns ``(per_pair, totals)``: ``per_pair`` is this rank's ``(N, 4)`` int64
+    ``(C, S, D, I)`` (:func:`b200lev.functional.error_counts`) and ``totals`` its column sums,
+    int64[4], summed over the ranks.  The corpus WER is ``(S + D + I) / (C + S + D)``."""
+    per_pair, flags = _ops.error_counts_impl(ref, hyp, eos, include_eos, batch_first,
+                                             float(ins_cost), float(del_cost), float(sub_cost))
+    if warn:
+        F._warn_flags(flags, eos, include_eos, False, False)
+    totals = per_pair.sum(0)
+    if dist.is_available() and dist.is_initialized():
+        if dist.get_backend(process_group) == "gloo" and totals.is_cuda:
+            host = totals.cpu()
+            dist.all_reduce(host, op=dist.ReduceOp.SUM, group=process_group)
+            totals = host.to(totals.device)
+        else:
+            dist.all_reduce(totals, op=dist.ReduceOp.SUM, group=process_group)
+    return per_pair, totals
+
+
 def score_corpora_sharded(ref, hyp, process_group=None, **score_kwargs):
     """``scoring.score_corpora`` over the ranks of a process group: the aligned corpora are cut
     into contiguous blocks of utterances (:func:`shard_bounds`), every rank scores its block on

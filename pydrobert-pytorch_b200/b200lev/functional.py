@@ -28,6 +28,7 @@ from . import _ops, config
 
 __all__ = [
     "edit_distance",
+    "error_counts",
     "error_rate",
     "fill_after_eos",
     "hard_optimal_completion_distillation_loss",
@@ -208,6 +209,44 @@ def prefix_edit_distances(
     """Functional version of PrefixEditDistances (SM:553-583)."""
     return _string_matching(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost,
                             sub_cost, warn, norm, True, exclude_last, padding, False, 1)
+
+
+@script
+def error_counts(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> torch.Tensor:
+    """Per pair the correct, substitution, deletion and insertion counts (sclite's C/S/D/I):
+    ``(N, 4)`` long, columns in that order.
+
+    They are the op counts along the path that :func:`error_rate` counts its errors on
+    (SM:292-314: every cell takes the substitution candidate unless the insertion candidate is
+    smaller, then the deletion candidate only if it is smaller still), also for uniform costs.
+    Lengths follow ``eos`` / ``include_eos`` as in :func:`error_rate`, so ``C + S + D`` is the
+    reference length, ``C + S + I`` the hypothesis length and ``S + D + I`` equals
+    ``error_rate(..., norm=False)`` with the same costs.  ``warn`` covers the two missing-eos
+    warnings."""
+    if ref.dim() != 2 or hyp.dim() != 2:
+        raise RuntimeError("ref and hyp must be 2 dimensional")
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            out, flags = _ops.error_counts_impl(ref, hyp, eos, include_eos, batch_first,
+                                                float(ins_cost), float(del_cost), float(sub_cost))
+            if warn:
+                _warn_flags(flags, eos, include_eos, False, False)
+            return out
+    out, flags = torch.ops.b200lev.error_counts(ref, hyp, eos, include_eos, batch_first, ins_cost,
+                                                del_cost, sub_cost)
+    if warn:
+        _warn_flags(flags, eos, include_eos, False, False)
+    return out
 
 
 def _optimal_completion(

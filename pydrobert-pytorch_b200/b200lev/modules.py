@@ -16,6 +16,7 @@ from . import functional as F
 
 __all__ = [
     "EditDistance",
+    "ErrorCounts",
     "ErrorRate",
     "FillAfterEndOfSequence",
     "HardOptimalCompletionDistillationLoss",
@@ -106,6 +107,21 @@ class EditDistance(_StringMatching):
     def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
         return F.edit_distance(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
                                self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class ErrorCounts(_StringMatching):
+    """Correct, substitution, deletion and insertion counts (sclite's C/S/D/I) per pair along
+    the path ErrorRate counts its errors on: ``(N, 4)`` long (see
+    :func:`b200lev.functional.error_counts`)"""
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, batch_first: bool = False,
+                 ins_cost: float = config.DEFT_INS_COST, del_cost: float = config.DEFT_DEL_COST,
+                 sub_cost: float = config.DEFT_SUB_COST, warn: bool = True):
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
+        return F.error_counts(ref, hyp, self.eos, self.include_eos, self.batch_first, self.ins_cost,
+                              self.del_cost, self.sub_cost, self.warn)
 
 
 class ErrorRate(_StringMatching):

@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
+#include <cstdlib>
 
 #include "lev_common.cuh"
 
@@ -403,6 +404,44 @@ extern "C" int b200lev_prefix(const b200lev_tokens_t* ref, const b200lev_tokens_
                               int32_t* flags, void* stream) {
     return lev_string_match(ref, hyp, opts, LEV_MODE_PREFIX, out, out_stride_i, out_stride_n,
                             workspace, workspace_bytes, flags, nullptr, stream);
+}
+
+// Per pair (C, S, D, I) along the path of error_rate's count mode (SM:292-314; unit costs after
+// SM:168-174 take the same cell).  R <= 64 with one token width: the short form, one launch
+// straight from the raw tokens (lev_counts.cuh).  Otherwise K0 + K1 with the insertion channel.
+extern "C" int b200lev_error_counts(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                                    const b200lev_opts_t* opts, int64_t* out, void* workspace,
+                                    size_t workspace_bytes, int32_t* flags, void* stream) {
+    if (opts && opts->ref_group != 1) {
+        lev_set_error("error counts: ref_group must be 1, got %d", opts->ref_group);
+        return B200LEV_ERR_ARG;
+    }
+    LevLayout L;
+    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_FINAL, out, workspace, workspace_bytes, &L);
+    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = lev_ws_base(workspace);
+    b200lev_opts_t o = *opts;
+    o.norm = 0;
+    o.exclude_last = 0;
+    o.return_mistakes = 1;
+    LevParams p;
+    bool cm, fp;
+    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
+    const bool trace = getenv("B200LEV_TRACE") != nullptr;
+    if (L.R <= 64 && ref->elem_bytes == hyp->elem_bytes) {
+        if (trace)
+            fprintf(stderr, "b200lev: error counts, lev_counts_short_kernel, R=%lld H=%lld P=%lld %s\n",
+                    (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
+        return lev_counts_short_launch(ref, hyp, &o, p, fp, out, st);
+    }
+    if (trace)
+        fprintf(stderr, "b200lev: error counts, pack + lev_warp_kernel, R=%lld H=%lld P=%lld %s\n",
+                (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
+    p.out = reinterpret_cast<float*>(out);  // (lev_common.cuh: the counts go where FINAL's values go)
+    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
+    if (rc == B200LEV_OK) rc = lev_launch_counts_dp(p, fp, st);
+    return rc;
 }
 
 extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,

@@ -125,7 +125,8 @@ struct LevParams {
     float mult;  // SM:168-174
     int norm, exclude_last;
     float padding;
-    // FINAL: out[n];  PREFIX: out[i*out_si + n*out_sn]
+    // FINAL: out[n];  PREFIX: out[i*out_si + n*out_sn];  error counts (lev_launch_counts_dp): int64
+    // (C, S, D, I) of pair n at ((int64_t*)out)[4n .. 4n+3]
     float* out;
     int64_t out_si, out_sn;
     int Hout;
@@ -208,6 +209,12 @@ int lev_launch_dp(const LevParams& p, int mode, bool count_mode, bool float_path
 int lev_launch_group(const LevParams& p, int mode, bool count_mode, cudaStream_t st);
 int lev_launch_mask16(const LevParams& p, bool float_path, cudaStream_t st);
 int lev_launch_cta(const LevParams& p, int mode, bool count_mode, bool float_path, cudaStream_t st);
+// b200lev_error_counts: K1 with the insertion channel, after K0 (lev_dp.cu), and the short form
+// for R <= 64 straight from the raw tokens (lev_counts.cuh; `p` supplies the costs)
+int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st);
+int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                            const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                            int64_t* out, cudaStream_t st);
 // lanes per pair if the shapes admit the group kernel (its histogram is then built at
 // pack time), else 0
 int lev_group_eligible(int64_t R, int64_t H, int64_t P);

@@ -31,11 +31,11 @@
 #include "lev_arith.cuh"
 
 // number of per-warp shared-memory columns (boundary channels + row minima)
-template <typename V, bool COUNT, int MODE>
+template <typename V, bool COUNT, int MODE, bool OPS = false>
 struct LevBufs {
     static constexpr bool FLT_COST = !std::is_same<V, int>::value && !COUNT;
-    // MASK: + row minima + the chained bitmap word handed from strip to strip
-    static constexpr int NB = (COUNT ? 2 : (FLT_COST ? 3 : 1)) + (MODE == LEV_MODE_MASK ? 2 : 0);
+    // MASK: + row minima + the chained bitmap word handed from strip to strip; OPS: + insertions
+    static constexpr int NB = (COUNT ? 2 : (FLT_COST ? 3 : 1)) + (MODE == LEV_MODE_MASK ? 2 : 0) + (OPS ? 1 : 0);
 };
 
 // One pair on one warp.  PASS: 0 = the only pass (FINAL/PREFIX) or the row-minimum
@@ -45,6 +45,8 @@ struct LevBufs {
 // (and from strip to strip through a shared-memory column), and stored once per row by the
 // last lane -- no atomics, no divergent branch per cell, and the largest set size (SM:510-511)
 // falls out of the same word.  Returns that size (valid on lane 31).
+// OPS (FINAL, COUNT only; b200lev_error_counts): one more int32 channel, the insertions along the
+// path the count cell picks, carried like the count channel; the epilogue writes (C, S, D, I).
 // tokens that do not fit in int32 (B200LEV_FLAG_WIDE_TOKENS): read the caller's tensors
 // directly and compare in 64 bits.  Slow (strided gathers) but exact; uniform per launch.
 __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes, int64_t idx) {
@@ -56,7 +58,7 @@ __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes
     }
 }
 
-template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE>
+template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE, bool OPS>
 __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair, const int r,
                                               const int h, const int steps,
                                               const int* __restrict__ hyp_s_,
@@ -82,7 +84,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
     V* __restrict__ bnd_b = bufs + 2 * Hs;  // FLT_COST: fl(origin * del)
     V* __restrict__ rowmin = bufs + (LevBufs<V, COUNT, MODE>::NB - 2) * Hs;  // MASK only
     unsigned* __restrict__ bitcol = reinterpret_cast<unsigned*>(bufs + (LevBufs<V, COUNT, MODE>::NB - 1) * Hs);
-    (void)bnd_a; (void)bnd_b; (void)rowmin; (void)bitcol;
+    int* __restrict__ bnd_i = reinterpret_cast<int*>(bufs + 2 * Hs);  // OPS: insertions
+    (void)bnd_a; (void)bnd_b; (void)rowmin; (void)bitcol; (void)bnd_i;
 
     for (int k = 0; k < S; ++k) {
         const bool first = (k == 0), last = (k == S - 1);
@@ -90,6 +93,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
         const int j0 = jb + lane * C + 1;  // this lane's first column
         V v[C];
         V m[C];     // COUNT: mistake counts
+        int ic[C];  // OPS: insertions
         V jd[C];    // FLT_COST: fl(j * del), SM:258-263
         Tok rt[C];  // reference token of column j (ref position j-1)
         int ud[C];  // EQ: distinct-token rank of ref position j, or -1
@@ -98,6 +102,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
             const int j = j0 + c;
             v[c] = (j >= 0) ? (V)j * delc : BIG;
             m[c] = (V)(j >= 0 ? j : 0);  // SM:260
+            ic[c] = 0;                   // row 0: deletions only
             jd[c] = (j >= 0) ? (V)j * delc : (V)0;
             if (WIDE)
                 rt[c] = (j >= 1) ? (Tok)lev_load_raw(p.ref_raw, p.ref_eb,
@@ -110,7 +115,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
             // EQC: the bit of this column's token (ranks < 32), 0 for columns that are no target
             if (EQC) ud[c] = (j >= 0 && j < r) ? (int)(1u << (p.uid[(int64_t)refcol * p.Rp + j] & 31)) : 0;
         }
-        (void)m; (void)jd; (void)ud;
+        (void)m; (void)jd; (void)ud; (void)ic;
         unsigned bitrun = 0u;  // EQC chain register
         (void)bitrun;
         // chain registers: what this lane publishes to lane+1 at the next step
@@ -120,7 +125,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
         // boundary column, the other lanes pick it up from the shuffle at step l
         V pl_v = first ? BIG : (V)jb * delc;
         V pl_m = (V)(first ? 0 : jb);
-        (void)pl_m;
+        int pl_i = 0;
+        (void)pl_m; (void)pl_i;
         if (steps > 0) {
             const int nsteps = steps + 31;
             for (int s = 1; s <= nsteps; ++s) {
@@ -136,6 +142,14 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                     diag_m = pl_m;
                     pl_m = in_m;
                 }
+                int in_i = 0, diag_i = 0;
+                if (OPS) {
+                    const int sh_i = __shfl_up_sync(LEV_FULL_MASK, ic[C - 1], 1);
+                    in_i = (lane == 0) ? (first ? 0 : bnd_i[32 + s]) : sh_i;
+                    diag_i = pl_i;
+                    pl_i = in_i;
+                }
+                (void)in_i; (void)diag_i;
                 if (FLT_COST) {
                     const V sh_ob = __shfl_up_sync(LEV_FULL_MASK, ob, 1);
                     const V sh_oj = __shfl_up_sync(LEV_FULL_MASK, oj, 1);
@@ -158,6 +172,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                     if (COUNT) {
                         // SM:292-314: (cost, count); ties: sub over ins over del
                         V dc = diag_v, dm = diag_m, lc = in_v, lm = in_m;
+                        int di = diag_i, li = in_i;
+                        (void)di; (void)li;
 #pragma unroll
                         for (int c = 0; c < C; ++c) {
                             const V uc = v[c], um = m[c];
@@ -174,6 +190,14 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                             const bool keep = del_c >= cc;                      // SM:309
                             cc = keep ? cc : del_c;
                             mm = keep ? mm : lm + (V)1;  // SM:311-313
+                            if (OPS) {  // the insertion count of the predecessor picked, +1 for ins
+                                const int ui = ic[c];
+                                int ii = ps ? di : ui + 1;
+                                ii = keep ? ii : li;
+                                di = ui;
+                                li = ii;
+                                ic[c] = ii;
+                            }
                             dc = uc;
                             dm = um;
                             lc = cc;
@@ -254,6 +278,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         if (!last) {
                             bnd_v[32 + i] = v[C - 1];
                             if (COUNT) bnd_a[32 + i] = m[C - 1];
+                            if (OPS) bnd_i[32 + i] = ic[C - 1];
                             if (FLT_COST) {
                                 bnd_a[32 + i] = ob;
                                 bnd_b[32 + i] = oj;
@@ -267,8 +292,17 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                 }
             }
         }
-        if (MODE == LEV_MODE_FINAL && last && lane == 31)  // SM:390-405
+        if (OPS && last && lane == 31) {
+            // m = S + D + I; C + S + D = r and C + S + I = h
+            const int ins = ic[C - 1], del = ins + r - h, sub = (int)m[C - 1] - ins - del;
+            int64_t* __restrict__ o = reinterpret_cast<int64_t*>(p.out) + (int64_t)pair * 4;
+            o[0] = h - sub - ins;
+            o[1] = sub;
+            o[2] = del;
+            o[3] = ins;
+        } else if (MODE == LEV_MODE_FINAL && last && lane == 31) {  // SM:390-405
             p.out[pair] = lev_finalize((float)(COUNT ? m[C - 1] : v[C - 1]), p, r, h > 0);
+        }
         __syncwarp();
     }
     return set_max;
@@ -276,22 +310,22 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
 
 // Returns -1 when the largest target set still has to be counted from the bitmaps in global
 // memory (atomic pass), else that size as lane 31 saw it (chained pass).
-template <typename V, bool COUNT, int MODE, int C, bool WIDE = false>
+template <typename V, bool COUNT, int MODE, int C, bool WIDE = false, bool OPS = false>
 __device__ __forceinline__ int lev_warp_pair_all(const LevParams& p, int pair, int r, int h,
                                                  int steps, const int* hyp_s, V* bufs, int Hs,
                                                  bool one_word) {
-    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE>(p, pair, r, h, steps, hyp_s, bufs, Hs);
+    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs);
     if (MODE == LEV_MODE_MASK) {
-        if (one_word) return lev_warp_pair<V, COUNT, MODE, C, 2, WIDE>(p, pair, r, h, steps, hyp_s, bufs, Hs);
-        lev_warp_pair<V, COUNT, MODE, C, 1, WIDE>(p, pair, r, h, steps, hyp_s, bufs, Hs);
+        if (one_word) return lev_warp_pair<V, COUNT, MODE, C, 2, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
+        lev_warp_pair<V, COUNT, MODE, C, 1, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
     }
     return -1;
 }
 
 // CMASK: bit c set => the kernel carries a C = 2^c variant (1, 2, 4, 8); each pair
 // takes the smallest variant whose single strip covers its r + 1 columns, the largest
-// one (multi-strip) otherwise.
-template <typename V, bool COUNT, int MODE, int CMASK>
+// one (multi-strip) otherwise.  OPS: the error-counts epilogue (FINAL, COUNT).
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false>
 __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     LEV_DYN_SMEM(int, smem);
     const int lane = threadIdx.x & 31;
@@ -299,7 +333,7 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     const int wpc = blockDim.x >> 5;
     // (even: every warp's slice starts 8-byte aligned, the 64-bit-token path stores int64)
     const int Hs = (p.H + 65) & ~1;
-    constexpr int NB = LevBufs<V, COUNT, MODE>::NB;
+    constexpr int NB = LevBufs<V, COUNT, MODE, OPS>::NB;
     int* hyp_s = smem + (size_t)warp * (2 + NB) * Hs;  // 2*Hs ints: room for int64 tokens
     V* bufs = reinterpret_cast<V*>(hyp_s + 2 * Hs);
     const bool wide = (*p.wide_flag & B200LEV_FLAG_WIDE_TOKENS) != 0;
@@ -327,16 +361,16 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
         const bool one_word = MODE == LEV_MODE_MASK && p.ndist[pair / p.ref_group] <= 32;
         int set_max = -1;
         if (wide)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true>(
+            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true, OPS>(
                 p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 1) && (cols <= 32 || !(CMASK & 14)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 1>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 1, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 2) && (cols <= 64 || !(CMASK & 12)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 2>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 2, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 4) && (cols <= 128 || !(CMASK & 8)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 4>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 4, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if (CMASK & 8)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 8>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 8, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
 
         if (MODE == LEV_MODE_PREFIX) {
             // SM:279-285 (row 0) and SM:379-386 (tail := padding)
@@ -380,9 +414,9 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     }
 }
 
-template <typename V, bool COUNT, int MODE, int CMASK>
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false>
 static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
-    constexpr int NB = LevBufs<V, COUNT, MODE>::NB;
+    constexpr int NB = LevBufs<V, COUNT, MODE, OPS>::NB;
     const size_t per_warp = (size_t)(2 + NB) * (size_t)((p.H + 65) & ~1) * sizeof(int);
     const size_t budget = 200 * 1024;
     if (per_warp > budget) {
@@ -395,7 +429,7 @@ static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
     // keep at least two CTAs per SM resident when the rows are short
     while (wpc > 1 && per_warp * wpc > 100 * 1024) --wpc;
     const size_t smem = per_warp * wpc;
-    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK>;
+    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK, OPS>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)smem);
@@ -464,3 +498,15 @@ int lev_launch_dp(const LevParams& p_, int mode, bool count_mode, bool float_pat
     lev_set_error("mask mode is defined on the cost row only (SM:479-491)");
     return B200LEV_ERR_ARG;
 }
+
+// b200lev_error_counts, references longer than the short form takes (lev_counts.cuh): K1 with the
+// count cell and the insertion channel, after K0.  No group, CTA or bit-vector kernel: they carry
+// no path.
+int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st) {
+    if (p.P <= 0) return B200LEV_OK;
+    if (!float_path) return lev_launch_variant<int, true, LEV_MODE_FINAL, 10, true>(p, st);
+    return lev_launch_variant<float, true, LEV_MODE_FINAL, 4, true>(p, st);
+}
+
+// the short form (R <= 64): one lane per pair from the raw tokens
+#include "lev_counts.cuh"
