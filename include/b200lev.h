@@ -83,10 +83,16 @@ int b200lev_device_count(void);
 /* Scratch bytes needed by the calls below for these shapes (packed tokens, lengths,
  * bucketing tables).  kind: B200LEV_WS_FINAL for b200lev_final*, B200LEV_WS_PREFIX for
  * b200lev_prefix (adds the raw prefix rows), B200LEV_WS_COMPLETION for the completion
- * calls (adds the distinct-token tables and bitmaps). */
+ * calls (adds the distinct-token tables and bitmaps), B200LEV_WS_ALIGN for
+ * b200lev_error_alignment (adds every DP cell's 2-bit choice).  The alignment kind adds, for
+ * ref->T <= 64 with equal token widths, 8 or 16 bytes per hypothesis position and pair (R <= 32
+ * or not); otherwise (H + 31) * 64 * ceil((R + 1) / 256) bytes or (H + 31) * 32 *
+ * ceil((R + 1) / 128) bytes per pair, whichever is larger, plus one int32 per pair: about
+ * 15 kB per pair at R = H = 200, 1 MB at R = H = 2000. */
 #define B200LEV_WS_FINAL 0
 #define B200LEV_WS_COMPLETION 1
 #define B200LEV_WS_PREFIX 2
+#define B200LEV_WS_ALIGN 3
 size_t b200lev_workspace_bytes(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                                int32_t kind, int32_t exclude_last);
 
@@ -121,6 +127,21 @@ int b200lev_prefix(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
 int b200lev_error_counts(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                          const b200lev_opts_t *opts, int64_t *out, void *workspace,
                          size_t workspace_bytes, int32_t *flags, void *stream);
+
+/*
+ * The edit operations along the path b200lev_error_counts counts, one per step, in forward
+ * order from the start of both sequences to cell (h, r): 0 correct, 1 substitution,
+ * 2 deletion, 3 insertion.  Row 0 of the DP is all deletions and column 0 all insertions.
+ * Per pair the histogram of the ops equals b200lev_error_counts with the same arguments.
+ * out: device int8, step k of pair n at out[k*out_stride_k + n*out_stride_n], k in
+ * [0, ref->T + hyp->T); steps from the path length r + I on hold -1.  opts as for
+ * b200lev_error_counts (ref_group must be 1).
+ * Workspace: b200lev_workspace_bytes(ref, hyp, B200LEV_WS_ALIGN, 0).
+ */
+int b200lev_error_alignment(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
+                            const b200lev_opts_t *opts, int8_t *out, int64_t out_stride_k,
+                            int64_t out_stride_n, void *workspace, size_t workspace_bytes,
+                            int32_t *flags, void *stream);
 
 /*
  * optimal_completion (SM:464-517), two phases around the one host read the

@@ -224,6 +224,53 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
 
 
 # ---------------------------------------------------------------------------------------
+# error alignment: the ops along the error-counts path
+# ---------------------------------------------------------------------------------------
+def error_alignment_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
+                         batch_first: bool, ins_cost: float, del_cost: float, sub_cost: float
+                         ) -> Tuple[Tensor, Tensor]:
+    """Per pair the edit operations along the path ``error_counts_impl`` counts, ``(out, flags)``:
+    int8 ``(R + H, N)`` (``(N, R + H)`` with ``batch_first``; 0 correct, 1 substitution,
+    2 deletion, 3 insertion, -1 past the path's end) and the int32[1] warning flags, on the device
+    of ``ref``.  One C call (``b200lev_error_alignment``)."""
+    R, H, n = _shapes(ref, hyp, batch_first, 1)
+    ref, hyp = _as_tokens(ref), _as_tokens(hyp)
+    pl = _host.Placement(ref, hyp)
+    ref, hyp, dev = pl.to_dev(ref), pl.to_dev(hyp), pl.dev
+    L = _abi.lib()
+    with _DeviceGuard(dev):
+        rt, ht = _tok_struct(ref, batch_first), _tok_struct(hyp, batch_first)
+        o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, False, False, 0, True, 1)
+        flags = torch.zeros(1, dtype=torch.int32, device=dev)
+        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 3, 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        if batch_first:
+            out = torch.empty((n, R + H), dtype=torch.int8, device=dev)
+            sk, sn = 1, R + H
+        else:
+            out = torch.empty((R + H, n), dtype=torch.int8, device=dev)
+            sk, sn = n, 1
+        _abi.check(L.b200lev_error_alignment(ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o),
+                                             out.data_ptr(), sk, sn, ws.data_ptr(), nbytes,
+                                             flags.data_ptr(), _stream(dev)))
+    return pl.back(out), pl.back(flags)
+
+
+error_alignment = torch.library.custom_op("b200lev::error_alignment", error_alignment_impl,
+                                          mutates_args=())
+
+
+@error_alignment.register_fake
+def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
+    if batch_first:
+        (_, R), (n, H) = ref.shape, hyp.shape
+    else:
+        (R, _), (H, n) = ref.shape, hyp.shape
+    shape = (n, R + H) if batch_first else (R + H, n)
+    return ref.new_empty(shape, dtype=torch.int8), ref.new_empty((1,), dtype=torch.int32)
+
+
+# ---------------------------------------------------------------------------------------
 # optimal completion
 # ---------------------------------------------------------------------------------------
 def optimal_completion_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,

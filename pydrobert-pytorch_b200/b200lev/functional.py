@@ -27,7 +27,9 @@ import torch
 from . import _ops, config
 
 __all__ = [
+    "alignment_positions",
     "edit_distance",
+    "error_alignment",
     "error_counts",
     "error_rate",
     "fill_after_eos",
@@ -247,6 +249,61 @@ def error_counts(
     if warn:
         _warn_flags(flags, eos, include_eos, False, False)
     return out
+
+
+@script
+def error_alignment(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> torch.Tensor:
+    """Per pair the edit operations along the path :func:`error_counts` counts: int8
+    ``(R + H, N)``, or ``(N, R + H)`` with ``batch_first``, where R and H are the padded lengths.
+
+    Step ``k`` of a pair is 0 (correct), 1 (substitution), 2 (deletion) or 3 (insertion), in
+    forward order from the start of both sequences; steps from the path length ``r + I`` on hold
+    -1.  Per pair the histogram of the ops equals :func:`error_counts` with the same arguments.
+    Arguments, lengths and warnings are those of :func:`error_counts`.  The output's shape
+    depends on the input shapes only, so the call reads nothing back to the host (with
+    ``warn=False``).  :func:`alignment_positions` maps the steps to token positions."""
+    if ref.dim() != 2 or hyp.dim() != 2:
+        raise RuntimeError("ref and hyp must be 2 dimensional")
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            out, flags = _ops.error_alignment_impl(ref, hyp, eos, include_eos, batch_first,
+                                                   float(ins_cost), float(del_cost), float(sub_cost))
+            if warn:
+                _warn_flags(flags, eos, include_eos, False, False)
+            return out
+    out, flags = torch.ops.b200lev.error_alignment(ref, hyp, eos, include_eos, batch_first, ins_cost,
+                                                   del_cost, sub_cost)
+    if warn:
+        _warn_flags(flags, eos, include_eos, False, False)
+    return out
+
+
+@script
+def alignment_positions(ops: torch.Tensor, batch_first: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The token positions the steps of :func:`error_alignment` consume: ``(ref_pos, hyp_pos)``,
+    int64, shaped like ``ops``.
+
+    ``ref_pos[k]`` is the index of the reference token step ``k`` consumes (correct,
+    substitution or deletion), -1 for an insertion and for padding; ``hyp_pos[k]`` the index of
+    the hypothesis token (correct, substitution or insertion), -1 for a deletion and for
+    padding.  Gathering the tokens at both turns the ops into confusion pairs or display
+    columns."""
+    dim = 1 if batch_first else 0
+    on_ref = (ops >= 0) & (ops != 3)
+    on_hyp = (ops >= 0) & (ops != 2)
+    ref_pos = (on_ref.long().cumsum(dim) - 1).masked_fill(~on_ref, -1)
+    hyp_pos = (on_hyp.long().cumsum(dim) - 1).masked_fill(~on_hyp, -1)
+    return ref_pos, hyp_pos
 
 
 def _optimal_completion(

@@ -16,6 +16,7 @@ from . import functional as F
 
 __all__ = [
     "EditDistance",
+    "ErrorAlignment",
     "ErrorCounts",
     "ErrorRate",
     "FillAfterEndOfSequence",
@@ -107,6 +108,20 @@ class EditDistance(_StringMatching):
     def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
         return F.edit_distance(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
                                self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class ErrorAlignment(_StringMatching):
+    """The edit operations per pair along the path ErrorCounts counts: int8 ``(R + H, N)``, or
+    ``(N, R + H)`` with ``batch_first`` (see :func:`b200lev.functional.error_alignment`)"""
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, batch_first: bool = False,
+                 ins_cost: float = config.DEFT_INS_COST, del_cost: float = config.DEFT_DEL_COST,
+                 sub_cost: float = config.DEFT_SUB_COST, warn: bool = True):
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
+        return F.error_alignment(ref, hyp, self.eos, self.include_eos, self.batch_first, self.ins_cost,
+                                 self.del_cost, self.sub_cost, self.warn)
 
 
 class ErrorCounts(_StringMatching):

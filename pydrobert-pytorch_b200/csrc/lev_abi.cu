@@ -160,7 +160,7 @@ static int lev_begin(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                      int null_status = B200LEV_ERR_ARG) {
     const int rc = lev_check_tokens(ref, hyp, o);
     if (rc) return rc;
-    *L = lev_layout(ref, hyp, kind, kind == B200LEV_WS_FINAL ? 0 : o->exclude_last);
+    *L = lev_layout(ref, hyp, kind, kind == B200LEV_WS_FINAL || kind == B200LEV_WS_ALIGN ? 0 : o->exclude_last);
     if (hyp->N == 0 || L->Hout <= 0 || inner <= 0) return LEV_EMPTY;
     if (!out || !ws) {
         lev_set_error("NULL output or workspace");
@@ -429,7 +429,7 @@ extern "C" int b200lev_error_counts(const b200lev_tokens_t* ref, const b200lev_t
     bool cm, fp;
     lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
     const bool trace = getenv("B200LEV_TRACE") != nullptr;
-    if (L.R <= 64 && ref->elem_bytes == hyp->elem_bytes) {
+    if (lev_counts_short_form(ref, hyp)) {
         if (trace)
             fprintf(stderr, "b200lev: error counts, lev_counts_short_kernel, R=%lld H=%lld P=%lld %s\n",
                     (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
@@ -441,6 +441,48 @@ extern "C" int b200lev_error_counts(const b200lev_tokens_t* ref, const b200lev_t
     p.out = reinterpret_cast<float*>(out);  // (lev_common.cuh: the counts go where FINAL's values go)
     rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
     if (rc == B200LEV_OK) rc = lev_launch_counts_dp(p, fp, st);
+    return rc;
+}
+
+// Per pair the ops along the path b200lev_error_counts counts (lev_align.cuh): the same two forms,
+// each keeping every cell's choice in the workspace and walking it back.  Short form: one launch,
+// the lane walks its own trace.  Long form: K0, K1 with the trace, then one thread per pair walks.
+extern "C" int b200lev_error_alignment(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                                       const b200lev_opts_t* opts, int8_t* out, int64_t out_stride_k,
+                                       int64_t out_stride_n, void* workspace, size_t workspace_bytes,
+                                       int32_t* flags, void* stream) {
+    if (opts && opts->ref_group != 1) {
+        lev_set_error("error alignment: ref_group must be 1, got %d", opts->ref_group);
+        return B200LEV_ERR_ARG;
+    }
+    LevLayout L;
+    const int64_t steps = (ref && hyp) ? ref->T + hyp->T : 0;
+    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_ALIGN, out, workspace, workspace_bytes, &L, steps);
+    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = lev_ws_base(workspace);
+    b200lev_opts_t o = *opts;
+    o.norm = 0;
+    o.exclude_last = 0;
+    o.return_mistakes = 1;
+    LevParams p;
+    bool cm, fp;
+    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
+    const bool trace = getenv("B200LEV_TRACE") != nullptr;
+    if (lev_counts_short_form(ref, hyp)) {
+        if (trace)
+            fprintf(stderr, "b200lev: error alignment, lev_counts_short_kernel (trace), R=%lld H=%lld P=%lld %s\n",
+                    (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
+        return lev_align_short_launch(ref, hyp, &o, p, fp, (uint32_t*)(ws + L.off_trace), out, out_stride_k,
+                                      out_stride_n, st);
+    }
+    if (trace)
+        fprintf(stderr, "b200lev: error alignment, pack + lev_warp_kernel (trace) + lev_align_walk_kernel, "
+                "R=%lld H=%lld P=%lld %s\n", (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
+    lev_align_set(&p, ws + L.off_trace, L.trace_pair_bytes, L.H + 31, (int*)(ws + L.off_align_ins), out,
+                  out_stride_k, out_stride_n, (int)steps);
+    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
+    if (rc == B200LEV_OK) rc = lev_launch_align_dp(p, fp, st);
     return rc;
 }
 

@@ -35,6 +35,23 @@ __host__ __device__ static inline int lev_group_bin(int r, int h, int G, int H) 
     return (LEV_GROUP_NCLS - 1 - lev_group_class(r, G)) * (H + 1) + (H - h);
 }
 
+// b200lev_error_counts / b200lev_error_alignment: the short form (lev_counts.cuh, one lane per
+// pair from the raw tokens) takes references up to 64 tokens of the hypotheses' width; the long
+// form (K0 + lev_warp_kernel) everything else
+static inline bool lev_counts_short_form(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp) {
+    return ref->T <= 64 && ref->elem_bytes == hyp->elem_bytes;
+}
+
+// b200lev_error_alignment, long form: lev_warp_kernel's fixed strip widths (C columns per lane:
+// one uint16 of 2-bit choices for int32 cells, one byte for fp32 cells) and the trace bytes of
+// one pair, [strip][anti-diagonal step][lane] with H + 31 steps per strip
+#define LEV_ALIGN_C_INT 8
+#define LEV_ALIGN_C_FLT 4
+static inline int64_t lev_align_pair_bytes(int64_t R, int64_t H, int C) {
+    const int64_t W = 32 * C;
+    return (R + W) / W * (H + 31) * 32 * (C / 4);
+}
+
 // Workspace layout (device scratch supplied by the caller).  All offsets are
 // multiples of 128 bytes.
 struct LevLayout {
@@ -56,10 +73,14 @@ struct LevLayout {
     size_t off_bv_counter;
     // pack kernel, few long sequences: [N first-eos words][ceil(N / 32) tickets] per side
     size_t off_split_ref, off_split_hyp;
+    // error alignment (kind 3): the cells' 2-bit choices -- short form [row][word][pair], long
+    // form trace_pair_bytes per pair -- and, long form, the insertion count of each pair
+    size_t off_trace, off_align_ins;
+    int64_t trace_pair_bytes;
     size_t bytes;
 };
 
-// kind: 0 = final value, 1 = completion (mask mode), 2 = prefix table
+// kind: 0 = final value, 1 = completion (mask mode), 2 = prefix table, 3 = error alignment
 static inline LevLayout lev_layout(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                                    int kind, int exclude_last) {
     const int for_completion = (kind == 1);
@@ -105,6 +126,19 @@ static inline LevLayout lev_layout(const b200lev_tokens_t* ref, const b200lev_to
     }
     L.off_split_ref = take(sizeof(int32_t) * (size_t)(L.Nref + (L.Nref + 31) / 32));
     L.off_split_hyp = take(sizeof(int32_t) * (size_t)(L.P + (L.P + 31) / 32));
+    L.off_trace = L.off_align_ins = 0;
+    L.trace_pair_bytes = 0;
+    if (kind == B200LEV_WS_ALIGN) {
+        if (lev_counts_short_form(ref, hyp)) {
+            L.off_trace = take(sizeof(uint32_t) * (size_t)(L.R <= 32 ? 2 : 4) * L.H * L.P);
+        } else {
+            const int64_t bi = lev_align_pair_bytes(L.R, L.H, LEV_ALIGN_C_INT);
+            const int64_t bf = lev_align_pair_bytes(L.R, L.H, LEV_ALIGN_C_FLT);
+            L.trace_pair_bytes = bi > bf ? bi : bf;
+            L.off_trace = take((size_t)L.trace_pair_bytes * L.P);
+            L.off_align_ins = take(sizeof(int32_t) * (size_t)L.P);
+        }
+    }
     L.bytes = o;
     return L;
 }
@@ -127,15 +161,19 @@ struct LevParams {
     float padding;
     // FINAL: out[n];  PREFIX: out[i*out_si + n*out_sn];  error counts (lev_launch_counts_dp): int64
     // (C, S, D, I) of pair n at ((int64_t*)out)[4n .. 4n+3]
+    // ALIGN (the long form of b200lev_error_alignment, lev_align_set below): out holds the int8 ops,
+    // out_si / out_sn their step / pair strides and Hout the steps per pair.  The FINAL-mode
+    // instantiations of K1 with TRACE read these five fields and dbits, umax, Hr and Hr16 with the
+    // alignment's meaning: a new FINAL-mode use of any of them must not reach that path.
     float* out;
     int64_t out_si, out_sn;
     int Hout;
     // MASK
     const int32_t* uid;  // [Nref][Rp] rank of ref[j] among the pair's distinct tokens
     const int32_t* ndist;  // [Nref] number of distinct tokens of the reference
-    uint32_t* dbits;     // [Hout][P][Wd]
+    uint32_t* dbits;     // [Hout][P][Wd]  (ALIGN: the choice trace)
     int Wd;
-    int* umax;
+    int* umax;           // (ALIGN: the insertions of each pair)
     int* flags;            // caller's warning flags (may be NULL)
     const int* wide_flag;  // never NULL: workspace state words K0 fills: [0] flags (incl.
                            // B200LEV_FLAG_WIDE_TOKENS), [1], [2] biased token range
@@ -155,9 +193,32 @@ struct LevParams {
     int* gmeta_order;  // same storage viewed as int[P]: pair order of the CTA kernel
     int32_t* raw32;          // [P][Hr]   raw prefix rows (32-bit group path)
     unsigned short* raw16;   // [P][Hr16] same storage, packed path
-    int64_t Hr, Hr16;
+    int64_t Hr, Hr16;  // (ALIGN: trace bytes per pair, step slots per strip)
     int nbins;
 };
+// Error alignment, long form (lev_launch_align_dp), in the fields final mode leaves unused (so
+// the struct, and every kernel that takes it, stays as it is): lev_warp_kernel's per-cell choices
+// (lev_align_trace, lev_align_pair_bytes per pair, lev_align_ns steps per strip), the insertions
+// of each pair, and the ops the walk writes (int8, step k of pair n at ops[k*sk + n*sn], k < Tout)
+#define lev_align_trace(p) reinterpret_cast<unsigned char*>((p).dbits)
+#define lev_align_ins(p) ((p).umax)
+#define lev_align_pair_bytes_of(p) ((p).Hr)
+#define lev_align_ns(p) ((p).Hr16)
+#define lev_align_ops(p) reinterpret_cast<int8_t*>((p).out)
+#define lev_align_ops_sk(p) ((p).out_si)
+#define lev_align_ops_sn(p) ((p).out_sn)
+#define lev_align_tout(p) ((p).Hout)
+static inline void lev_align_set(LevParams* p, void* trace, int64_t pair_bytes, int64_t ns, int* ins,
+                                 int8_t* ops, int64_t sk, int64_t sn, int tout) {
+    p->dbits = reinterpret_cast<uint32_t*>(trace);
+    p->Hr = pair_bytes;
+    p->Hr16 = ns;
+    p->umax = ins;
+    p->out = reinterpret_cast<float*>(ops);
+    p->out_si = sk;
+    p->out_sn = sn;
+    p->Hout = tout;
+}
 
 
 #if defined(__CUDACC__) || defined(B200LEV_EMU)
@@ -215,6 +276,14 @@ int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st);
 int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                             const b200lev_opts_t* o, const LevParams& p, bool float_path,
                             int64_t* out, cudaStream_t st);
+// b200lev_error_alignment: K1 with the choice trace, then the walk (lev_dp.cu / lev_align.cuh),
+// after K0; and the short form with its trace (lev_counts.cuh).  `trace` is the workspace
+// region the layout of kind 3 gives.
+int lev_launch_align_dp(const LevParams& p, bool float_path, cudaStream_t st);
+int lev_align_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                           const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                           uint32_t* trace, int8_t* ops, int64_t ops_sk, int64_t ops_sn,
+                           cudaStream_t st);
 // lanes per pair if the shapes admit the group kernel (its histogram is then built at
 // pack time), else 0
 int lev_group_eligible(int64_t R, int64_t H, int64_t P);

@@ -19,6 +19,10 @@
 // hypothesis token; a hypothesis token outside int32 equals no reference token of a warp that
 // takes the fast path.
 //
+// TRACE (b200lev_error_alignment): each row also packs its cells' choices as 2-bit op codes
+// (lev_align.cuh) into RM / 16 words, stored [row][word][pair]; after the last row the lane walks
+// its own trace back from (h, r) and writes the ops instead of the counts.
+//
 // Compiled as part of lev_dp.cu (included once, at its end), next to the long form.
 #pragma once
 #include "lev_arith.cuh"
@@ -37,6 +41,14 @@ struct LevCountsArgs {
     float ins_f, del_f, sub_f;
     int64_t* out;   // [P][4]
     int32_t* flags;  // may be NULL
+};
+// TRACE: the choice rows ([H][RM / 16][P] words) and the ops (step k of pair n at
+// ops[k*ops_sk + n*ops_sn], k < Tout = R + H)
+struct LevAlignArgs : LevCountsArgs {
+    uint32_t* trace;
+    int8_t* ops;
+    int64_t ops_sk, ops_sn;
+    int Tout;
 };
 
 template <typename V>
@@ -58,9 +70,24 @@ template <bool EXACT>
 struct LevCntPath {
     static constexpr bool value = EXACT;
 };
+// TRACE: the path tag also carries where the next row's choice words go (the lambdas below name
+// no other state for the trace, so the instantiations without it stay as they were)
+template <bool EXACT>
+struct LevCntTracePath {
+    static constexpr bool value = EXACT;
+    uint32_t* row;  // word 0 of the next row; word k at row[k * P]
+};
+template <bool TRACE, int NW>
+struct LevRowTrace {
+    unsigned w[NW] = {};
+};
+template <int NW>
+struct LevRowTrace<false, NW> {};
 
-template <typename TT, typename V, int RM>
-__global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(const LevCountsArgs a) {
+template <typename TT, typename V, int RM, bool TRACE = false>
+__global__ void __launch_bounds__(32 * LEV_CNT_WARPS)
+    lev_counts_short_kernel(const typename std::conditional<TRACE, LevAlignArgs, LevCountsArgs>::type a) {
+    constexpr int NW = RM / 16;  // TRACE: words per row
     constexpr bool IS_INT = std::is_same<V, int>::value;
     const int lane = threadIdx.x & 31;
     const int64_t nblocks = (a.P + 31) / 32;
@@ -141,6 +168,8 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
             w[0] = w[0] + 256u;
             V left = v[0];
             unsigned lw = w[0];
+            LevRowTrace<TRACE, NW> tr;  // TRACE: this row's choices
+            (void)tr;
 #pragma unroll
             for (int j = 1; j <= RM; ++j) {
                 unsigned neq;
@@ -159,12 +188,19 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
                 const bool keep = del_c >= c;  // SM:309
                 c = keep ? c : del_c;
                 cw = keep ? cw : lw;
+                if constexpr (TRACE) tr.w[(j - 1) >> 4] |= (keep ? (ps ? neq : 3u) : 2u) << (2 * ((j - 1) & 15));
                 diag = up;
                 dw = uw;
                 left = c;
                 lw = cw;
                 v[j] = c;
                 w[j] = cw;
+            }
+            if constexpr (TRACE) {
+                if (path.row != nullptr) {  // (NULL: a lane past the batch)
+#pragma unroll
+                    for (int k = 0; k < NW; ++k) path.row[(int64_t)k * a.P] = tr.w[k];
+                }
             }
         };
         // the hypothesis, CH rows per trip: the CH loads go out together
@@ -191,6 +227,9 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
                     if (in) {
                         ++hlen;
                         row(path, x);
+                        if constexpr (TRACE) {
+                            if (path.row != nullptr) path.row += (int64_t)NW * a.P;
+                        }
                     }
                 }
                 if (!__any_sync(LEV_FULL_MASK, live)) break;  // every hypothesis of the warp ended
@@ -198,10 +237,18 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
         };
         bool exact = false;
         if (sizeof(TT) == 8) exact = __any_sync(LEV_FULL_MASK, wide);
-        if (exact)
-            hypothesis(LevCntPath<true>{});
-        else
-            hypothesis(LevCntPath<false>{});
+        if constexpr (TRACE) {
+            uint32_t* const row0 = pair < a.P ? a.trace + pair : nullptr;
+            if (exact)
+                hypothesis(LevCntTracePath<true>{row0});
+            else
+                hypothesis(LevCntTracePath<false>{row0});
+        } else {
+            if (exact)
+                hypothesis(LevCntPath<true>{});
+            else
+                hypothesis(LevCntPath<false>{});
+        }
         if (a.has_eos && a.include_eos && live) myflags |= B200LEV_FLAG_HYP_NO_EOS;
 
         // ---- cell (h, r) ---------------------------------------------------------------------
@@ -210,7 +257,15 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
         for (int j = 0; j <= RM; ++j) wf = j == rlen ? w[j] : wf;
         const int ni = (int)(wf >> 8), ns = (int)(wf & 255u);
         const int nd = ni + rlen - hlen;
-        if (pair < a.P) {
+        if constexpr (TRACE) {
+            if (pair < a.P) {
+                LevTraceRows t;
+                t.base = a.trace + pair;
+                t.row_stride = (int64_t)NW * a.P;
+                t.word_stride = a.P;
+                lev_align_walk(t, hlen, rlen, rlen + ni, a.Tout, a.ops + pair * a.ops_sn, a.ops_sk);
+            }
+        } else if (pair < a.P) {
             int64_t* __restrict__ o = a.out + pair * 4;
             o[0] = hlen - ns - ni;
             o[1] = ns;
@@ -224,28 +279,37 @@ __global__ void __launch_bounds__(32 * LEV_CNT_WARPS) lev_counts_short_kernel(co
 }
 
 // ---- host side ---------------------------------------------------------------------------------
-template <typename TT, typename V>
-static void lev_counts_launch_t(const LevCountsArgs& a, cudaStream_t st) {
+template <typename TT, typename V, bool TRACE>
+static void lev_counts_launch_t(const LevAlignArgs& a_, cudaStream_t st) {
+    const typename std::conditional<TRACE, LevAlignArgs, LevCountsArgs>::type& a = a_;
     const int64_t n = (a.P + 32 * LEV_CNT_WARPS - 1) / (32 * LEV_CNT_WARPS);
     const int64_t cap = (int64_t)148 * 16;
     const dim3 grid((unsigned)(n < cap ? n : cap)), block(32 * LEV_CNT_WARPS);
     if (a.R <= 32)
-        lev_launch(lev_counts_short_kernel<TT, V, 32>, grid, block, 0, st, a);
+        lev_launch(lev_counts_short_kernel<TT, V, 32, TRACE>, grid, block, 0, st, a);
     else
-        lev_launch(lev_counts_short_kernel<TT, V, 64>, grid, block, 0, st, a);
+        lev_launch(lev_counts_short_kernel<TT, V, 64, TRACE>, grid, block, 0, st, a);
 }
 
 template <typename TT>
-static void lev_counts_launch_tt(const LevCountsArgs& a, bool float_path, cudaStream_t st) {
-    if (float_path)
-        lev_counts_launch_t<TT, float>(a, st);
-    else
-        lev_counts_launch_t<TT, int>(a, st);
+static void lev_counts_launch_tt(const LevAlignArgs& a, bool float_path, bool trace, cudaStream_t st) {
+    if (trace) {
+        if (float_path)
+            lev_counts_launch_t<TT, float, true>(a, st);
+        else
+            lev_counts_launch_t<TT, int, true>(a, st);
+    } else {
+        if (float_path)
+            lev_counts_launch_t<TT, float, false>(a, st);
+        else
+            lev_counts_launch_t<TT, int, false>(a, st);
+    }
 }
 
-int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                            const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                            int64_t* out, cudaStream_t st) {
+// the two entry points' launch: `a` carries either the counts' output or the trace and the ops
+static int lev_counts_short_run(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                                const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                                LevAlignArgs& a, cudaStream_t st) {
     if (ref->T > 64) {
         lev_set_error("short error-counts form: R = %lld > 64", (long long)ref->T);
         return B200LEV_ERR_ARG;
@@ -255,8 +319,6 @@ int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t*
                       hyp->elem_bytes);
         return B200LEV_ERR_ARG;
     }
-    LevCountsArgs a;
-    memset(&a, 0, sizeof(a));
     a.ref = ref->data;
     a.hyp = hyp->data;
     a.ref_st = ref->stride_t;
@@ -275,18 +337,40 @@ int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t*
     a.ins_f = p.ins_f;
     a.del_f = p.del_f;
     a.sub_f = p.sub_f;
-    a.out = out;
     a.flags = p.flags;
     lev_prof_begin(LEV_PROF_DP, st);
     switch (ref->elem_bytes) {
-        case 8: lev_counts_launch_tt<int64_t>(a, float_path, st); break;
-        case 4: lev_counts_launch_tt<int32_t>(a, float_path, st); break;
-        case 2: lev_counts_launch_tt<int16_t>(a, float_path, st); break;
-        case 1: lev_counts_launch_tt<int8_t>(a, float_path, st); break;
+        case 8: lev_counts_launch_tt<int64_t>(a, float_path, a.trace != nullptr, st); break;
+        case 4: lev_counts_launch_tt<int32_t>(a, float_path, a.trace != nullptr, st); break;
+        case 2: lev_counts_launch_tt<int16_t>(a, float_path, a.trace != nullptr, st); break;
+        case 1: lev_counts_launch_tt<int8_t>(a, float_path, a.trace != nullptr, st); break;
         default:
             lev_set_error("token width %d bytes", ref->elem_bytes);
             return B200LEV_ERR_ARG;
     }
     lev_prof_end(LEV_PROF_DP, st);
     return lev_check_cuda("lev_counts_short_kernel");
+}
+
+int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                            const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                            int64_t* out, cudaStream_t st) {
+    LevAlignArgs a;
+    memset(&a, 0, sizeof(a));
+    a.out = out;
+    return lev_counts_short_run(ref, hyp, o, p, float_path, a, st);
+}
+
+int lev_align_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                           const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                           uint32_t* trace, int8_t* ops, int64_t ops_sk, int64_t ops_sn,
+                           cudaStream_t st) {
+    LevAlignArgs a;
+    memset(&a, 0, sizeof(a));
+    a.trace = trace;
+    a.ops = ops;
+    a.ops_sk = ops_sk;
+    a.ops_sn = ops_sn;
+    a.Tout = (int)(ref->T + hyp->T);
+    return lev_counts_short_run(ref, hyp, o, p, float_path, a, st);
 }

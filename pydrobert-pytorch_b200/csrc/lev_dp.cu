@@ -29,6 +29,7 @@
 // the rest, in the reference's operation order (including its deletion term
 // min_k v[k] + (fl(j*d) - fl(k*d)), SM:263-266,317, tracked by run origin).
 #include "lev_arith.cuh"
+#include "lev_align.cuh"
 
 // number of per-warp shared-memory columns (boundary channels + row minima)
 template <typename V, bool COUNT, int MODE, bool OPS = false>
@@ -47,6 +48,9 @@ struct LevBufs {
 // falls out of the same word.  Returns that size (valid on lane 31).
 // OPS (FINAL, COUNT only; b200lev_error_counts): one more int32 channel, the insertions along the
 // path the count cell picks, carried like the count channel; the epilogue writes (C, S, D, I).
+// TRACE (on top of OPS; b200lev_error_alignment, C = 8 or 4): every row's C choices of a lane as
+// one uint16 / byte of 2-bit op codes (lev_align.cuh) into the pair's trace, and the epilogue
+// writes the insertion count alone.
 // tokens that do not fit in int32 (B200LEV_FLAG_WIDE_TOKENS): read the caller's tensors
 // directly and compare in 64 bits.  Slow (strided gathers) but exact; uniform per launch.
 __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes, int64_t idx) {
@@ -58,7 +62,7 @@ __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes
     }
 }
 
-template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE, bool OPS>
+template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE, bool OPS, bool TRACE = false>
 __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair, const int r,
                                               const int h, const int steps,
                                               const int* __restrict__ hyp_s_,
@@ -174,6 +178,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         V dc = diag_v, dm = diag_m, lc = in_v, lm = in_m;
                         int di = diag_i, li = in_i;
                         (void)di; (void)li;
+                        unsigned tr = 0u;  // TRACE: this row's C choices
+                        (void)tr;
 #pragma unroll
                         for (int c = 0; c < C; ++c) {
                             const V uc = v[c], um = m[c];
@@ -198,12 +204,19 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                                 li = ii;
                                 ic[c] = ii;
                             }
+                            if constexpr (TRACE)
+                                tr |= (keep ? (ps ? (neq01 != (V)0 ? 1u : 0u) : 3u) : 2u) << (2 * c);
                             dc = uc;
                             dm = um;
                             lc = cc;
                             lm = mm;
                             v[c] = cc;
                             m[c] = mm;
+                        }
+                        if constexpr (TRACE) {
+                            typedef typename LevTraceStrips<C>::Field Field;
+                            reinterpret_cast<Field*>(lev_align_trace(p) + (int64_t)pair * lev_align_pair_bytes_of(p))
+                                [((int64_t)k * lev_align_ns(p) + (s - 1)) * 32 + lane] = (Field)tr;
                         }
                     } else if (FLT_COST) {
                         // SM:290-293,316-317 in fp32, deletion term by run origin:
@@ -293,13 +306,17 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
             }
         }
         if (OPS && last && lane == 31) {
-            // m = S + D + I; C + S + D = r and C + S + I = h
-            const int ins = ic[C - 1], del = ins + r - h, sub = (int)m[C - 1] - ins - del;
-            int64_t* __restrict__ o = reinterpret_cast<int64_t*>(p.out) + (int64_t)pair * 4;
-            o[0] = h - sub - ins;
-            o[1] = sub;
-            o[2] = del;
-            o[3] = ins;
+            if constexpr (TRACE) {
+                lev_align_ins(p)[pair] = ic[C - 1];
+            } else {
+                // m = S + D + I; C + S + D = r and C + S + I = h
+                const int ins = ic[C - 1], del = ins + r - h, sub = (int)m[C - 1] - ins - del;
+                int64_t* __restrict__ o = reinterpret_cast<int64_t*>(p.out) + (int64_t)pair * 4;
+                o[0] = h - sub - ins;
+                o[1] = sub;
+                o[2] = del;
+                o[3] = ins;
+            }
         } else if (MODE == LEV_MODE_FINAL && last && lane == 31) {  // SM:390-405
             p.out[pair] = lev_finalize((float)(COUNT ? m[C - 1] : v[C - 1]), p, r, h > 0);
         }
@@ -310,11 +327,11 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
 
 // Returns -1 when the largest target set still has to be counted from the bitmaps in global
 // memory (atomic pass), else that size as lane 31 saw it (chained pass).
-template <typename V, bool COUNT, int MODE, int C, bool WIDE = false, bool OPS = false>
+template <typename V, bool COUNT, int MODE, int C, bool WIDE = false, bool OPS = false, bool TRACE = false>
 __device__ __forceinline__ int lev_warp_pair_all(const LevParams& p, int pair, int r, int h,
                                                  int steps, const int* hyp_s, V* bufs, int Hs,
                                                  bool one_word) {
-    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs);
+    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs);
     if (MODE == LEV_MODE_MASK) {
         if (one_word) return lev_warp_pair<V, COUNT, MODE, C, 2, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
         lev_warp_pair<V, COUNT, MODE, C, 1, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
@@ -324,8 +341,9 @@ __device__ __forceinline__ int lev_warp_pair_all(const LevParams& p, int pair, i
 
 // CMASK: bit c set => the kernel carries a C = 2^c variant (1, 2, 4, 8); each pair
 // takes the smallest variant whose single strip covers its r + 1 columns, the largest
-// one (multi-strip) otherwise.  OPS: the error-counts epilogue (FINAL, COUNT).
-template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false>
+// one (multi-strip) otherwise.  OPS: the error-counts epilogue (FINAL, COUNT).  TRACE: the
+// error-alignment trace (with OPS; one C only, CMASK 8 or 4).
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false>
 __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     LEV_DYN_SMEM(int, smem);
     const int lane = threadIdx.x & 31;
@@ -361,16 +379,16 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
         const bool one_word = MODE == LEV_MODE_MASK && p.ndist[pair / p.ref_group] <= 32;
         int set_max = -1;
         if (wide)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true, OPS>(
+            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true, OPS, TRACE>(
                 p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 1) && (cols <= 32 || !(CMASK & 14)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 1, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 1, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 2) && (cols <= 64 || !(CMASK & 12)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 2, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 2, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 4) && (cols <= 128 || !(CMASK & 8)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 4, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 4, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if (CMASK & 8)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 8, false, OPS>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 8, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
 
         if (MODE == LEV_MODE_PREFIX) {
             // SM:279-285 (row 0) and SM:379-386 (tail := padding)
@@ -414,7 +432,7 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     }
 }
 
-template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false>
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false>
 static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
     constexpr int NB = LevBufs<V, COUNT, MODE, OPS>::NB;
     const size_t per_warp = (size_t)(2 + NB) * (size_t)((p.H + 65) & ~1) * sizeof(int);
@@ -429,7 +447,7 @@ static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
     // keep at least two CTAs per SM resident when the rows are short
     while (wpc > 1 && per_warp * wpc > 100 * 1024) --wpc;
     const size_t smem = per_warp * wpc;
-    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK, OPS>;
+    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK, OPS, TRACE>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)smem);
@@ -506,6 +524,24 @@ int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st) {
     if (p.P <= 0) return B200LEV_OK;
     if (!float_path) return lev_launch_variant<int, true, LEV_MODE_FINAL, 10, true>(p, st);
     return lev_launch_variant<float, true, LEV_MODE_FINAL, 4, true>(p, st);
+}
+
+// b200lev_error_alignment, the long form: K1 with the count cell, the insertion channel and the
+// choice trace at one strip width, then the walk, one thread per pair
+template <typename V, int C>
+static int lev_launch_align_t(const LevParams& p, cudaStream_t st) {
+    int rc = lev_launch_variant<V, true, LEV_MODE_FINAL, C, true, true>(p, st);
+    if (rc) return rc;
+    int64_t blocks = ((int64_t)p.P + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    lev_launch(lev_align_walk_kernel<C>, dim3((unsigned)blocks), dim3(256), 0, st, p);
+    return lev_check_cuda("lev_align_walk_kernel");
+}
+
+int lev_launch_align_dp(const LevParams& p, bool float_path, cudaStream_t st) {
+    if (p.P <= 0) return B200LEV_OK;
+    if (!float_path) return lev_launch_align_t<int, LEV_ALIGN_C_INT>(p, st);
+    return lev_launch_align_t<float, LEV_ALIGN_C_FLT>(p, st);
 }
 
 // the short form (R <= 64): one lane per pair from the raw tokens
