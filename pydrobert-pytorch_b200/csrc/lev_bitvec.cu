@@ -99,8 +99,10 @@ int lev_bitvec_launch(LevBvRoute route, const b200lev_tokens_t* ref, const b200l
     a.hyp_len = (int32_t*)(ws + L.off_hyp_len);
     a.counter = (int*)(ws + L.off_bv_counter);
     a.flags = p.flags;
-    a.slots_log2 = 4;  // buckets of 4 ways: on average at most one token per bucket
-    while ((1 << a.slots_log2) < a.R) ++a.slots_log2;
+    // buckets of 4 ways: on average at most one token per bucket; a key's low s bits hold a
+    // position or R (no match), so 2^s > R
+    a.slots_log2 = 4;
+    while ((1 << a.slots_log2) <= a.R) ++a.slots_log2;
     a.mode = mode;
     a.norm = o->norm;
     a.exclude_last = mode == LEV_MODE_PREFIX ? o->exclude_last : 0;

@@ -4,7 +4,6 @@
 #pragma once
 #include "lev_common.cuh"
 
-#define LEV_BV_EMPTY ((int)0x80000000)  // key of a free way (a token with this value: exact path)
 constexpr int LEV_BV_NT = 4;  // tables per warp = runs of identical references per pass
 
 struct LevBvArgs {
@@ -21,7 +20,7 @@ struct LevBvArgs {
     int32_t* flags;    // caller's warning flags, may be NULL
     int32_t* state;  // workspace state words; [3] != 0 = "not for this path" (lev_bv_took)
     int check_state;   // device-selected mode: veto through state[3] instead of multi-pass
-    int slots_log2;    // hash buckets per table (power of two >= R), 4 ways each
+    int slots_log2;    // s: 2^s hash buckets per table, 4 ways each; 2^s > R (positions fit s bits)
     int mode, norm, exclude_last, Hout;
     float mult, padding;
     float* out;
@@ -29,18 +28,33 @@ struct LevBvArgs {
     double* acc;     // FINAL, short-reference kernel: += [sum(out), sum(ref_len per pair), #pairs] (may be NULL)
 };
 
-// Bucketed hash: 4 ways per bucket, one 128-bit read of the keys and one 32-bit read of the
-// position bytes settle a probe -- no loop, so 32 lanes with 32 different tokens cost the same
-// as one.  A run leader builds its table with the first of a few multipliers under which no
-// bucket overflows (load <= 1 token per bucket on average: a couple of tries at most).
-// (a build with R = 128 distinct tokens in 128 buckets fails with p = 0.38: 16 tries leave
-// 2e-7 of the runs to the slow exact path; the typical R ~ 100 needs 1.2 tries on average)
+// Bucketed hash: 4 ways per bucket.  x = v * mult (odd mult: a bijection on 32 bits) picks the
+// bucket with its top s bits, and its low 32 - s bits -- the residual -- tell apart every int32
+// token of that bucket.  A way holds (x << s) | position, so ONE 128-bit read of the bucket and
+// four DPX add-mins settle a look-up (lev_bv_row): no loop, no position side table, and 32 lanes
+// with 32 different tokens cost the same as one.  A run leader builds its table with the first
+// of a few multipliers under which no bucket overflows (load <= 1 token per bucket on average: a
+// couple of tries at most).
+// (a build with R = 127 distinct tokens in 128 buckets fails with p = 0.35: 16 tries leave
+// 6e-8 of the runs to the slow exact path; R = 128 has 256 buckets, p = 0.04; the typical
+// R ~ 100 needs 1.2 tries on average)
 constexpr int LEV_BV_TRIES = 16;
 __device__ __forceinline__ unsigned lev_bv_mult(int seed) {
     return (0x9E3779B1u * (2u * (unsigned)seed + 1u)) ^ ((unsigned)seed * 0x85EBCA6Au);
 }
-__device__ __forceinline__ unsigned lev_bv_hash(int v, unsigned mult, int buckets_log2) {
-    return ((unsigned)v * mult) >> (32 - buckets_log2);
+// A free way holds the all-ones residual and position z = R (the all-zero row of the match
+// masks): a token with that residual reads z from it, which is right as long as no real way
+// holds it -- and a real way with that residual holds a position < R, which the min prefers.
+__device__ __forceinline__ unsigned lev_bv_free_way(int s, int z) { return (~0u << s) | (unsigned)z; }
+// The row of a token: nx = -(x << s) (= v * (mult * -2^s), one multiply), z = R < 2^s.  A way's
+// key + nx is its position when the residuals agree and >= 2^s otherwise, so the min over the
+// four ways and z is the position of the way holding the token, or z.  The table build stops at
+// the way this picks, so the build and the look-ups agree on it.
+__device__ __forceinline__ unsigned lev_bv_row(const uint4 k, unsigned nx, unsigned z) {
+    unsigned u = __viaddmin_u32(k.x, nx, z);
+    u = __viaddmin_u32(k.y, nx, u);
+    u = __viaddmin_u32(k.z, nx, u);
+    return __viaddmin_u32(k.w, nx, u);
 }
 
 // Runs of identical references inside a block of 32 consecutive pairs, from each lane's
@@ -107,20 +121,22 @@ int lev_bvfused_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st, void
 
 // The lanes of a run build its hash table together (warp-collective: every lane calls it).
 // Lane i of a run of n lanes takes positions i, i + n, ...: it claims a free way of the token's
-// bucket with a CAS on the key word (an equal key already there = duplicate), then writes its
-// position byte.  Which occurrence ends up representing a token is a race, and does not
-// matter: a position byte only has to be the SAME for every occurrence and for the hypothesis
-// look-ups, which all read the finished table.  Positions past the eos may get in too: their
-// rows receive no bits, so matching them is no match.  A build whose bucket overflows is
-// retried under the next multiplier.  Returns 1 if the run has no usable table (tokens outside
-// int32, or LEV_BV_TRIES overflowing builds): the caller compares tokens one by one.
+// bucket with a CAS, and stops early at a way whose residual is the token's (a duplicate).
+// Which occurrence ends up representing a token is a race, and does not matter: a position only
+// has to be the SAME for every occurrence and for the hypothesis look-ups, which all read the
+// finished table.  Positions past the eos may get in too: their rows receive no bits, so matching
+// them is no match.  A build whose bucket overflows is retried under the next multiplier.
+// Returns 1 if the run has no usable table (tokens outside int32, or LEV_BV_TRIES overflowing
+// builds): the caller compares tokens one by one.
 template <typename TT>
-__device__ __forceinline__ int lev_bv_build_table(const LevBvArgs& a, int4* keys4, unsigned* posw,
-                                                  const int nb, const TT* __restrict__ rsrc,
-                                                  const int rst, const LevBvRuns& runs,
-                                                  const bool active, const int tb, const int run_pos,
-                                                  const int exact0, const int lane, int* seed_out) {
+__device__ __forceinline__ int lev_bv_build_table(const LevBvArgs& a, uint4* keys4, const int nb,
+                                                  const TT* __restrict__ rsrc, const int rst,
+                                                  const LevBvRuns& runs, const bool active,
+                                                  const int tb, const int run_pos, const int exact0,
+                                                  const int lane, int* seed_out) {
     constexpr int NT = LEV_BV_NT;
+    const int s = a.slots_log2;
+    const unsigned efree = lev_bv_free_way(s, a.R);
     int seed = 0;
     int exact = exact0;
     bool need = active && !exact;
@@ -133,15 +149,13 @@ __device__ __forceinline__ int lev_bv_build_table(const LevBvArgs& a, int4* keys
         if (clear == 0) break;
         __syncwarp();
         for (int i = lane; i < nb * NT; i += 32)
-            if ((clear >> (i % NT)) & 1u) {
-                keys4[i] = make_int4(LEV_BV_EMPTY, LEV_BV_EMPTY, LEV_BV_EMPTY, LEV_BV_EMPTY);
-                posw[i] = (unsigned)a.R * 0x01010101u;  // free ways point at the all-zero row
-            }
+            if ((clear >> (i % NT)) & 1u) keys4[i] = make_uint4(efree, efree, efree, efree);
         __syncwarp();
-        bool overflow = false, hopeless = false;
+        bool overflow = false;
         if (need) {
             seed = attempt;
             const unsigned hmul = lev_bv_mult(seed);
+            const unsigned lim = 1u << s;
             for (int t0 = run_pos; t0 < a.R; t0 += 8 * runs.len) {
                 int vv[8];  // 8 of my positions at a time: the loads overlap
 #pragma unroll
@@ -151,21 +165,13 @@ __device__ __forceinline__ int lev_bv_build_table(const LevBvArgs& a, int4* keys
                 for (int k = 0; k < 8; ++k) {
                     const int t = t0 + k * runs.len;
                     if (t >= a.R) break;
-                    const int v = vv[k];
-                    if (v == LEV_BV_EMPTY) {  // the one token value a key word cannot hold
-                        hopeless = true;
-                        continue;
-                    }
-                    const int idx = (int)lev_bv_hash(v, hmul, a.slots_log2) * NT + tb;
-                    int* kk = reinterpret_cast<int*>(&keys4[idx]);
+                    const unsigned x = (unsigned)vv[k] * hmul;
+                    const unsigned key = (x << s) | (unsigned)t;
+                    unsigned* kk = reinterpret_cast<unsigned*>(&keys4[(int)(x >> (32 - s)) * NT + tb]);
                     int w = 0;
                     for (; w < 4; ++w) {
-                        const int old = atomicCAS(&kk[w], LEV_BV_EMPTY, v);
-                        if (old == LEV_BV_EMPTY) {
-                            reinterpret_cast<unsigned char*>(&posw[idx])[w] = (unsigned char)t;
-                            break;
-                        }
-                        if (old == v) break;
+                        const unsigned old = atomicCAS(&kk[w], efree, key);
+                        if (old == efree || old - (x << s) < lim) break;  // claimed / the token is there
                     }
                     overflow |= w == 4;
                 }
@@ -173,12 +179,7 @@ __device__ __forceinline__ int lev_bv_build_table(const LevBvArgs& a, int4* keys
         }
         // the run retries (next multiplier) if any of its lanes met a full bucket
         const bool run_bad = (__ballot_sync(LEV_FULL_MASK, overflow) & runs.mask) != 0;
-        const bool run_hopeless = (__ballot_sync(LEV_FULL_MASK, hopeless) & runs.mask) != 0;
         need = need && run_bad;
-        if (active && run_hopeless) {
-            need = false;
-            exact = 1;
-        }
         if (need && attempt == LEV_BV_TRIES - 1) {
             need = false;
             exact = 1;

@@ -11,10 +11,10 @@
 //      compares with its left neighbour), first eos, "needs 64-bit compares" (lev_bvf_scan)
 //   B  per run, its lanes build ONE bucketed hash table token -> first-claimed position
 //      (lev_bv_build_table, lev_bitvec.cuh), then set, for every reference position, its bit in
-//      the match mask Peq[position byte] of the run (shared-memory atomicOr)
+//      the match mask Peq[position] of the run (shared-memory atomicOr)
 //   C  every lane streams ITS hypothesis column (rows of 32 neighbouring pairs: one coalesced
 //      256-byte load per row, two halves of 8 rows in flight), and per token: hash -> 128-bit
-//      read of the bucket's keys -> position byte -> 128-bit read of Peq -> Myers step ->
+//      read of the bucket's keys -> position (lev_bv_row) -> 128-bit read of Peq -> Myers step ->
 //      one output row (32 neighbouring pairs: one 128-byte store).  The eos / length logic of
 //      SM:195-228 and the freezing of SM:286-288 run inside the stream: a lane stops stepping
 //      at its first eos, rows beyond become `padding`.
@@ -29,12 +29,11 @@
 #include "lev_bitvec.cuh"
 
 #ifndef LEV_BVF_WARPS_PER_CTA
-#define LEV_BVF_WARPS_PER_CTA 4
+#define LEV_BVF_WARPS_PER_CTA 4  // at most: fewer where the tables of that many do not fit (host)
 #endif
 #ifndef LEV_BVF_CTAS_PER_SM
 #define LEV_BVF_CTAS_PER_SM 3  // resident CTAs per SM the launch bounds and the grid are sized for
 #endif
-constexpr int LEV_BVF_WARPS = LEV_BVF_WARPS_PER_CTA;
 // tuning switches (scripts/gpu_ab.sh builds one library per setting)
 #ifndef LEV_BVF_NBUF
 #define LEV_BVF_NBUF 4  // chunk buffers of the hypothesis stream: loads run NBUF - 1 trips ahead
@@ -182,8 +181,8 @@ __device__ __forceinline__ LevBvfScan lev_bvf_scan(const LevBvArgs& a, const TT*
 // compute -- and store -- exactly what that pair's own lane does, so nothing in here is
 // predicated on "is my pair real".
 template <typename TT, int W, int KIND>
-__device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, unsigned* posw,
-                                              unsigned* M, const int nb, const int tab_words,
+__device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, uint4* keys4, unsigned* M,
+                                              const int nb, const int tab_words,
                                               const int64_t block, const int64_t next_block,
                                               const bool first_block, const int lane) {
     constexpr int NT = LEV_BV_NT;
@@ -261,18 +260,18 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
 
         // ---- B: the run's hash table, then its match masks -----------------------------------
         int seed = 0;
-        const int exact = lev_bv_build_table<TT>(a, keys4, posw, nb, rsrc, rst, runs, active, tb,
-                                                 run_pos, scan.wide ? 1 : 0, lane, &seed);
+        const int exact = lev_bv_build_table<TT>(a, keys4, nb, rsrc, rst, runs, active, tb, run_pos,
+                                                 scan.wide ? 1 : 0, lane, &seed);
         {
             uint4* mz = reinterpret_cast<uint4*>(M);
             for (int i = lane; i < tab_words / 4; i += 32) mz[i] = make_uint4(0u, 0u, 0u, 0u);
         }
         __syncwarp();
         const unsigned hmul = lev_bv_mult(seed);
+        const unsigned nmul = hmul * (0u - (1u << a.slots_log2));  // v * nmul = -(x << s)
         const int hshift = 32 - a.slots_log2;
-        // my run's slice of the tables: bucket b is keys_tb[b * NT] / posw_tb[b * NT]
-        const int4* __restrict__ keys_tb = keys4 + tb;
-        const unsigned* __restrict__ posw_tb = posw + tb;
+        // my run's slice of the tables: bucket b is keys_tb[b * NT]
+        const uint4* __restrict__ keys_tb = keys4 + tb;
         const unsigned* __restrict__ M_tb = M + tb * W;
         if (active && !exact) {
             for (int t0 = run_pos; t0 < rlen; t0 += 8 * runs.len) {
@@ -284,16 +283,9 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
                 for (int k = 0; k < 8; ++k) {
                     const int t = t0 + k * runs.len;
                     if (t >= rlen) break;
-                    const int v = vv[k];
-                    const int bk = (int)(((unsigned)v * hmul) >> hshift) * NT;
-                    const int4 kk = keys_tb[bk];
-                    const unsigned pw = posw_tb[bk];
-                    int sel = 0x5554;  // first matching way, the rule the hypothesis look-ups use too
-                    if (kk.w == v) sel = 0x5553;
-                    if (kk.z == v) sel = 0x5552;
-                    if (kk.y == v) sel = 0x5551;
-                    if (kk.x == v) sel = 0x5550;
-                    const unsigned u = __byte_perm(pw, (unsigned)Z, sel);
+                    const unsigned v = (unsigned)vv[k];
+                    // the rule the hypothesis look-ups use too
+                    const unsigned u = lev_bv_row(keys_tb[(int)((v * hmul) >> hshift) * NT], v * nmul, Z);
                     const int b = t + o;
                     atomicOr(&M[(u * NT + tb) * W + (b >> 5)], 1u << (b & 31));
                 }
@@ -370,20 +362,12 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
                 score += (down_s - up_s) & in_m;
             }
         };
-        // the run's table: one 128-bit read of the bucket's keys + one 32-bit read of its
-        // position bytes settle a look-up -- no probe loop.  The selector picks the position
-        // byte of the matching way, or the byte Z (= the all-zero row) when no way matches.
+        // the run's table: one 128-bit read of the bucket's keys settles a look-up -- no probe
+        // loop; a token no way holds reads row Z (= the all-zero row)
         auto row_hashed = [&](int64_t, int v, int hi) -> const unsigned* {
-            const int bk = (int)(((unsigned)v * hmul) >> hshift) * NT;
-            const int4 kk = keys_tb[bk];
-            const unsigned pw = posw_tb[bk];
-            int sel = 0x5554;
-            sel = kk.w == v ? 0x5553 : sel;
-            sel = kk.z == v ? 0x5552 : sel;
-            sel = kk.y == v ? 0x5551 : sel;
-            sel = kk.x == v ? 0x5550 : sel;
-            if (sizeof(TT) == 8) sel = hi != (v >> 31) ? 0x5554 : sel;  // not an int32 token: no key equals it
-            const unsigned u = __byte_perm(pw, (unsigned)Z, sel);
+            const unsigned uv = (unsigned)v;
+            unsigned u = lev_bv_row(keys_tb[(int)((uv * hmul) >> hshift) * NT], uv * nmul, Z);
+            if (sizeof(TT) == 8) u = hi != (v >> 31) ? (unsigned)Z : u;  // not an int32 token: no key holds it
             return M_tb + u * (NT * W);
         };
         auto row_exact = [&](int64_t x, int, int) -> const unsigned* {
@@ -501,22 +485,19 @@ __device__ __forceinline__ void lev_bvf_block(const LevBvArgs& a, int4* keys4, u
 }
 
 // Warps are independent: each takes the block of 32 pairs of its own index, then claims further
-// blocks from a global counter.  Per warp: keys [nb][NT] int4 (4 ways), posw [nb][NT] words
-// (4 position bytes), M [(R + 1)][NT][W] words.
+// blocks from a global counter.  Per warp: keys [nb][NT] uint4 (4 ways), M [(R + 1)][NT][W] words.
 template <typename TT, int W, int KIND>
-__global__ void __launch_bounds__(32 * LEV_BVF_WARPS, LEV_BVF_CTAS_PER_SM) lev_bv_fused_kernel(const LevBvArgs a) {
+__global__ void __launch_bounds__(32 * LEV_BVF_WARPS_PER_CTA, LEV_BVF_CTAS_PER_SM) lev_bv_fused_kernel(const LevBvArgs a) {
     if (a.check_state && !lev_bv_took(a.state)) return;  // the probe handed the batch back
-    LEV_DYN_SMEM(int, smem);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    LEV_DYN_SMEM(unsigned, smem);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
     const int nb = 1 << a.slots_log2;
     const int tab_words = ((a.R + 1) * W * LEV_BV_NT + 3) & ~3;
-    int* mine = smem + (size_t)warp * (nb * LEV_BV_NT * 5 + tab_words);
-    int4* keys4 = reinterpret_cast<int4*>(mine);
-    unsigned* posw = reinterpret_cast<unsigned*>(keys4 + nb * LEV_BV_NT);
-    unsigned* M = posw + nb * LEV_BV_NT;
+    uint4* keys4 = reinterpret_cast<uint4*>(smem + (size_t)warp * (nb * LEV_BV_NT * 4 + tab_words));
+    unsigned* M = reinterpret_cast<unsigned*>(keys4 + nb * LEV_BV_NT);
     const int64_t nblocks = ((int64_t)a.P + 31) / 32;
-    const int64_t stride = (int64_t)gridDim.x * LEV_BVF_WARPS;
-    const int64_t first = (int64_t)blockIdx.x * LEV_BVF_WARPS + warp;
+    const int64_t stride = (int64_t)gridDim.x * warps;
+    const int64_t first = (int64_t)blockIdx.x * warps + warp;
     // The first block of a warp is its own; further ones are claimed from a counter (zeroed by
     // the probe or a memset), one block AHEAD so that the stream of the current block can
     // announce the next one to L2.  A warp's blocks take different times (ragged hypotheses,
@@ -534,7 +515,7 @@ __global__ void __launch_bounds__(32 * LEV_BVF_WARPS, LEV_BVF_CTAS_PER_SM) lev_b
     bool first_block = true;
     while (block >= 0) {
         const int64_t next = claim();
-        lev_bvf_block<TT, W, KIND>(a, keys4, posw, M, nb, tab_words, block, next, first_block, lane);
+        lev_bvf_block<TT, W, KIND>(a, keys4, M, nb, tab_words, block, next, first_block, lane);
         block = next;
         first_block = false;
     }
@@ -575,8 +556,8 @@ __global__ void __launch_bounds__(128) lev_bv_probe_kernel(const LevBvArgs a, co
 // ---- host side ---------------------------------------------------------------------------------
 // every resident slot gets a CTA (the warps walk the blocks with a grid stride; a warp of a
 // big batch takes 2-3 blocks, and a full machine during the early rounds beats equal shares)
-static unsigned lev_bvf_grid(int64_t P, int per_sm) {
-    const int64_t n = (P + 32 * LEV_BVF_WARPS - 1) / (32 * LEV_BVF_WARPS);
+static unsigned lev_bvf_grid(int64_t P, int warps, int per_sm) {
+    const int64_t n = (P + 32 * warps - 1) / (32 * warps);
     int64_t cap = (int64_t)148 * per_sm;
     if (const char* e = getenv("B200LEV_BVF_CTAS")) cap = atoll(e) > 0 ? atoll(e) : cap;  // tests
     return (unsigned)(n < cap ? n : cap);
@@ -586,8 +567,14 @@ template <typename TT, int W>
 static void lev_bvf_launch_w(const LevBvArgs& a, cudaStream_t st) {
     const int nb = 1 << a.slots_log2;
     const int tab_words = ((a.R + 1) * W * LEV_BV_NT + 3) & ~3;
-    const size_t smem = sizeof(int) * (size_t)(nb * LEV_BV_NT * 5 + tab_words) * LEV_BVF_WARPS;
-    const dim3 grid(lev_bvf_grid(a.P, LEV_BVF_CTAS_PER_SM)), block(32 * LEV_BVF_WARPS);
+    const size_t warp_bytes = sizeof(unsigned) * (size_t)(nb * LEV_BV_NT * 4 + tab_words);
+    // as many warps per CTA (up to the launch bounds') as let LEV_BVF_CTAS_PER_SM CTAs share the
+    // 228 KB of an SM (1 KB of it reserved per CTA): at R = 128 the 256-bucket tables take 3
+    const size_t per_cta = 228 * 1024 / LEV_BVF_CTAS_PER_SM - 1024;
+    int warps = (int)(per_cta / warp_bytes);
+    warps = warps < 1 ? 1 : (warps > LEV_BVF_WARPS_PER_CTA ? LEV_BVF_WARPS_PER_CTA : warps);
+    const size_t smem = warp_bytes * warps;
+    const dim3 grid(lev_bvf_grid(a.P, warps, LEV_BVF_CTAS_PER_SM)), block(32 * warps);
     auto go = [&](auto kern) {
         if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         lev_launch(kern, grid, block, smem, st, a);
