@@ -20,8 +20,9 @@
  *    8 bytes (signed) are accepted, int64 being the reference's ("long tensor",
  *    SM:588-596).
  *  - `flags` (device int32[1], may be NULL) receives an OR of B200LEV_FLAG_*: the
- *    data-dependent conditions behind the reference's three warnings.  The host
- *    reads it back only when `warn=True` (one 4-byte D2H).
+ *    data-dependent conditions behind the reference's three warnings (the host
+ *    reads it back only when `warn=True`, one 4-byte D2H) and behind the error the
+ *    reference raises for a loss target that is not a class.
  */
 #ifndef B200LEV_H_
 #define B200LEV_H_
@@ -33,7 +34,7 @@
 extern "C" {
 #endif
 
-#define B200LEV_ABI_VERSION 2
+#define B200LEV_ABI_VERSION 3
 
 #define B200LEV_OK 0
 #define B200LEV_ERR_ARG (-1)       /* bad argument (shape, stride, dtype, NULL) */
@@ -48,6 +49,9 @@ extern "C" {
 #define B200LEV_FLAG_HYP_NO_EOS 2
 #define B200LEV_FLAG_EMPTY_REF 4
 #define B200LEV_FLAG_WIDE_TOKENS 8
+/* b200lev_ocd_forward: a target outside [0, V) other than ignore_index (torch's cross_entropy
+ * raises "Target t is out of bounds."); the kernels skip such targets and read nothing for them */
+#define B200LEV_FLAG_BAD_TARGET 16
 
 /* A borrowed, strided 2-D token view: element (t, n) of a (T, N) "sequence first"
  * tensor lives at data + (t*stride_t + n*stride_n) * elem_bytes.  A batch_first
@@ -176,23 +180,26 @@ int b200lev_completion_fill(const b200lev_tokens_t *ref, const b200lev_tokens_t 
  * optimal_completion(padding=ignore_index, exclude_last=True).
  *   logits : (A, B, V) element (a, b, v) at logits[a*ls_a + b*ls_b + v]   (dtype code)
  *   targets: int64 (A, B, U) element at targets[a*ts_a + b*ts_b + u]
- *   weight : NULL or float[V]
+ *   weight : NULL or V class weights in the ACCUMULATION type (see below): float[V], or
+ *            double[V] when dtype is F64
  *   seq_axis: 0 if A is the hypothesis axis (seq-first), 1 if B is (batch_first)
  * Scratch/outputs are in the ACCUMULATION type: fp32, or fp64 when dtype is F64.
  * Forward writes per[A*B] (row-major (a, b)), lse[A*B], and -- for mean/sum -- the
  * scalar loss[0] plus denom[] (per-sequence number of steps with targets, length =
  * size of the non-sequence axis).  Backward reads grad_out (accumulation type; one
  * element for mean/sum, A*B for none) and writes grad_logits (dtype of logits,
- * contiguous (A, B, V)).
+ * contiguous (A, B, V)).  A target outside [0, V) other than ignore_index is skipped; the
+ * forward ORs B200LEV_FLAG_BAD_TARGET into *flags (device int32[1], may be NULL) for it.
  */
 int b200lev_ocd_forward(const void *logits, int32_t dtype, int64_t A, int64_t B, int64_t V,
                         int64_t ls_a, int64_t ls_b, const int64_t *targets, int64_t U,
-                        int64_t ts_a, int64_t ts_b, const float *weight,
+                        int64_t ts_a, int64_t ts_b, const void *weight,
                         int64_t ignore_index, int32_t reduction, int32_t seq_axis,
-                        void *per, void *lse, void *denom, void *loss, void *stream);
+                        void *per, void *lse, void *denom, void *loss, int32_t *flags,
+                        void *stream);
 int b200lev_ocd_backward(const void *logits, int32_t dtype, int64_t A, int64_t B, int64_t V,
                          int64_t ls_a, int64_t ls_b, const int64_t *targets, int64_t U,
-                         int64_t ts_a, int64_t ts_b, const float *weight,
+                         int64_t ts_a, int64_t ts_b, const void *weight,
                          int64_t ignore_index, int32_t reduction, int32_t seq_axis,
                          const void *lse, const void *denom, const void *grad_out,
                          void *grad_logits, void *stream);

@@ -276,7 +276,7 @@ def hard_optimal_completion_distillation_loss(
     """SM:1188-1251 in float64.  Returns ``(loss, dloss/dlogits)``; for
     ``reduction='none'`` the gradient is taken for ``sum(loss * grad_output)``
     (``grad_output`` defaults to ones)."""
-    lg = np.asarray(logits.detach().cpu().float().numpy() if hasattr(logits, "detach")
+    lg = np.asarray(logits.detach().cpu().double().numpy() if hasattr(logits, "detach")
                     else logits).astype(np.float64)
     hyp_np = _np_tokens(hyp)
     if lg.ndim != 3:
@@ -300,8 +300,9 @@ def hard_optimal_completion_distillation_loss(
     tgc = np.where(valid, tg, 0)
     picked = np.take_along_axis(lg, tgc, axis=2)  # (A, B, U)
     wt = w[tgc] * valid
-    # cross_entropy(reduction='none', weight) = w[t] * (lse - logit[t])   SM:1232-1238
-    per = (wt * (lse[..., None] - picked)).sum(2) / np.maximum(cnt, 1)  # SM:1239-1241
+    # cross_entropy(reduction='none', weight) = w[t] * (lse - logit[t]), and 0 at ignore_index even
+    # where the stand-in class 0 of an ignored slot has a -inf logit   SM:1232-1238
+    per = np.where(valid, wt * (lse[..., None] - picked), 0.0).sum(2) / np.maximum(cnt, 1)  # SM:1239-1241
     seq_dim = 1 if batch_first else 0
     sm = np.exp(lg - lse[..., None])
     # d per / d logits = (sum_t w_t / cnt) * softmax - scatter(w_t / cnt)
@@ -335,7 +336,7 @@ def minimum_error_rate_loss(
     grad_output=None,
 ) -> Tuple[np.ndarray, np.ndarray]:
     """SM:1400-1472 with the softmax/reduction in float64.  Returns ``(loss, dloss/dlog_probs)``."""
-    lp = np.asarray(log_probs.detach().cpu().float().numpy() if hasattr(log_probs, "detach")
+    lp = np.asarray(log_probs.detach().cpu().double().numpy() if hasattr(log_probs, "detach")
                     else log_probs).astype(np.float64)
     ref, hyp = _np_tokens(ref), _np_tokens(hyp)
     if lp.ndim != 2:

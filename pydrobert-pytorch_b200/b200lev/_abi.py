@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libb200lev.so")
 
 OK = 0
-FLAG_REF_NO_EOS, FLAG_HYP_NO_EOS, FLAG_EMPTY_REF, FLAG_WIDE_TOKENS = 1, 2, 4, 8
+FLAG_REF_NO_EOS, FLAG_HYP_NO_EOS, FLAG_EMPTY_REF, FLAG_WIDE_TOKENS, FLAG_BAD_TARGET = 1, 2, 4, 8, 16
 F32, F16, BF16, F64 = 0, 1, 2, 3
 REDUCE = {"none": 0, "mean": 1, "sum": 2}
 
@@ -54,7 +54,7 @@ SIGNATURES = {
                                                c_i64, c_vp]),
     "b200lev_ocd_forward": (ctypes.c_int, [c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_i64, c_vp,
                                            c_i64, c_i64, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp,
-                                           c_vp, c_vp, c_vp, c_vp]),
+                                           c_vp, c_vp, c_vp, c_vp, c_vp]),
     "b200lev_ocd_backward": (ctypes.c_int, [c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_i64, c_vp,
                                             c_i64, c_i64, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp,
                                             c_vp, c_vp, c_vp, c_vp]),
@@ -111,7 +111,7 @@ def lib() -> ctypes.CDLL:
                 "b200lev has no CPU fallback."
             )
         _lib = _bind(ctypes.CDLL(LIB_PATH))
-        if _lib.b200lev_abi_version() != 2:
+        if _lib.b200lev_abi_version() != 3:
             raise B200LevError("libb200lev.so ABI version mismatch")
     return _lib
 

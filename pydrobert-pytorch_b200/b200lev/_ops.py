@@ -342,32 +342,48 @@ def _rowmajor_last(t: Tensor) -> Tensor:
     return t if t.stride(-1) == 1 or t.size(-1) <= 1 else t.contiguous()
 
 
-def _weight_on(w: Optional[Tensor], dev: torch.device) -> Optional[Tensor]:
-    return None if w is None else w.detach().to(device=dev, dtype=torch.float32).contiguous()
+def _check_weight(w: Optional[Tensor], V: int) -> None:
+    # the kernels read weight[t] for every target t in [0, V)
+    if w is not None and (w.dim() != 1 or w.size(0) != V):
+        raise RuntimeError(f"weight tensor should be defined either for all {V} classes or no classes but "
+                           f"got weight tensor of shape: {list(w.shape)}")
+
+
+def _weight_on(w: Optional[Tensor], dev: torch.device, acc: torch.dtype) -> Optional[Tensor]:
+    """The class weights as the kernels read them: in the accumulation dtype of the logits."""
+    return None if w is None else w.detach().to(device=dev, dtype=acc).contiguous()
 
 
 def ocd_loss_impl(logits: Tensor, targets: Tensor, weight: Optional[Tensor], ignore_index: int,
                   reduction: int, seq_axis: int) -> Tuple[Tensor, Tensor, Tensor]:
     """_string.py:1229-1251 given the optimal-completion targets.  Returns
-    ``(loss, lse, denom)`` (lse/denom are saved for the backward)."""
+    ``(loss, lse, denom)`` (lse/denom are saved for the backward).  A target outside [0, V)
+    other than ``ignore_index`` raises IndexError, as cross_entropy does (_string.py:1232-1238):
+    the kernel flags it, read back with one 4-byte D2H."""
     pl = _host.Placement(logits, targets)
     dev = pl.dev
     A, B, V = logits.shape
     U = targets.size(-1)
+    _check_weight(weight, V)
     logits = _rowmajor_last(pl.to_dev(logits.detach()))
     targets = pl.to_dev(targets).contiguous()
     acc = _acc_dtype(logits)
-    w = _weight_on(weight, dev)
+    w = _weight_on(weight, dev, acc)
     per = torch.empty((A, B), dtype=acc, device=dev)
     lse = torch.empty((A, B), dtype=acc, device=dev)
     denom = torch.empty(max(B if seq_axis == 0 else A, 1), dtype=acc, device=dev)
-    loss = torch.zeros((), dtype=acc, device=dev)
+    loss = torch.empty((), dtype=acc, device=dev)  # written by the reduction whenever it is returned
+    flags = torch.zeros(1, dtype=torch.int32, device=dev)
     with _DeviceGuard(dev):
         _abi.check(_abi.lib().b200lev_ocd_forward(
             logits.data_ptr(), _float_code(logits), A, B, V, logits.stride(0), logits.stride(1),
             targets.data_ptr(), U, targets.stride(0), targets.stride(1),
             None if w is None else w.data_ptr(), ignore_index, reduction, seq_axis,
-            per.data_ptr(), lse.data_ptr(), denom.data_ptr(), loss.data_ptr(), _stream(dev)))
+            per.data_ptr(), lse.data_ptr(), denom.data_ptr(), loss.data_ptr(), flags.data_ptr(),
+            _stream(dev)))
+    if int(flags.item()) & _abi.FLAG_BAD_TARGET:
+        bad = targets[(targets != ignore_index) & ((targets < 0) | (targets >= V))]
+        raise IndexError(f"Target {int(bad[0])} is out of bounds.")
     out = per if reduction == 0 else loss
     return pl.back(out.to(logits.dtype)), pl.back(lse), pl.back(denom)
 
@@ -377,7 +393,8 @@ ocd_loss = torch.library.custom_op("b200lev::ocd_loss", ocd_loss_impl, mutates_a
 
 @ocd_loss.register_fake
 def _(logits, targets, weight, ignore_index, reduction, seq_axis):
-    A, B, _ = logits.shape
+    A, B, V = logits.shape
+    _check_weight(weight, V)
     acc = _acc_dtype(logits)
     out = logits.new_empty((A, B) if reduction == 0 else ())
     return out, logits.new_empty((A, B), dtype=acc), logits.new_empty(
@@ -394,7 +411,7 @@ def ocd_loss_backward_impl(grad_out: Tensor, logits: Tensor, targets: Tensor, we
     logits = _rowmajor_last(pl.to_dev(logits.detach()))
     targets = pl.to_dev(targets).contiguous()
     acc = _acc_dtype(logits)
-    w = _weight_on(weight, dev)
+    w = _weight_on(weight, dev, acc)
     go = grad_out.detach().to(device=dev, dtype=acc).contiguous()
     lse, denom = lse.to(dev), denom.to(dev)
     grad = torch.empty((A, B, V), dtype=logits.dtype, device=dev)

@@ -60,9 +60,10 @@ template <int DT>
 __global__ void __launch_bounds__(256)
 lev_ocd_fwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t rows, int64_t B,
                    int64_t V, int64_t ls_a, int64_t ls_b, const int64_t* __restrict__ targets,
-                   int64_t U, int64_t ts_a, int64_t ts_b, const float* __restrict__ weight,
-                   int64_t ignore_index, typename LevElem<DT>::Acc* __restrict__ per,
-                   typename LevElem<DT>::Acc* __restrict__ lse_out) {
+                   int64_t U, int64_t ts_a, int64_t ts_b,
+                   const typename LevElem<DT>::Acc* __restrict__ weight, int64_t ignore_index,
+                   typename LevElem<DT>::Acc* __restrict__ per,
+                   typename LevElem<DT>::Acc* __restrict__ lse_out, int32_t* __restrict__ flags) {
     typedef typename LevElem<DT>::Acc A;
     const int lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -85,11 +86,14 @@ lev_ocd_fwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t r
     int cnt = 0;
     for (int64_t u = lane; u < U; u += 32) {
         const int64_t t = tg[u];
-        if (t != ignore_index) {
-            const A w = weight ? (A)weight[t] : (A)1;
-            acc += w * (lse - (A)LevElem<DT>::ld(z + t));  // SM:1232-1238
-            cnt += 1;
+        if (t == ignore_index) continue;
+        if (t < 0 || t >= V) {  // not a class: reported (the reference raises), never read
+            if (flags) atomicOr(flags, B200LEV_FLAG_BAD_TARGET);
+            continue;
         }
+        const A w = weight ? weight[t] : (A)1;
+        acc += w * (lse - (A)LevElem<DT>::ld(z + t));  // SM:1232-1238
+        cnt += 1;
     }
     acc = lev_warp_sum(acc);
     cnt = lev_warp_sum(cnt);
@@ -168,8 +172,9 @@ template <int DT>
 __global__ void __launch_bounds__(256)
 lev_ocd_bwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t rows, int64_t B,
                    int64_t V, int64_t ls_a, int64_t ls_b, const int64_t* __restrict__ targets,
-                   int64_t U, int64_t ts_a, int64_t ts_b, const float* __restrict__ weight,
-                   int64_t ignore_index, int reduction, int seq_axis, int64_t nseq,
+                   int64_t U, int64_t ts_a, int64_t ts_b,
+                   const typename LevElem<DT>::Acc* __restrict__ weight, int64_t ignore_index,
+                   int reduction, int seq_axis, int64_t nseq,
                    const typename LevElem<DT>::Acc* __restrict__ lse_in,
                    const typename LevElem<DT>::Acc* __restrict__ denom,
                    const typename LevElem<DT>::Acc* __restrict__ grad_out,
@@ -193,8 +198,8 @@ lev_ocd_bwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t r
     int cnt = 0;
     for (int64_t u = lane; u < U; u += 32) {
         const int64_t t = tg[u];
-        if (t != ignore_index) {
-            wsum += weight ? (A)weight[t] : (A)1;
+        if (t != ignore_index && t >= 0 && t < V) {  // the forward reports the others
+            wsum += weight ? weight[t] : (A)1;
             cnt += 1;
         }
     }
@@ -209,8 +214,8 @@ lev_ocd_bwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t r
     // the targets of one row are distinct (sorted-unique), so these stores do not collide
     for (int64_t u = lane; u < U; u += 32) {
         const int64_t t = tg[u];
-        if (t != ignore_index) {
-            const A w = weight ? (A)weight[t] : (A)1;
+        if (t != ignore_index && t >= 0 && t < V) {
+            const A w = weight ? weight[t] : (A)1;
             LevElem<DT>::st(g + t, coef * lev_exp<A>((A)LevElem<DT>::ld(z + t) - lse) - go * w * inv);
         }
     }
@@ -219,16 +224,16 @@ lev_ocd_bwd_kernel(const typename LevElem<DT>::T* __restrict__ logits, int64_t r
 template <int DT>
 static int lev_ocd_forward_t(const void* logits, int64_t A_, int64_t B, int64_t V, int64_t ls_a,
                              int64_t ls_b, const int64_t* targets, int64_t U, int64_t ts_a,
-                             int64_t ts_b, const float* weight, int64_t ignore_index,
+                             int64_t ts_b, const void* weight, int64_t ignore_index,
                              int reduction, int seq_axis, void* per, void* lse, void* denom,
-                             void* loss, cudaStream_t st) {
+                             void* loss, int32_t* flags, cudaStream_t st) {
     typedef typename LevElem<DT>::Acc A;
     const int64_t rows = A_ * B;
     if (rows > 0) {
         dim3 block(256), grid((unsigned)((rows + 7) / 8));
         lev_launch(lev_ocd_fwd_kernel<DT>, grid, block, 0, st,
                    (const typename LevElem<DT>::T*)logits, rows, B, V, ls_a, ls_b, targets, U, ts_a,
-                   ts_b, weight, ignore_index, (A*)per, (A*)lse);
+                   ts_b, (const A*)weight, ignore_index, (A*)per, (A*)lse, flags);
     }
     if (reduction != B200LEV_REDUCE_NONE)
         lev_launch(lev_ocd_reduce_kernel<A>, dim3(1), dim3(1024), 0, st, (const A*)per, A_, B, targets,
@@ -239,7 +244,7 @@ static int lev_ocd_forward_t(const void* logits, int64_t A_, int64_t B, int64_t 
 template <int DT>
 static int lev_ocd_backward_t(const void* logits, int64_t A_, int64_t B, int64_t V, int64_t ls_a,
                               int64_t ls_b, const int64_t* targets, int64_t U, int64_t ts_a,
-                              int64_t ts_b, const float* weight, int64_t ignore_index,
+                              int64_t ts_b, const void* weight, int64_t ignore_index,
                               int reduction, int seq_axis, const void* lse, const void* denom,
                               const void* grad_out, void* grad, cudaStream_t st) {
     typedef typename LevElem<DT>::Acc A;
@@ -247,7 +252,7 @@ static int lev_ocd_backward_t(const void* logits, int64_t A_, int64_t B, int64_t
     if (rows <= 0) return B200LEV_OK;
     dim3 block(256), grid((unsigned)((rows + 7) / 8));
     lev_launch(lev_ocd_bwd_kernel<DT>, grid, block, 0, st, (const typename LevElem<DT>::T*)logits,
-               rows, B, V, ls_a, ls_b, targets, U, ts_a, ts_b, weight, ignore_index, reduction,
+               rows, B, V, ls_a, ls_b, targets, U, ts_a, ts_b, (const A*)weight, ignore_index, reduction,
                seq_axis, seq_axis == 0 ? B : A_, (const A*)lse, (const A*)denom, (const A*)grad_out,
                (typename LevElem<DT>::T*)grad);
     return lev_check_cuda("lev_ocd_bwd_kernel");
@@ -266,12 +271,13 @@ static int lev_ocd_backward_t(const void* logits, int64_t A_, int64_t B, int64_t
 
 extern "C" int b200lev_ocd_forward(const void* logits, int32_t dtype, int64_t A, int64_t B,
                                    int64_t V, int64_t ls_a, int64_t ls_b, const int64_t* targets,
-                                   int64_t U, int64_t ts_a, int64_t ts_b, const float* weight,
+                                   int64_t U, int64_t ts_a, int64_t ts_b, const void* weight,
                                    int64_t ignore_index, int32_t reduction, int32_t seq_axis,
-                                   void* per, void* lse, void* denom, void* loss, void* stream) {
+                                   void* per, void* lse, void* denom, void* loss, int32_t* flags,
+                                   void* stream) {
 #define CALL(DT)                                                                                  \
     lev_ocd_forward_t<DT>(logits, A, B, V, ls_a, ls_b, targets, U, ts_a, ts_b, weight,            \
-                          ignore_index, reduction, seq_axis, per, lse, denom, loss,               \
+                          ignore_index, reduction, seq_axis, per, lse, denom, loss, flags,        \
                           (cudaStream_t)stream)
     LEV_DT_SWITCH(dtype, CALL)
 #undef CALL
@@ -279,7 +285,7 @@ extern "C" int b200lev_ocd_forward(const void* logits, int32_t dtype, int64_t A,
 
 extern "C" int b200lev_ocd_backward(const void* logits, int32_t dtype, int64_t A, int64_t B,
                                     int64_t V, int64_t ls_a, int64_t ls_b, const int64_t* targets,
-                                    int64_t U, int64_t ts_a, int64_t ts_b, const float* weight,
+                                    int64_t U, int64_t ts_a, int64_t ts_b, const void* weight,
                                     int64_t ignore_index, int32_t reduction, int32_t seq_axis,
                                     const void* lse, const void* denom, const void* grad_out,
                                     void* grad_logits, void* stream) {

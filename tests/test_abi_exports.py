@@ -13,9 +13,10 @@ def _declared():
     return sorted(set(re.findall(r"\b(b200lev_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_abi_v2_header_symbols_are_exported_and_bound():
-    """ABI version 2: every symbol the header declares is exported and bound, and the entry points
-    version 2 retired are no longer exported."""
+def test_abi_v3_header_symbols_are_exported_and_bound():
+    """ABI version 3 (the class weight of the OCD loss in the accumulation type, and its
+    out-of-range target flag): every symbol the header declares is exported and bound, and the
+    entry points version 2 retired are no longer exported."""
     import __graft_entry__ as entry
     from b200lev import _abi
 
@@ -27,7 +28,7 @@ def test_abi_v2_header_symbols_are_exported_and_bound():
         assert hasattr(lib, n), f"{n} declared in b200lev.h but not exported"
         assert n in _abi.SIGNATURES, f"{n} has no ctypes signature in _abi.py"
     assert set(_abi.SIGNATURES) == set(names)
-    assert _abi.lib().b200lev_abi_version() == 2
+    assert _abi.lib().b200lev_abi_version() == 3
     for n in ("b200lev_pack", "b200lev_final_packed", "b200lev_prefix_packed",
               "b200lev_workspace_ref_lens", "b200lev_workspace_hyp_lens", "b200lev_err_sum"):
         assert not hasattr(lib, n), f"{n} is still exported"
