@@ -109,6 +109,26 @@ int b200lev_final(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
                   size_t workspace_bytes, int32_t *flags, void *stream);
 
 /*
+ * Every reference of a group against every hypothesis of it: ref holds G groups of A sequences
+ * (ref->N = G*A, reference (g, a) is column g*A + a) and hyp G groups of B (hyp->N = G*B,
+ * hypothesis (g, b) is column g*B + b).  out[(g*A + a)*B + b] is b200lev_final of reference
+ * column g*A + a against hypothesis column g*B + b with the same opts, bit for bit, without the
+ * cross product being materialised by the caller.  opts as for b200lev_final; ref_group must be 1.
+ * G*A*B must be below 2^31.  Where b200lev_final would send the expanded pairs to the short-reference
+ * kernel (unit costs after SM:168-174, ref->T <= 64, equal token widths, unit batch strides) that
+ * kernel reads the hypotheses in place; otherwise the expanded (hyp->T, G*A*B) hypotheses are
+ * gathered into the workspace first.  out: device float[G*A*B].
+ * Workspace: b200lev_final_cross_workspace_bytes(ref, hyp, A, B, opts) -- the costs decide the
+ * route and so the size; it is b200lev_workspace_bytes of the expanded pairs, plus
+ * hyp->T * G*A*B * hyp->elem_bytes (rounded up) and 128 bytes on the gather route.
+ */
+size_t b200lev_final_cross_workspace_bytes(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
+                                           int64_t A, int64_t B, const b200lev_opts_t *opts);
+int b200lev_final_cross(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp, int64_t A, int64_t B,
+                        const b200lev_opts_t *opts, float *out, void *workspace, size_t workspace_bytes,
+                        int32_t *flags, void *stream);
+
+/*
  * prefix_error_rates (SM:520-550) / prefix_edit_distances (SM:553-583).
  *   out: device float, element (i, n) at out[i*out_stride_i + n*out_stride_n],
  *        i in [0, H+1) or [0, H) when exclude_last.
@@ -216,6 +236,19 @@ int b200lev_mwer_forward(const float *er, const void *log_probs, int32_t dtype, 
 int b200lev_mwer_backward(const float *er, const void *log_probs, int32_t dtype, int64_t N,
                           int64_t M, int64_t lp_sn, int64_t lp_sm, int32_t sub_avg,
                           int32_t reduction, const void *grad_out, void *grad, void *stream);
+
+/*
+ * Minimum-Bayes-risk selection over N n-best lists of M hypotheses (decoding only, no gradient).
+ *   er: float[N*M*M] from b200lev_final_cross of the hypotheses against themselves (A = B = M):
+ *       er[(n*M + a)*M + i] scores hypothesis i against hypothesis a as the reference.
+ *   log_probs (N, M) strided, dtype code.
+ * p = softmax(log_probs[n]) in the accumulation type (fp32; fp64 for F64), rounded to the dtype;
+ * risk[n*M + i] = sum over a of p_a * er[n, a, i] (dtype of log_probs, contiguous (N, M)); every
+ * column is summed in the same order, so identical hypotheses get bitwise identical risks.
+ * best[n] (int64) = the arg min of risk[n, :], equal risks to the lowest index.  M >= 1.
+ */
+int b200lev_mbr(const float *er, const void *log_probs, int32_t dtype, int64_t N, int64_t M,
+                int64_t lp_sn, int64_t lp_sm, void *risk, int64_t *best, void *stream);
 
 /* b200lev_final and the bulk-scoring totals in one call: `out` as b200lev_final, and
  * acc[0] += sum(out), acc[1] += sum over pairs of the reference length, acc[2] += #pairs (fp64

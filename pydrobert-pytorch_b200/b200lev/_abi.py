@@ -63,6 +63,9 @@ SIGNATURES = {
     "b200lev_mwer_backward": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_i32,
                                              c_i32, c_vp, c_vp, c_vp]),
     "b200lev_final_sums": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp, c_vp]),
+    "b200lev_final_cross_workspace_bytes": (c_sz, [_PT, _PT, c_i64, c_i64, _PO]),
+    "b200lev_final_cross": (ctypes.c_int, [_PT, _PT, c_i64, c_i64, _PO, c_vp, c_vp, c_sz, c_vp, c_vp]),
+    "b200lev_mbr": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "b200lev_error_counts": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_error_alignment": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_i64, c_i64, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_after_eos_mask": (ctypes.c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp]),

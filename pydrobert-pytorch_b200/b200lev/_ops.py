@@ -271,6 +271,127 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
 
 
 # ---------------------------------------------------------------------------------------
+# pairwise: every reference of a group against every hypothesis of it; minimum Bayes risk
+# ---------------------------------------------------------------------------------------
+def _pairwise_shapes(ref: Tensor, hyp: Tensor, batch_first: bool) -> Tuple[int, int, int]:
+    """``(G, A, B)`` of ``ref`` ``(R, G, A)`` and ``hyp`` ``(H, G, B)`` (``(G, A, R)`` and
+    ``(G, B, H)`` with ``batch_first``)."""
+    if ref.dim() != 3 or hyp.dim() != 3:
+        raise RuntimeError("ref and hyp must be 3 dimensional")
+    if batch_first:
+        (G, A, _), (Gh, B, _) = ref.shape, hyp.shape
+    else:
+        (_, G, A), (_, Gh, B) = ref.shape, hyp.shape
+    if G != Gh:
+        raise RuntimeError("ref and hyp group dimensions must match")
+    return G, A, B
+
+
+def _flat_tokens(t: Tensor, batch_first: bool) -> Tensor:
+    """The 3-D token tensor as the 2-D ``(T, G*K)`` (``(G*K, T)``) view the C ABI reads (a copy
+    only when the group and member axes do not merge)."""
+    if batch_first:
+        return t.reshape(t.size(0) * t.size(1), t.size(2))
+    return t.reshape(t.size(0), t.size(1) * t.size(2))
+
+
+def _pairwise_device(ref: Tensor, hyp: Tensor, dev: torch.device, G: int, A: int, B: int,
+                     eos: Optional[int], include_eos: bool, batch_first: bool, ins_cost: float,
+                     del_cost: float, sub_cost: float, norm: bool, return_mistakes: bool
+                     ) -> Tuple[Tensor, Tensor]:
+    """Device tensors in, ``(out (G, A, B) fp32, flags)`` out: one ``b200lev_final_cross`` call."""
+    out = torch.empty((G, A, B), dtype=torch.float32, device=dev)
+    flags = torch.zeros(1, dtype=torch.int32, device=dev)
+    if G * A * B == 0:
+        return out, flags
+    L = _abi.lib()
+    # (the flattened tensors may be copies: held here until the kernels are enqueued, since the
+    # token structs keep only their data pointers)
+    ref2, hyp2 = _flat_tokens(ref, batch_first), _flat_tokens(hyp, batch_first)
+    with _DeviceGuard(dev):
+        rt = _tok_struct(ref2, batch_first)
+        ht = _tok_struct(hyp2, batch_first)
+        o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, norm, False, 0, return_mistakes, 1)
+        nbytes = L.b200lev_final_cross_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), A, B,
+                                                       ctypes.byref(o))
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        _abi.check(L.b200lev_final_cross(ctypes.byref(rt), ctypes.byref(ht), A, B, ctypes.byref(o),
+                                         out.data_ptr(), ws.data_ptr(), nbytes, flags.data_ptr(),
+                                         _stream(dev)))
+    return out, flags
+
+
+def pairwise_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool, batch_first: bool,
+                  ins_cost: float, del_cost: float, sub_cost: float, norm: bool, return_mistakes: bool
+                  ) -> Tuple[Tensor, Tensor]:
+    """``(out, flags)``: ``out[g, a, b]`` (fp32 ``(G, A, B)``) is ``string_matching`` of
+    reference ``(g, a)`` against hypothesis ``(g, b)``, and the int32[1] warning flags, on the
+    device of ``ref``."""
+    G, A, B = _pairwise_shapes(ref, hyp, batch_first)
+    ref, hyp = _as_tokens(ref), _as_tokens(hyp)
+    pl = _host.Placement(ref, hyp)
+    out, flags = _pairwise_device(pl.to_dev(ref), pl.to_dev(hyp), pl.dev, G, A, B, eos, include_eos,
+                                  batch_first, ins_cost, del_cost, sub_cost, norm, return_mistakes)
+    return pl.back(out), pl.back(flags)
+
+
+pairwise = torch.library.custom_op("b200lev::pairwise", pairwise_impl, mutates_args=())
+
+
+@pairwise.register_fake
+def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, norm, return_mistakes):
+    G, A, B = _pairwise_shapes(ref, hyp, batch_first)
+    return ref.new_empty((G, A, B), dtype=torch.float32), ref.new_empty((1,), dtype=torch.int32)
+
+
+def _mbr_shapes(log_probs: Tensor, hyp: Tensor, batch_first: bool) -> Tuple[int, int]:
+    if log_probs.dim() != 2:
+        raise RuntimeError("log_probs must be 2 dimensional")
+    if hyp.dim() != 3:
+        raise RuntimeError("hyp must be 3 dimensional")
+    N, M = (hyp.size(0), hyp.size(1)) if batch_first else (hyp.size(1), hyp.size(2))
+    if log_probs.size(0) != N or log_probs.size(1) != M:
+        raise RuntimeError("ref and hyp batch_size and sample dimensions must match")
+    if M < 1:
+        raise RuntimeError(f"Batch must have at least one sample, got {M}")
+    return N, M
+
+
+def minimum_bayes_risk_impl(log_probs: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
+                            batch_first: bool, norm: bool, ins_cost: float, del_cost: float,
+                            sub_cost: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """``(best, risk, flags)``: int64 ``(N,)``, ``(N, M)`` in the dtype of ``log_probs`` and the
+    int32[1] warning flags.  Two C calls: ``b200lev_final_cross`` of the hypotheses against
+    themselves (error rates with ``norm``, edit distances without), then ``b200lev_mbr``."""
+    N, M = _mbr_shapes(log_probs, hyp, batch_first)
+    code = _float_code(log_probs)
+    hyp = _as_tokens(hyp)
+    pl = _host.Placement(log_probs, hyp)
+    dev = pl.dev
+    lp, hyp = pl.to_dev(log_probs.detach()), pl.to_dev(hyp)
+    er, flags = _pairwise_device(hyp, hyp, dev, N, M, M, eos, include_eos, batch_first, ins_cost,
+                                 del_cost, sub_cost, norm, norm)
+    risk = torch.empty((N, M), dtype=lp.dtype, device=dev)
+    best = torch.empty(N, dtype=torch.long, device=dev)
+    if N > 0:
+        with _DeviceGuard(dev):
+            _abi.check(_abi.lib().b200lev_mbr(er.data_ptr(), lp.data_ptr(), code, N, M, lp.stride(0),
+                                              lp.stride(1), risk.data_ptr(), best.data_ptr(), _stream(dev)))
+    return pl.back(best), pl.back(risk), pl.back(flags)
+
+
+minimum_bayes_risk = torch.library.custom_op("b200lev::minimum_bayes_risk", minimum_bayes_risk_impl,
+                                             mutates_args=())
+
+
+@minimum_bayes_risk.register_fake
+def _(log_probs, hyp, eos, include_eos, batch_first, norm, ins_cost, del_cost, sub_cost):
+    N, M = _mbr_shapes(log_probs, hyp, batch_first)
+    return (log_probs.new_empty((N,), dtype=torch.long), log_probs.new_empty((N, M)),
+            log_probs.new_empty((1,), dtype=torch.int32))
+
+
+# ---------------------------------------------------------------------------------------
 # optimal completion
 # ---------------------------------------------------------------------------------------
 def optimal_completion_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,

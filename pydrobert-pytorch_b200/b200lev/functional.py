@@ -34,8 +34,11 @@ __all__ = [
     "error_rate",
     "fill_after_eos",
     "hard_optimal_completion_distillation_loss",
+    "minimum_bayes_risk",
     "minimum_error_rate_loss",
     "optimal_completion",
+    "pairwise_edit_distances",
+    "pairwise_error_rates",
     "prefix_edit_distances",
     "prefix_error_rates",
     "sequence_log_probs",
@@ -304,6 +307,153 @@ def alignment_positions(ops: torch.Tensor, batch_first: bool = False) -> Tuple[t
     ref_pos = (on_ref.long().cumsum(dim) - 1).masked_fill(~on_ref, -1)
     hyp_pos = (on_hyp.long().cumsum(dim) - 1).masked_fill(~on_hyp, -1)
     return ref_pos, hyp_pos
+
+
+def _pairwise(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int],
+    include_eos: bool,
+    norm: bool,
+    batch_first: bool,
+    ins_cost: float,
+    del_cost: float,
+    sub_cost: float,
+    warn: bool,
+    return_mistakes: bool,
+) -> torch.Tensor:
+    if ref.dim() != 3 or hyp.dim() != 3:
+        raise RuntimeError("ref and hyp must be 3 dimensional")
+    if ref.size(0 if batch_first else 1) != hyp.size(0 if batch_first else 1):
+        raise RuntimeError("ref and hyp group dimensions must match")
+    uniform = (ins_cost == del_cost) and (del_cost == sub_cost) and (sub_cost > 0.0)
+    if not uniform and return_mistakes and warn:  # SM:175-180
+        warnings.warn(
+            "The behaviour for non-uniform error rates has changed after v0.3.0. "
+            "Please switch to edit_distance functions for old behaviour. Set "
+            "warn=False to suppress this warning"
+        )
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            out, flags = _ops.pairwise_impl(ref, hyp, eos, include_eos, batch_first, float(ins_cost),
+                                            float(del_cost), float(sub_cost), norm, return_mistakes)
+            if warn:
+                _warn_flags(flags, eos, include_eos, norm, False)
+            return out
+    out, flags = torch.ops.b200lev.pairwise(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost,
+                                            sub_cost, norm, return_mistakes)
+    if warn:
+        _warn_flags(flags, eos, include_eos, norm, False)
+    return out
+
+
+@script
+def pairwise_error_rates(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    norm: bool = True,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> torch.Tensor:
+    """Every reference of a group against every hypothesis of it: fp32 ``(G, A, B)``.
+
+    ``ref`` is ``(R, G, A)`` and ``hyp`` ``(H, G, B)`` (``(G, A, R)`` and ``(G, B, H)`` with
+    ``batch_first``).  ``out[g, a, b]`` is, bit for bit, :func:`error_rate` of reference
+    ``(g, a)`` against hypothesis ``(g, b)`` with the same arguments, without the ``G·A·B`` pairs
+    being materialised.  Lengths, costs and warnings are those of :func:`error_rate`.  The output's
+    shape depends on the input shapes only, so the call reads nothing back to the host (with
+    ``warn=False``)."""
+    return _pairwise(ref, hyp, eos, include_eos, norm, batch_first, ins_cost, del_cost, sub_cost,
+                     warn, True)
+
+
+@script
+def pairwise_edit_distances(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    norm: bool = False,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> torch.Tensor:
+    """:func:`pairwise_error_rates` with :func:`edit_distance` in place of :func:`error_rate`:
+    ``out[g, a, b]`` is, bit for bit, :func:`edit_distance` of reference ``(g, a)`` against
+    hypothesis ``(g, b)``."""
+    return _pairwise(ref, hyp, eos, include_eos, norm, batch_first, ins_cost, del_cost, sub_cost,
+                     warn, False)
+
+
+@script
+def minimum_bayes_risk(
+    log_probs: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = True,
+    batch_first: bool = False,
+    norm: bool = True,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Minimum-Bayes-risk selection from n-best lists: ``(best, risk)``.
+
+    ``hyp`` is ``(H, N, M)`` (``(N, M, H)`` with ``batch_first``): N lists of M hypotheses, with
+    model scores ``log_probs`` ``(N, M)``.  Each hypothesis is scored against every other one of
+    its list, which stands in for the reference::
+
+        risk[n, i] = sum_j softmax(log_probs[n])_j * er(ref=hyp[n, j], hyp=hyp[n, i])
+
+    where ``er`` is :func:`pairwise_error_rates` with these arguments (with ``norm=False``,
+    :func:`pairwise_edit_distances`).  ``best`` (int64 ``(N,)``) is the arg min of ``risk``, equal
+    risks going to the lowest index.  ``risk`` has the dtype of ``log_probs`` and is accumulated
+    in fp32 (fp64 for fp64 ``log_probs``); identical hypotheses get identical risks.  A ``-inf``
+    log-probability gives its hypothesis zero weight.  The defaults are those of
+    :func:`minimum_error_rate_loss`.
+
+    For decoding only: neither output carries a gradient."""
+    if log_probs.dim() != 2:
+        raise RuntimeError("log_probs must be 2 dimensional")
+    if hyp.dim() != 3:
+        raise RuntimeError("hyp must be 3 dimensional")
+    if batch_first:
+        batch_size, samples = hyp.size(0), hyp.size(1)
+    else:
+        batch_size, samples = hyp.size(1), hyp.size(2)
+    if log_probs.size(0) != batch_size or log_probs.size(1) != samples:
+        raise RuntimeError("ref and hyp batch_size and sample dimensions must match")
+    if samples < 1:
+        raise RuntimeError(f"Batch must have at least one sample, got {samples}")
+    uniform = (ins_cost == del_cost) and (del_cost == sub_cost) and (sub_cost > 0.0)
+    if not uniform and norm and warn:  # SM:175-180 (the error-rate form)
+        warnings.warn(
+            "The behaviour for non-uniform error rates has changed after v0.3.0. "
+            "Please switch to edit_distance functions for old behaviour. Set "
+            "warn=False to suppress this warning"
+        )
+    lp = log_probs.detach()
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            best, risk, flags = _ops.minimum_bayes_risk_impl(lp, hyp, eos, include_eos, batch_first, norm,
+                                                             float(ins_cost), float(del_cost),
+                                                             float(sub_cost))
+            if warn:
+                _warn_flags(flags, eos, include_eos, norm, False)
+            return best, risk
+    best, risk, flags = torch.ops.b200lev.minimum_bayes_risk(lp, hyp, eos, include_eos, batch_first, norm,
+                                                             ins_cost, del_cost, sub_cost)
+    if warn:
+        _warn_flags(flags, eos, include_eos, norm, False)
+    return best, risk
 
 
 def _optimal_completion(

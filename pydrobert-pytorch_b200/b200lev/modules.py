@@ -21,8 +21,11 @@ __all__ = [
     "ErrorRate",
     "FillAfterEndOfSequence",
     "HardOptimalCompletionDistillationLoss",
+    "MinimumBayesRisk",
     "MinimumErrorRateLoss",
     "OptimalCompletion",
+    "PairwiseEditDistances",
+    "PairwiseErrorRates",
     "PrefixEditDistances",
     "PrefixErrorRates",
     "SequenceLogProbabilities",
@@ -157,6 +160,67 @@ class ErrorRate(_StringMatching):
     def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
         return F.error_rate(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
                             self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class PairwiseEditDistances(_StringMatching):
+    """Every reference of a group against every hypothesis of it, as EditDistance: ``(G, A, B)``
+    (see :func:`b200lev.functional.pairwise_edit_distances`)"""
+
+    __constants__ = EditDistance.__constants__
+    norm: bool
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, norm: bool = False,
+                 batch_first: bool = False, ins_cost: float = config.DEFT_INS_COST,
+                 del_cost: float = config.DEFT_DEL_COST, sub_cost: float = config.DEFT_SUB_COST,
+                 warn: bool = True):
+        norm = argcheck.is_bool(norm, "norm")
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+        self.norm = norm
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
+        return F.pairwise_edit_distances(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
+                                         self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class PairwiseErrorRates(_StringMatching):
+    """Every reference of a group against every hypothesis of it, as ErrorRate: ``(G, A, B)``
+    (see :func:`b200lev.functional.pairwise_error_rates`)"""
+
+    __constants__ = EditDistance.__constants__
+    norm: bool
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, norm: bool = True,
+                 batch_first: bool = False, ins_cost: float = config.DEFT_INS_COST,
+                 del_cost: float = config.DEFT_DEL_COST, sub_cost: float = config.DEFT_SUB_COST,
+                 warn: bool = True):
+        norm = argcheck.is_bool(norm, "norm")
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+        self.norm = norm
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
+        return F.pairwise_error_rates(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
+                                      self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class MinimumBayesRisk(_StringMatching):
+    """Minimum-Bayes-risk selection from n-best lists: ``(best, risk)`` for ``log_probs`` ``(N, M)``
+    and ``hyp`` ``(H, N, M)`` (see :func:`b200lev.functional.minimum_bayes_risk`; decoding only,
+    no gradient)"""
+
+    __constants__ = EditDistance.__constants__
+    norm: bool
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = True, batch_first: bool = False,
+                 norm: bool = True, ins_cost: float = config.DEFT_INS_COST,
+                 del_cost: float = config.DEFT_DEL_COST, sub_cost: float = config.DEFT_SUB_COST,
+                 warn: bool = True):
+        norm = argcheck.is_bool(norm, "norm")
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+        self.norm = norm
+
+    def forward(self, log_probs: torch.Tensor, hyp: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        return F.minimum_bayes_risk(log_probs, hyp, self.eos, self.include_eos, self.batch_first, self.norm,
+                                    self.ins_cost, self.del_cost, self.sub_cost, self.warn)
 
 
 class _Prefix(_StringMatching):

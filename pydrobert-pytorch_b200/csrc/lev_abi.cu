@@ -398,6 +398,131 @@ extern "C" int b200lev_final_sums(const b200lev_tokens_t* ref, const b200lev_tok
                             flags, acc, stream);
 }
 
+// ---- b200lev_final_cross: every reference of a group against every hypothesis of it ------------
+// The call is b200lev_final on the expanded pairs p = (g, a, b) -- reference column g*A + a (the
+// n-best form, ref_group = B), hypothesis column g*B + b -- without materialising the hypotheses
+// where Ks can read them in place: exactly where lev_bitvec_route sends the expanded shape to Ks,
+// Ks runs with cross addressing.  Everything else gathers the expanded (H, P) hypotheses into the
+// workspace and runs the b200lev_final body on them unchanged.
+struct LevCross {
+    b200lev_tokens_t hx;  // the expanded hypothesis view (N = P; the data and strides of `hyp`)
+    b200lev_opts_t o;     // the caller's options with ref_group = B
+    int64_t P;
+    bool short_form;      // Ks with cross addressing; else gather + the b200lev_final body
+    size_t gather_bytes;  // the gathered hypotheses, 128-byte aligned (0 on the short form)
+};
+
+// Checks the arguments of the cross entry points and fills `c`.  B200LEV_OK, or an error status.
+static int lev_cross_plan(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int64_t A, int64_t B,
+                          const b200lev_opts_t* opts, LevCross* c) {
+    if (!ref || !hyp || !opts) {
+        lev_set_error("NULL argument");
+        return B200LEV_ERR_ARG;
+    }
+    if (A < 0 || B < 0 || ref->N < 0 || hyp->N < 0) {
+        lev_set_error("final cross: negative A (%lld), B (%lld) or batch", (long long)A, (long long)B);
+        return B200LEV_ERR_ARG;
+    }
+    if (opts->ref_group != 1) {
+        lev_set_error("final cross: ref_group must be 1, got %d", opts->ref_group);
+        return B200LEV_ERR_ARG;
+    }
+    const int64_t G = A > 0 ? ref->N / A : (B > 0 ? hyp->N / B : 0);
+    if (ref->N != G * A || (G == 0 ? hyp->N != 0 : (hyp->N % G != 0 || hyp->N / G != B))) {
+        lev_set_error("final cross: ref has %lld sequences and hyp %lld, not G*A and G*B for A = %lld, B = %lld",
+                      (long long)ref->N, (long long)hyp->N, (long long)A, (long long)B);
+        return B200LEV_ERR_ARG;
+    }
+    const int eb = hyp->elem_bytes;
+    if (eb != 1 && eb != 2 && eb != 4 && eb != 8) {
+        lev_set_error("unsupported token element size %d", eb);
+        return B200LEV_ERR_ARG;
+    }
+    const int64_t lim = (int64_t)1 << 31;  // (ref->N = G*A and B below 2^31: the product cannot overflow)
+    if (G > 0 && (ref->N >= lim || B >= lim || ref->N * B >= lim)) {
+        lev_set_error("final cross: G*A*B pairs must be fewer than 2^31");
+        return B200LEV_ERR_ARG;
+    }
+    c->P = G > 0 ? ref->N * B : 0;
+    c->hx = *hyp;
+    c->hx.N = c->P;
+    c->o = *opts;
+    c->o.ref_group = B > 0 ? (int32_t)B : 1;
+    c->o.exclude_last = 0;
+    if (c->P > 0) {  // (before the gather kernel reads anything)
+        const int rc = lev_check_tokens(ref, &c->hx, &c->o);
+        if (rc) return rc;
+    }
+    LevParams p;
+    memset(&p, 0, sizeof(p));
+    bool cm, fp;
+    lev_classify_costs(&c->o, ref->T, hyp->T, &p, &cm, &fp);
+    p.R = (int)ref->T;
+    p.H = (int)hyp->T;
+    p.P = (int)c->P;
+    p.ref_group = c->o.ref_group;
+    c->short_form = c->P > 0 && lev_bitvec_route(ref, &c->hx, LEV_MODE_FINAL, p, cm, fp) == LEV_BV_SHORT;
+    c->gather_bytes = c->short_form ? 0 : (size_t)lev_round_up((int64_t)eb * hyp->T * c->P, 128);
+    return B200LEV_OK;
+}
+
+extern "C" size_t b200lev_final_cross_workspace_bytes(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                                                      int64_t A, int64_t B, const b200lev_opts_t* opts) {
+    LevCross c;
+    if (lev_cross_plan(ref, hyp, A, B, opts, &c) != B200LEV_OK) return 0;
+    // the b200lev_final workspace of the expanded shape; the gather path puts the gathered
+    // hypotheses in front of it (and aligns both)
+    return c.gather_bytes + lev_layout(ref, &c.hx, B200LEV_WS_FINAL, 0).bytes + (c.short_form ? 128 : 256);
+}
+
+extern "C" int b200lev_final_cross(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp, int64_t A,
+                                   int64_t B, const b200lev_opts_t* opts, float* out, void* workspace,
+                                   size_t workspace_bytes, int32_t* flags, void* stream) {
+    LevCross c;
+    int rc = lev_cross_plan(ref, hyp, A, B, opts, &c);
+    if (rc) return rc;
+    if (c.P == 0) return B200LEV_OK;
+    const bool trace = getenv("B200LEV_TRACE") != nullptr;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (c.short_form) {
+        LevLayout L;
+        rc = lev_begin(ref, &c.hx, &c.o, B200LEV_WS_FINAL, out, workspace, workspace_bytes, &L);
+        if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
+        if (trace)
+            fprintf(stderr, "b200lev: final cross, short cross form (lev_bv_short_kernel CROSS), A=%lld B=%lld P=%lld\n",
+                    (long long)A, (long long)B, (long long)c.P);
+        char* ws = lev_ws_base(workspace);
+        LevParams p;
+        bool cm, fp;
+        lev_params(ref, &c.hx, &c.o, L, ws, flags, &p, &cm, &fp);
+        p.out = out;
+        return lev_bitvec_launch(LEV_BV_SHORT, ref, &c.hx, &c.o, LEV_MODE_FINAL, L, ws, p, st, nullptr, nullptr,
+                                 A, B);
+    }
+    if (!out || !workspace) {
+        lev_set_error("NULL output or workspace");
+        return B200LEV_ERR_ARG;
+    }
+    const size_t need = b200lev_final_cross_workspace_bytes(ref, hyp, A, B, opts);
+    if (workspace_bytes < need) {
+        lev_set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+        return B200LEV_ERR_WORKSPACE;
+    }
+    if (trace)
+        fprintf(stderr, "b200lev: final cross, gather + final, A=%lld B=%lld P=%lld\n", (long long)A, (long long)B,
+                (long long)c.P);
+    char* base = lev_ws_base(workspace);
+    rc = lev_launch_cross_gather(hyp, A, B, c.P, base, st);
+    if (rc) return rc;
+    b200lev_tokens_t hg = c.hx;  // the gathered view: sequence-first, contiguous
+    hg.data = base;
+    hg.stride_t = c.P;
+    hg.stride_n = 1;
+    const size_t used = (size_t)(base - (char*)workspace) + c.gather_bytes;
+    return lev_string_match(ref, &hg, &c.o, LEV_MODE_FINAL, out, 0, 0, base + c.gather_bytes,
+                            workspace_bytes - used, flags, nullptr, stream);
+}
+
 extern "C" int b200lev_prefix(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                               const b200lev_opts_t* opts, float* out, int64_t out_stride_i,
                               int64_t out_stride_n, void* workspace, size_t workspace_bytes,

@@ -92,7 +92,10 @@ __device__ __forceinline__ void lev_bvs_totals(double sum_out, int sum_len, doub
     }
 }
 
-template <typename TT, int W, int KIND>
+// CROSS (final mode, b200lev_final_cross): pair p = (g, a, b) of G groups of A x B pairs reads
+// reference column p / ref_group (ref_group = B) and hypothesis column g * B + b, both taken once
+// per pair; the lanes of a warp then read at most B distinct hypothesis columns per row.
+template <typename TT, int W, int KIND, bool CROSS>
 __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_short_kernel(const LevBvArgs a) {
     constexpr bool PREFIX = KIND != 0, EXCL = KIND == 2;
     constexpr int CH = 4;
@@ -116,8 +119,10 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
         const int64_t pair = block * 32 + lane;
         const int64_t pc = pair < a.P ? pair : (int64_t)a.P - 1;
         const int64_t rcol = pc / a.ref_group;
+        const int64_t hcol =
+            CROSS ? (int64_t)((int)pc / lev_bv_cross_ab(a) * lev_bv_cross_b(a) + (int)pc % lev_bv_cross_b(a)) : pc;
         const TT* __restrict__ rsrc = reinterpret_cast<const TT*>(a.ref) + rcol;
-        const TT* __restrict__ hsrc = reinterpret_cast<const TT*>(a.hyp) + pc;
+        const TT* __restrict__ hsrc = reinterpret_cast<const TT*>(a.hyp) + hcol;
 
         // ---- my reference column -> registers (low and high halves of the tokens, packed two
         // positions per register); its length; does it need 64-bit compares; do its tokens sit
@@ -448,12 +453,14 @@ static void lev_bvs_launch_w(const LevBvArgs& a, cudaStream_t st) {
     int64_t cap = (int64_t)148 * (W == 1 ? 20 : 16);  // whole waves of the resident CTAs (5 / 4 per SM)
     if (const char* e = getenv("B200LEV_BVS_CTAS")) cap = atoll(e) > 0 ? atoll(e) : cap;  // (tests: many blocks per warp)
     const dim3 grid((unsigned)(n < cap ? n : cap)), block(32 * LEV_BVS_WARPS);
-    if (a.mode != LEV_MODE_PREFIX)
-        lev_launch(lev_bv_short_kernel<TT, W, 0>, grid, block, 0, st, a);
+    if (lev_bv_cross_b(a) > 0)  // (final mode only)
+        lev_launch(lev_bv_short_kernel<TT, W, 0, true>, grid, block, 0, st, a);
+    else if (a.mode != LEV_MODE_PREFIX)
+        lev_launch(lev_bv_short_kernel<TT, W, 0, false>, grid, block, 0, st, a);
     else if (!a.exclude_last)
-        lev_launch(lev_bv_short_kernel<TT, W, 1>, grid, block, 0, st, a);
+        lev_launch(lev_bv_short_kernel<TT, W, 1, false>, grid, block, 0, st, a);
     else
-        lev_launch(lev_bv_short_kernel<TT, W, 2>, grid, block, 0, st, a);
+        lev_launch(lev_bv_short_kernel<TT, W, 2, false>, grid, block, 0, st, a);
 }
 
 int lev_bvshort_launch(const LevBvArgs& a, int elem_bytes, cudaStream_t st) {

@@ -308,9 +308,16 @@ LevBvRoute lev_bitvec_route(const b200lev_tokens_t* ref, const b200lev_tokens_t*
                             const LevParams& p, bool count_mode, bool float_path);
 // `ws` is the aligned workspace laid out as `L`; `acc` (final mode, may be NULL) goes to Ks.
 // With LEV_BV_SELECTED `after_probe` (a cudaEvent_t, may be NULL) is recorded once the veto is final.
+// cross_b > 0 (LEV_BV_SHORT, final mode; b200lev_final_cross): `hyp` is the expanded (H, G*A*B) view
+// of the (H, G*B) hypotheses and Ks reads hypothesis column (p / (A*B)) * B + p % B for pair p.
 int lev_bitvec_launch(LevBvRoute route, const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                       const b200lev_opts_t* o, int mode, const LevLayout& L, char* ws,
-                      const LevParams& p, cudaStream_t st, void* after_probe, double* acc);
+                      const LevParams& p, cudaStream_t st, void* after_probe, double* acc,
+                      int64_t cross_a = 0, int64_t cross_b = 0);
+// b200lev_final_cross, gather path: out (H, G*A*B), sequence-first and contiguous, column p =
+// hypothesis column (p / (A*B)) * B + p % B of `hyp` (any strides), same element width
+int lev_launch_cross_gather(const b200lev_tokens_t* hyp, int64_t A, int64_t B, int64_t P, void* out,
+                            cudaStream_t st);
 // K7 (lev_loss.cu): acc[0] += sum(er), acc[1] += sum of the pairs' reference lengths, acc[2] += P
 // (P >= 1, ref_group >= 1)
 int lev_launch_err_sum(const float* er, const int32_t* ref_lens, int64_t P, int ref_group,

@@ -434,6 +434,95 @@ extern "C" int b200lev_mwer_backward(const float* er, const void* log_probs, int
 #undef CALL
 }
 
+// ======================= minimum-Bayes-risk epilogue ===================================
+// One warp per group, next to K6 and with its softmax: p = softmax(log_probs[n]) rounded to the
+// dtype of log_probs, risk[n, i] = sum_a p_a * er[n, a, i] in the accumulation type, rounded to
+// the dtype of log_probs, best[n] = its arg min.  Lane l sums column i = i0 + l over a = 0 .. M-1
+// in that order, p_a broadcast from the lane that computed it: every column is summed in the same
+// order, so identical hypotheses get bitwise identical risks, and equal risks go to the lowest i.
+template <int DT>
+__global__ void __launch_bounds__(256)
+lev_mbr_kernel(const float* __restrict__ er, const typename LevElem<DT>::T* __restrict__ lp, int64_t N,
+               int64_t M, int64_t sn, int64_t sm, typename LevElem<DT>::T* __restrict__ risk,
+               int64_t* __restrict__ best) {
+    typedef typename LevElem<DT>::Acc A;
+    const int lane = threadIdx.x & 31;
+    const int64_t n = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (n >= N) return;
+    const typename LevElem<DT>::T* row = lp + n * sn;
+    A mx = -(A)INFINITY;
+    for (int64_t m = lane; m < M; m += 32) {
+        const A x = (A)LevElem<DT>::ld(row + m * sm);
+        mx = x > mx ? x : mx;
+    }
+    mx = lev_warp_max(mx);
+    A se = (A)0;
+    for (int64_t m = lane; m < M; m += 32) se += lev_exp<A>((A)LevElem<DT>::ld(row + m * sm) - mx);
+    se = lev_warp_sum(se);
+    const float* __restrict__ e = er + n * M * M;
+    A bv = (A)INFINITY;
+    int64_t bi = M;  // (no finite risk: 0 below)
+    for (int64_t i0 = 0; i0 < M; i0 += 32) {
+        const int64_t i = i0 + lane;
+        A acc = (A)0;
+        for (int64_t a0 = 0; a0 < M; a0 += 32) {
+            const int64_t am = a0 + lane;
+            const A pm = am < M ? LevElem<DT>::round(lev_exp<A>((A)LevElem<DT>::ld(row + am * sm) - mx) / se) : (A)0;
+            const int kn = M - a0 < 32 ? (int)(M - a0) : 32;
+            for (int k = 0; k < kn; ++k) {
+                const A pa = __shfl_sync(LEV_FULL_MASK, pm, k);
+                if (i < M) acc += pa * (A)e[(a0 + k) * M + i];
+            }
+        }
+        if (i < M) {
+            const A r = LevElem<DT>::round(acc);
+            LevElem<DT>::st(risk + n * M + i, r);
+            if (r < bv) {
+                bv = r;
+                bi = i;
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const A ov = __shfl_xor_sync(LEV_FULL_MASK, bv, o);
+        const int64_t oi = __shfl_xor_sync(LEV_FULL_MASK, bi, o);
+        if (ov < bv || (ov == bv && oi < bi)) {
+            bv = ov;
+            bi = oi;
+        }
+    }
+    if (lane == 0) best[n] = bi < M ? bi : 0;
+}
+
+template <int DT>
+static int lev_mbr_t(const float* er, const void* lp, int64_t N, int64_t M, int64_t sn, int64_t sm, void* risk,
+                     int64_t* best, cudaStream_t st) {
+    lev_launch(lev_mbr_kernel<DT>, dim3((unsigned)((N + 7) / 8)), dim3(256), 0, st, er,
+               (const typename LevElem<DT>::T*)lp, N, M, sn, sm, (typename LevElem<DT>::T*)risk, best);
+    return lev_check_cuda("lev_mbr_kernel");
+}
+
+extern "C" int b200lev_mbr(const float* er, const void* log_probs, int32_t dtype, int64_t N, int64_t M,
+                           int64_t lp_sn, int64_t lp_sm, void* risk, int64_t* best, void* stream) {
+    if (N < 0 || M < 0 || (N > 0 && M < 1)) {
+        lev_set_error("mbr: need N >= 0 and M >= 1, got N = %lld, M = %lld", (long long)N, (long long)M);
+        return B200LEV_ERR_ARG;
+    }
+    if (N == 0) return B200LEV_OK;
+    if (!er || !log_probs || !risk || !best) {
+        lev_set_error("mbr: NULL pointer");
+        return B200LEV_ERR_ARG;
+    }
+    if (N >= ((int64_t)1 << 34)) {  // (grid of N / 8 CTAs)
+        lev_set_error("mbr: too many groups");
+        return B200LEV_ERR_UNSUPPORTED;
+    }
+#define CALL(DT) lev_mbr_t<DT>(er, log_probs, N, M, lp_sn, lp_sm, risk, best, (cudaStream_t)stream)
+    LEV_DT_SWITCH(dtype, CALL)
+#undef CALL
+}
+
 // ======================= K7: bulk error sums ===========================================
 // command_line.py:1135-1147 accumulates per-utterance .item()s on the host; here the
 // three totals stay on the device in fp64 (exact for integer error counts) so that a
