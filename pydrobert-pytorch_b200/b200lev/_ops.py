@@ -187,16 +187,14 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, nor
 
 
 # ---------------------------------------------------------------------------------------
-# error counts: (C, S, D, I) per pair
+# error counts: (C, S, D, I) per pair; error alignment: the ops along the same path
 # ---------------------------------------------------------------------------------------
-def error_counts_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
-                      batch_first: bool, ins_cost: float, del_cost: float, sub_cost: float
-                      ) -> Tuple[Tensor, Tensor]:
-    """Per pair the correct, substitution, deletion and insertion counts along the path the
-    count mode of ``error_rate`` takes (_string.py:292-314), ``(out, flags)``: int64 ``(N, 4)``
-    and the int32[1] warning flags, on the device of ``ref``.  One C call
-    (``b200lev_error_counts``)."""
-    _, _, n = _shapes(ref, hyp, batch_first, 1)
+def error_path_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool, batch_first: bool,
+                ins_cost: float, del_cost: float, sub_cost: float, align: bool
+                ) -> Tuple[Tensor, Tensor]:
+    """The body of both ops below: one C call, ``b200lev_error_alignment`` if ``align`` else
+    ``b200lev_error_counts``."""
+    R, H, n = _shapes(ref, hyp, batch_first, 1)
     ref, hyp = _as_tokens(ref), _as_tokens(hyp)
     pl = _host.Placement(ref, hyp)
     ref, hyp, dev = pl.to_dev(ref), pl.to_dev(hyp), pl.dev
@@ -205,13 +203,31 @@ def error_counts_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos:
         rt, ht = _tok_struct(ref, batch_first), _tok_struct(hyp, batch_first)
         o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, False, False, 0, True, 1)
         flags = torch.zeros(1, dtype=torch.int32, device=dev)
-        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 0, 0)
+        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 3 if align else 0, 0)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        out = torch.empty((n, 4), dtype=torch.long, device=dev)
-        _abi.check(L.b200lev_error_counts(ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o),
-                                          out.data_ptr(), ws.data_ptr(), nbytes, flags.data_ptr(),
-                                          _stream(dev)))
+        toks = (ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o))
+        rest = (ws.data_ptr(), nbytes, flags.data_ptr(), _stream(dev))
+        if not align:
+            out = torch.empty((n, 4), dtype=torch.long, device=dev)
+            _abi.check(L.b200lev_error_counts(*toks, out.data_ptr(), *rest))
+        else:
+            if batch_first:
+                out = torch.empty((n, R + H), dtype=torch.int8, device=dev)
+                sk, sn = 1, R + H
+            else:
+                out = torch.empty((R + H, n), dtype=torch.int8, device=dev)
+                sk, sn = n, 1
+            _abi.check(L.b200lev_error_alignment(*toks, out.data_ptr(), sk, sn, *rest))
     return pl.back(out), pl.back(flags)
+
+
+def error_counts_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
+                      batch_first: bool, ins_cost: float, del_cost: float, sub_cost: float
+                      ) -> Tuple[Tensor, Tensor]:
+    """Per pair the correct, substitution, deletion and insertion counts along the path the
+    count mode of ``error_rate`` takes (_string.py:292-314), ``(out, flags)``: int64 ``(N, 4)``
+    and the int32[1] warning flags, on the device of ``ref``."""
+    return error_path_impl(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, False)
 
 
 error_counts = torch.library.custom_op("b200lev::error_counts", error_counts_impl, mutates_args=())
@@ -223,37 +239,14 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
     return ref.new_empty((n, 4), dtype=torch.long), ref.new_empty((1,), dtype=torch.int32)
 
 
-# ---------------------------------------------------------------------------------------
-# error alignment: the ops along the error-counts path
-# ---------------------------------------------------------------------------------------
 def error_alignment_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool,
                          batch_first: bool, ins_cost: float, del_cost: float, sub_cost: float
                          ) -> Tuple[Tensor, Tensor]:
     """Per pair the edit operations along the path ``error_counts_impl`` counts, ``(out, flags)``:
     int8 ``(R + H, N)`` (``(N, R + H)`` with ``batch_first``; 0 correct, 1 substitution,
     2 deletion, 3 insertion, -1 past the path's end) and the int32[1] warning flags, on the device
-    of ``ref``.  One C call (``b200lev_error_alignment``)."""
-    R, H, n = _shapes(ref, hyp, batch_first, 1)
-    ref, hyp = _as_tokens(ref), _as_tokens(hyp)
-    pl = _host.Placement(ref, hyp)
-    ref, hyp, dev = pl.to_dev(ref), pl.to_dev(hyp), pl.dev
-    L = _abi.lib()
-    with _DeviceGuard(dev):
-        rt, ht = _tok_struct(ref, batch_first), _tok_struct(hyp, batch_first)
-        o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, False, False, 0, True, 1)
-        flags = torch.zeros(1, dtype=torch.int32, device=dev)
-        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 3, 0)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        if batch_first:
-            out = torch.empty((n, R + H), dtype=torch.int8, device=dev)
-            sk, sn = 1, R + H
-        else:
-            out = torch.empty((R + H, n), dtype=torch.int8, device=dev)
-            sk, sn = n, 1
-        _abi.check(L.b200lev_error_alignment(ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o),
-                                             out.data_ptr(), sk, sn, ws.data_ptr(), nbytes,
-                                             flags.data_ptr(), _stream(dev)))
-    return pl.back(out), pl.back(flags)
+    of ``ref``."""
+    return error_path_impl(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, True)
 
 
 error_alignment = torch.library.custom_op("b200lev::error_alignment", error_alignment_impl,

@@ -216,6 +216,39 @@ def prefix_edit_distances(
                             sub_cost, warn, norm, True, exclude_last, padding, False, 1)
 
 
+def _error_path(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int],
+    include_eos: bool,
+    batch_first: bool,
+    ins_cost: float,
+    del_cost: float,
+    sub_cost: float,
+    warn: bool,
+    align: bool,
+) -> torch.Tensor:
+    """:func:`error_alignment` if ``align`` else :func:`error_counts`."""
+    if ref.dim() != 2 or hyp.dim() != 2:
+        raise RuntimeError("ref and hyp must be 2 dimensional")
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            out, flags = _ops.error_path_impl(ref, hyp, eos, include_eos, batch_first,
+                                              float(ins_cost), float(del_cost), float(sub_cost), align)
+            if warn:
+                _warn_flags(flags, eos, include_eos, False, False)
+            return out
+    if align:
+        out, flags = torch.ops.b200lev.error_alignment(ref, hyp, eos, include_eos, batch_first,
+                                                       ins_cost, del_cost, sub_cost)
+    else:
+        out, flags = torch.ops.b200lev.error_counts(ref, hyp, eos, include_eos, batch_first,
+                                                    ins_cost, del_cost, sub_cost)
+    if warn:
+        _warn_flags(flags, eos, include_eos, False, False)
+    return out
+
+
 @script
 def error_counts(
     ref: torch.Tensor,
@@ -238,20 +271,8 @@ def error_counts(
     reference length, ``C + S + I`` the hypothesis length and ``S + D + I`` equals
     ``error_rate(..., norm=False)`` with the same costs.  ``warn`` covers the two missing-eos
     warnings."""
-    if ref.dim() != 2 or hyp.dim() != 2:
-        raise RuntimeError("ref and hyp must be 2 dimensional")
-    if not torch.jit.is_scripting():
-        if not _ops.needs_dispatcher():
-            out, flags = _ops.error_counts_impl(ref, hyp, eos, include_eos, batch_first,
-                                                float(ins_cost), float(del_cost), float(sub_cost))
-            if warn:
-                _warn_flags(flags, eos, include_eos, False, False)
-            return out
-    out, flags = torch.ops.b200lev.error_counts(ref, hyp, eos, include_eos, batch_first, ins_cost,
-                                                del_cost, sub_cost)
-    if warn:
-        _warn_flags(flags, eos, include_eos, False, False)
-    return out
+    return _error_path(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn,
+                       False)
 
 
 @script
@@ -275,20 +296,8 @@ def error_alignment(
     Arguments, lengths and warnings are those of :func:`error_counts`.  The output's shape
     depends on the input shapes only, so the call reads nothing back to the host (with
     ``warn=False``).  :func:`alignment_positions` maps the steps to token positions."""
-    if ref.dim() != 2 or hyp.dim() != 2:
-        raise RuntimeError("ref and hyp must be 2 dimensional")
-    if not torch.jit.is_scripting():
-        if not _ops.needs_dispatcher():
-            out, flags = _ops.error_alignment_impl(ref, hyp, eos, include_eos, batch_first,
-                                                   float(ins_cost), float(del_cost), float(sub_cost))
-            if warn:
-                _warn_flags(flags, eos, include_eos, False, False)
-            return out
-    out, flags = torch.ops.b200lev.error_alignment(ref, hyp, eos, include_eos, batch_first, ins_cost,
-                                                   del_cost, sub_cost)
-    if warn:
-        _warn_flags(flags, eos, include_eos, False, False)
-    return out
+    return _error_path(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn,
+                       True)
 
 
 @script

@@ -148,31 +148,6 @@ static inline char* lev_ws_base(const void* ws) {
     return (char*)(((uintptr_t)ws + 127) & ~(uintptr_t)127);
 }
 
-// The argument prologue of the string-matching entry points: checks the token views and the
-// options, lays out the workspace for `kind` and checks the caller's buffers.  Returns LEV_EMPTY
-// when the call has nothing to write (no pairs, no output rows, or `inner` <= 0), and NULL
-// buffers are then fine; else B200LEV_OK with *L filled, or an error status (`null_status` for a
-// NULL `out` or `ws`).
-static constexpr int LEV_EMPTY = 1;
-static int lev_begin(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                     const b200lev_opts_t* o, int kind, const void* out, const void* ws,
-                     size_t ws_bytes, LevLayout* L, int64_t inner = 1,
-                     int null_status = B200LEV_ERR_ARG) {
-    const int rc = lev_check_tokens(ref, hyp, o);
-    if (rc) return rc;
-    *L = lev_layout(ref, hyp, kind, kind == B200LEV_WS_FINAL || kind == B200LEV_WS_ALIGN ? 0 : o->exclude_last);
-    if (hyp->N == 0 || L->Hout <= 0 || inner <= 0) return LEV_EMPTY;
-    if (!out || !ws) {
-        lev_set_error("NULL output or workspace");
-        return null_status;
-    }
-    if (ws_bytes < L->bytes + 128) {
-        lev_set_error("workspace too small: %zu < %zu", ws_bytes, L->bytes + 128);
-        return B200LEV_ERR_WORKSPACE;
-    }
-    return B200LEV_OK;
-}
-
 // Fills the cost fields of `p`.  Returns count_mode / float_path through the out-params.
 static void lev_classify_costs(const b200lev_opts_t* o, int64_t R, int64_t H, LevParams* p,
                                bool* count_mode, bool* float_path) {
@@ -241,6 +216,47 @@ static void lev_params(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
     p->Hr = L.Hr;
     p->Hr16 = L.Hr16;
     lev_classify_costs(o, L.R, L.H, p, count_mode, float_path);
+}
+
+// What the prologue of a string-matching entry point sets up
+struct LevCall {
+    LevLayout L;
+    char* ws;          // the caller's workspace, aligned
+    b200lev_opts_t o;  // the options the call runs with
+    LevParams p;
+    bool count_mode, float_path;
+};
+
+// The argument prologue of the string-matching entry points: checks the token views and the
+// options, lays out the workspace for `kind` and checks the caller's buffers.  Returns LEV_EMPTY
+// when the call has nothing to write (no pairs, no output rows, or `inner` <= 0), and NULL
+// buffers are then fine (only c->L is filled); else B200LEV_OK with *c filled, or an error status
+// (`null_status` for a NULL `out` or `ws`).  The call runs with the caller's options after
+// `adjust` (may be NULL); the final value and the alignment ignore exclude_last (SM:165).
+static constexpr int LEV_EMPTY = 1;
+static int lev_begin(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                     const b200lev_opts_t* opts, int kind, const void* out, const void* ws,
+                     size_t ws_bytes, int32_t* flags, LevCall* c,
+                     void (*adjust)(b200lev_opts_t*) = nullptr, int64_t inner = 1,
+                     int null_status = B200LEV_ERR_ARG) {
+    const int rc = lev_check_tokens(ref, hyp, opts);
+    if (rc) return rc;
+    c->o = *opts;
+    if (adjust) adjust(&c->o);
+    if (kind == B200LEV_WS_FINAL || kind == B200LEV_WS_ALIGN) c->o.exclude_last = 0;
+    c->L = lev_layout(ref, hyp, kind, c->o.exclude_last);
+    if (hyp->N == 0 || c->L.Hout <= 0 || inner <= 0) return LEV_EMPTY;
+    if (!out || !ws) {
+        lev_set_error("NULL output or workspace");
+        return null_status;
+    }
+    if (ws_bytes < c->L.bytes + 128) {
+        lev_set_error("workspace too small: %zu < %zu", ws_bytes, c->L.bytes + 128);
+        return B200LEV_ERR_WORKSPACE;
+    }
+    c->ws = lev_ws_base(ws);
+    lev_params(ref, hyp, &c->o, c->L, c->ws, flags, &c->p, &c->count_mode, &c->float_path);
+    return B200LEV_OK;
 }
 
 // K0: pack both token tensors into the workspace.  It leaves what the DP kernels need to know
@@ -337,37 +353,33 @@ static int lev_string_match(const b200lev_tokens_t* ref, const b200lev_tokens_t*
                             int64_t out_sn, void* workspace, size_t workspace_bytes,
                             int32_t* flags, double* acc, void* stream) {
     const bool final = mode == LEV_MODE_FINAL;
-    LevLayout L;
+    LevCall c;
     int rc = lev_begin(ref, hyp, opts, final ? B200LEV_WS_FINAL : B200LEV_WS_PREFIX, out, workspace,
-                       workspace_bytes, &L);
+                       workspace_bytes, flags, &c);
     if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char* ws = lev_ws_base(workspace);
-    b200lev_opts_t o = *opts;
-    if (final) o.exclude_last = 0;  // SM:165
-    LevParams p;
-    bool cm, fp;
-    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
+    LevParams& p = c.p;
     p.out = out;
     if (!final) {
         p.out_si = out_si;
         p.out_sn = out_sn;
-        p.Hout = (int)L.Hout;
+        p.Hout = (int)c.L.Hout;
     }
     std::lock_guard<std::mutex> fork_lock(g_fork_mu);
-    const LevBvRoute bv = lev_bitvec_route(ref, hyp, mode, p, cm, fp);
+    const LevBvRoute bv = lev_bitvec_route(ref, hyp, mode, p, c.count_mode, c.float_path);
     LevFork fork;
     const bool forked = bv == LEV_BV_SELECTED && lev_fork_get(&fork);
     if (bv != LEV_BV_NONE) {
-        rc = lev_bitvec_launch(bv, ref, hyp, &o, mode, L, ws, p, st, forked ? fork.after_probe : nullptr, acc);
+        rc = lev_bitvec_launch(bv, ref, hyp, &c.o, mode, c.L, c.ws, p, st, forked ? fork.after_probe : nullptr,
+                               acc);
         if (rc) return rc;
     }
     if (bv == LEV_BV_NONE || bv == LEV_BV_SELECTED) {
         cudaStream_t side = lev_fork_begin(fork, forked);
         cudaStream_t cs = side ? side : st;  // the wavefront chain's stream
         p.bv_check = bv == LEV_BV_SELECTED;
-        rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, p.bv_check, cs);
-        if (rc == B200LEV_OK) rc = lev_launch_dp(p, mode, cm, fp, cs);
+        rc = lev_pack_tokens(ref, hyp, &c.o, c.L, c.ws, flags, p.bv_check, cs);
+        if (rc == B200LEV_OK) rc = lev_launch_dp(p, mode, c.count_mode, c.float_path, cs);
         if (side) {
             const int jr = lev_fork_join(fork, st);
             if (rc == B200LEV_OK) rc = jr;
@@ -375,7 +387,7 @@ static int lev_string_match(const b200lev_tokens_t* ref, const b200lev_tokens_t*
     }
     // (Ks accumulates the sums itself)
     if (rc == B200LEV_OK && acc != nullptr && bv != LEV_BV_SHORT)
-        rc = lev_launch_err_sum(out, p.ref_len, hyp->N, o.ref_group, acc, st);
+        rc = lev_launch_err_sum(out, p.ref_len, hyp->N, c.o.ref_group, acc, st);
     return rc;
 }
 
@@ -485,19 +497,15 @@ extern "C" int b200lev_final_cross(const b200lev_tokens_t* ref, const b200lev_to
     const bool trace = getenv("B200LEV_TRACE") != nullptr;
     cudaStream_t st = (cudaStream_t)stream;
     if (c.short_form) {
-        LevLayout L;
-        rc = lev_begin(ref, &c.hx, &c.o, B200LEV_WS_FINAL, out, workspace, workspace_bytes, &L);
+        LevCall k;
+        rc = lev_begin(ref, &c.hx, &c.o, B200LEV_WS_FINAL, out, workspace, workspace_bytes, flags, &k);
         if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
         if (trace)
             fprintf(stderr, "b200lev: final cross, short cross form (lev_bv_short_kernel CROSS), A=%lld B=%lld P=%lld\n",
                     (long long)A, (long long)B, (long long)c.P);
-        char* ws = lev_ws_base(workspace);
-        LevParams p;
-        bool cm, fp;
-        lev_params(ref, &c.hx, &c.o, L, ws, flags, &p, &cm, &fp);
-        p.out = out;
-        return lev_bitvec_launch(LEV_BV_SHORT, ref, &c.hx, &c.o, LEV_MODE_FINAL, L, ws, p, st, nullptr, nullptr,
-                                 A, B);
+        k.p.out = out;
+        return lev_bitvec_launch(LEV_BV_SHORT, ref, &c.hx, &k.o, LEV_MODE_FINAL, k.L, k.ws, k.p, st, nullptr,
+                                 nullptr, A, B);
     }
     if (!out || !workspace) {
         lev_set_error("NULL output or workspace");
@@ -531,92 +539,84 @@ extern "C" int b200lev_prefix(const b200lev_tokens_t* ref, const b200lev_tokens_
                             workspace, workspace_bytes, flags, nullptr, stream);
 }
 
+// b200lev_error_counts (`counts`) and b200lev_error_alignment (`align`: `ops` with its strides).
 // Per pair (C, S, D, I) along the path of error_rate's count mode (SM:292-314; unit costs after
-// SM:168-174 take the same cell).  R <= 64 with one token width: the short form, one launch
-// straight from the raw tokens (lev_counts.cuh).  Otherwise K0 + K1 with the insertion channel.
-extern "C" int b200lev_error_counts(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                                    const b200lev_opts_t* opts, int64_t* out, void* workspace,
-                                    size_t workspace_bytes, int32_t* flags, void* stream) {
+// SM:168-174 take the same cell), or the ops along that path (lev_align.cuh): the alignment keeps
+// every cell's choice in the workspace and walks it back.  R <= 64 with one token width: the short
+// form, one launch straight from the raw tokens (lev_counts.cuh), where the lane walks its own
+// trace.  Otherwise K0 + K1 with the insertion channel, and for the alignment the trace, then one
+// thread per pair walks.
+static int lev_error_path(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                          const b200lev_opts_t* opts, bool align, int64_t* counts, int8_t* ops,
+                          int64_t ops_sk, int64_t ops_sn, void* workspace, size_t workspace_bytes,
+                          int32_t* flags, void* stream) {
+    const char* what = align ? "error alignment" : "error counts";
     if (opts && opts->ref_group != 1) {
-        lev_set_error("error counts: ref_group must be 1, got %d", opts->ref_group);
+        lev_set_error("%s: ref_group must be 1, got %d", what, opts->ref_group);
         return B200LEV_ERR_ARG;
     }
-    LevLayout L;
-    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_FINAL, out, workspace, workspace_bytes, &L);
+    LevCall c;
+    const int64_t steps = (ref && hyp) ? ref->T + hyp->T : 0;
+    int rc = lev_begin(ref, hyp, opts, align ? B200LEV_WS_ALIGN : B200LEV_WS_FINAL,
+                       align ? (void*)ops : (void*)counts, workspace, workspace_bytes, flags, &c,
+                       [](b200lev_opts_t* o) {
+                           o->norm = 0;
+                           o->return_mistakes = 1;
+                       },
+                       align ? steps : 1);
     if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char* ws = lev_ws_base(workspace);
-    b200lev_opts_t o = *opts;
-    o.norm = 0;
-    o.exclude_last = 0;
-    o.return_mistakes = 1;
-    LevParams p;
-    bool cm, fp;
-    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
-    const bool trace = getenv("B200LEV_TRACE") != nullptr;
-    if (lev_counts_short_form(ref, hyp)) {
-        if (trace)
-            fprintf(stderr, "b200lev: error counts, lev_counts_short_kernel, R=%lld H=%lld P=%lld %s\n",
-                    (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
-        return lev_counts_short_launch(ref, hyp, &o, p, fp, out, st);
+    LevParams& p = c.p;
+    if (align) {
+        p.trace = (unsigned char*)(c.ws + c.L.off_trace);
+        p.trace_pair_bytes = c.L.trace_pair_bytes;
+        p.trace_steps = c.L.H + 31;
+        p.align_ins = (int*)(c.ws + c.L.off_align_ins);
+        p.ops = ops;
+        p.ops_sk = ops_sk;
+        p.ops_sn = ops_sn;
+        p.ops_steps = (int)steps;
+    } else {
+        p.counts = counts;
     }
-    if (trace)
-        fprintf(stderr, "b200lev: error counts, pack + lev_warp_kernel, R=%lld H=%lld P=%lld %s\n",
-                (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
-    p.out = reinterpret_cast<float*>(out);  // (lev_common.cuh: the counts go where FINAL's values go)
-    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
-    if (rc == B200LEV_OK) rc = lev_launch_counts_dp(p, fp, st);
+    const bool short_form = lev_counts_short_form(ref, hyp);
+    if (getenv("B200LEV_TRACE"))
+        fprintf(stderr, "b200lev: %s, %s, R=%lld H=%lld P=%lld %s\n", what,
+                short_form ? (align ? "lev_counts_short_kernel (trace)" : "lev_counts_short_kernel")
+                           : (align ? "pack + lev_warp_kernel (trace) + lev_align_walk_kernel"
+                                    : "pack + lev_warp_kernel"),
+                (long long)c.L.R, (long long)c.L.H, (long long)c.L.P, c.float_path ? "fp32" : "int32");
+    if (short_form) return lev_counts_short_launch(ref, hyp, &c.o, p, c.float_path, st);
+    rc = lev_pack_tokens(ref, hyp, &c.o, c.L, c.ws, flags, 0, st);
+    if (rc == B200LEV_OK) rc = lev_launch_counts_dp(p, c.float_path, st);
     return rc;
 }
 
-// Per pair the ops along the path b200lev_error_counts counts (lev_align.cuh): the same two forms,
-// each keeping every cell's choice in the workspace and walking it back.  Short form: one launch,
-// the lane walks its own trace.  Long form: K0, K1 with the trace, then one thread per pair walks.
+extern "C" int b200lev_error_counts(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                                    const b200lev_opts_t* opts, int64_t* out, void* workspace,
+                                    size_t workspace_bytes, int32_t* flags, void* stream) {
+    return lev_error_path(ref, hyp, opts, false, out, nullptr, 0, 0, workspace, workspace_bytes, flags,
+                          stream);
+}
+
 extern "C" int b200lev_error_alignment(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                                        const b200lev_opts_t* opts, int8_t* out, int64_t out_stride_k,
                                        int64_t out_stride_n, void* workspace, size_t workspace_bytes,
                                        int32_t* flags, void* stream) {
-    if (opts && opts->ref_group != 1) {
-        lev_set_error("error alignment: ref_group must be 1, got %d", opts->ref_group);
-        return B200LEV_ERR_ARG;
-    }
-    LevLayout L;
-    const int64_t steps = (ref && hyp) ? ref->T + hyp->T : 0;
-    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_ALIGN, out, workspace, workspace_bytes, &L, steps);
-    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    char* ws = lev_ws_base(workspace);
-    b200lev_opts_t o = *opts;
-    o.norm = 0;
-    o.exclude_last = 0;
-    o.return_mistakes = 1;
-    LevParams p;
-    bool cm, fp;
-    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
-    const bool trace = getenv("B200LEV_TRACE") != nullptr;
-    if (lev_counts_short_form(ref, hyp)) {
-        if (trace)
-            fprintf(stderr, "b200lev: error alignment, lev_counts_short_kernel (trace), R=%lld H=%lld P=%lld %s\n",
-                    (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
-        return lev_align_short_launch(ref, hyp, &o, p, fp, (uint32_t*)(ws + L.off_trace), out, out_stride_k,
-                                      out_stride_n, st);
-    }
-    if (trace)
-        fprintf(stderr, "b200lev: error alignment, pack + lev_warp_kernel (trace) + lev_align_walk_kernel, "
-                "R=%lld H=%lld P=%lld %s\n", (long long)L.R, (long long)L.H, (long long)L.P, fp ? "fp32" : "int32");
-    lev_align_set(&p, ws + L.off_trace, L.trace_pair_bytes, L.H + 31, (int*)(ws + L.off_align_ins), out,
-                  out_stride_k, out_stride_n, (int)steps);
-    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
-    if (rc == B200LEV_OK) rc = lev_launch_align_dp(p, fp, st);
-    return rc;
+    return lev_error_path(ref, hyp, opts, true, nullptr, out, out_stride_k, out_stride_n, workspace,
+                          workspace_bytes, flags, stream);
 }
 
 extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                                         const b200lev_opts_t* opts, void* workspace,
                                         size_t workspace_bytes, int32_t* umax, int32_t* flags,
                                         void* stream) {
-    LevLayout L;
-    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_COMPLETION, umax, workspace, workspace_bytes, &L);
+    LevCall c;
+    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_COMPLETION, umax, workspace, workspace_bytes, flags, &c,
+                       [](b200lev_opts_t* o) {
+                           o->return_mistakes = 0;  // SM:479-491: the mask is always taken on the cost row
+                           o->norm = 0;
+                       });
     if (rc < 0) return rc;
     if (!umax) {  // (an empty batch still writes U = 0)
         lev_set_error("NULL umax");
@@ -625,19 +625,14 @@ extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200l
     cudaStream_t st = (cudaStream_t)stream;
     if (cudaMemsetAsync(umax, 0, sizeof(int32_t), st) != cudaSuccess) return lev_check_cuda("memset");
     if (rc == LEV_EMPTY) return B200LEV_OK;
-    char* ws = lev_ws_base(workspace);
-    b200lev_opts_t o = *opts;
-    o.return_mistakes = 0;  // SM:479-491: the mask is always taken on the cost row
-    o.norm = 0;
-    LevParams p;
-    bool cm, fp;
-    lev_params(ref, hyp, &o, L, ws, flags, &p, &cm, &fp);
-    rc = lev_pack_tokens(ref, hyp, &o, L, ws, flags, 0, st);
+    const LevLayout& L = c.L;
+    LevParams& p = c.p;
+    rc = lev_pack_tokens(ref, hyp, &c.o, L, c.ws, flags, 0, st);
     if (rc) return rc;
-    int32_t* uid = (int32_t*)(ws + L.off_uid);
-    int64_t* dtok = (int64_t*)(ws + L.off_dtok);
-    int32_t* ndist = (int32_t*)(ws + L.off_ndist);
-    uint32_t* dbits = (uint32_t*)(ws + L.off_dbits);
+    int32_t* uid = (int32_t*)(c.ws + L.off_uid);
+    int64_t* dtok = (int64_t*)(c.ws + L.off_dtok);
+    int32_t* ndist = (int32_t*)(c.ws + L.off_ndist);
+    uint32_t* dbits = (uint32_t*)(c.ws + L.off_dbits);
     rc = lev_launch_uid(ref, p.ref_tok, p.wide_flag, p.ref_len, uid, dtok, ndist, L.Rp, st);
     if (rc) return rc;
     if (cudaMemsetAsync(dbits, 0, sizeof(uint32_t) * (size_t)L.Hout * L.P * L.Wd, st) != cudaSuccess)
@@ -648,7 +643,7 @@ extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200l
     p.Wd = (int)L.Wd;
     p.umax = umax;
     p.Hout = (int)L.Hout;
-    return lev_launch_dp(p, LEV_MODE_MASK, false, fp, st);
+    return lev_launch_dp(p, LEV_MODE_MASK, false, c.float_path, st);
 }
 
 extern "C" int b200lev_completion_fill(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
@@ -656,13 +651,13 @@ extern "C" int b200lev_completion_fill(const b200lev_tokens_t* ref, const b200le
                                        size_t workspace_bytes, int64_t U, int64_t* out,
                                        int64_t out_stride_i, int64_t out_stride_n, void* stream) {
     // (a NULL output counts as a bad workspace here)
-    LevLayout L;
+    LevCall c;
     const int rc = lev_begin(ref, hyp, opts, B200LEV_WS_COMPLETION, out, workspace, workspace_bytes,
-                             &L, U, B200LEV_ERR_WORKSPACE);
+                             nullptr, &c, nullptr, U, B200LEV_ERR_WORKSPACE);
     if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
-    const char* ws = lev_ws_base(workspace);
-    return lev_launch_completion_fill((const uint32_t*)(ws + L.off_dbits),
-                                      (const int64_t*)(ws + L.off_dtok), (const int*)(ws + L.off_flags), L.Rp,
+    const LevLayout& L = c.L;
+    return lev_launch_completion_fill((const uint32_t*)(c.ws + L.off_dbits),
+                                      (const int64_t*)(c.ws + L.off_dtok), (const int*)(c.ws + L.off_flags), L.Rp,
                                       L.Hout, L.P, L.Wd,
                                       opts->ref_group, U, opts->padding, out, out_stride_i,
                                       out_stride_n, (cudaStream_t)stream);

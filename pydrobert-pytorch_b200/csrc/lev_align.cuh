@@ -79,11 +79,10 @@ __global__ void __launch_bounds__(256) lev_align_walk_kernel(const LevParams p) 
          pair += (int64_t)gridDim.x * blockDim.x) {
         const int r = p.ref_len[pair], h = p.hyp_len[pair];
         LevTraceStrips<C> a;
-        a.base = reinterpret_cast<const Field*>(lev_align_trace(p) + pair * lev_align_pair_bytes_of(p));
+        a.base = reinterpret_cast<const Field*>(p.trace + pair * p.trace_pair_bytes);
         a.r = r;
         a.S = (r + 32 * C) / (32 * C);
-        a.ns = lev_align_ns(p);
-        lev_align_walk(a, h, r, r + lev_align_ins(p)[pair], lev_align_tout(p),
-                       lev_align_ops(p) + pair * lev_align_ops_sn(p), lev_align_ops_sk(p));
+        a.ns = p.trace_steps;
+        lev_align_walk(a, h, r, r + p.align_ins[pair], p.ops_steps, p.ops + pair * p.ops_sn, p.ops_sk);
     }
 }

@@ -114,10 +114,8 @@ int lev_bitvec_launch(LevBvRoute route, const b200lev_tokens_t* ref, const b200l
     a.out_si = p.out_si;
     if (route == LEV_BV_SHORT) {  // R <= 64: lane = pair, reference in registers, no tables (lev_bvshort.cu)
         a.acc = mode == LEV_MODE_FINAL ? acc : nullptr;
-        // set on every Ks call, so that whatever the Kb fields held before, a plain call has
-        // cross_b = 0 and never takes the cross instantiation
-        lev_bv_cross_ab(a) = (int)(cross_a * cross_b);  // (< 2^31: b200lev_final_cross bounds the pairs)
-        lev_bv_cross_b(a) = (int)cross_b;
+        a.cross_ab = (int)(cross_a * cross_b);  // (< 2^31: b200lev_final_cross bounds the pairs)
+        a.cross_b = (int)cross_b;
         if (getenv("B200LEV_TRACE"))
             fprintf(stderr, "b200lev: short bit-vector kernel, mode %d, R=%d H=%d P=%d\n", mode, a.R, a.H, a.P);
         return lev_bvshort_launch(a, ref->elem_bytes, st);

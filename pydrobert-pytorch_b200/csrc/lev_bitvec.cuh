@@ -26,14 +26,10 @@ struct LevBvArgs {
     float* out;
     int64_t out_si;  // prefix: elements between output rows (pairs are adjacent)
     double* acc;     // FINAL, short-reference kernel: += [sum(out), sum(ref_len per pair), #pairs] (may be NULL)
+    // b200lev_final_cross through Ks (final mode): pair p reads hypothesis column
+    // (p / cross_ab) * cross_b + p % cross_b, cross_ab = A * B and cross_b = B (0: the plain form)
+    int cross_ab, cross_b;
 };
-// b200lev_final_cross through Ks (final mode): pair p reads hypothesis column
-// (p / cross_ab) * cross_b + p % cross_b, cross_ab = A * B and cross_b = B (0: the plain form).  The
-// two ride in fields only Kb reads, so the struct, and every kernel that takes it, stays as it is
-// (two trailing fields would move the scalar arguments lev_bv_probe_kernel takes after the struct,
-// and so change its SASS).  lev_bitvec_launch sets both on every Ks call.
-#define lev_bv_cross_ab(a) ((a).slots_log2)
-#define lev_bv_cross_b(a) ((a).check_state)
 
 // Bucketed hash: 4 ways per bucket.  x = v * mult (odd mult: a bijection on 32 bits) picks the
 // bucket with its top s bits, and its low 32 - s bits -- the residual -- tell apart every int32

@@ -120,7 +120,7 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
         const int64_t pc = pair < a.P ? pair : (int64_t)a.P - 1;
         const int64_t rcol = pc / a.ref_group;
         const int64_t hcol =
-            CROSS ? (int64_t)((int)pc / lev_bv_cross_ab(a) * lev_bv_cross_b(a) + (int)pc % lev_bv_cross_b(a)) : pc;
+            CROSS ? (int64_t)((int)pc / a.cross_ab * a.cross_b + (int)pc % a.cross_b) : pc;
         const TT* __restrict__ rsrc = reinterpret_cast<const TT*>(a.ref) + rcol;
         const TT* __restrict__ hsrc = reinterpret_cast<const TT*>(a.hyp) + hcol;
 
@@ -453,7 +453,7 @@ static void lev_bvs_launch_w(const LevBvArgs& a, cudaStream_t st) {
     int64_t cap = (int64_t)148 * (W == 1 ? 20 : 16);  // whole waves of the resident CTAs (5 / 4 per SM)
     if (const char* e = getenv("B200LEV_BVS_CTAS")) cap = atoll(e) > 0 ? atoll(e) : cap;  // (tests: many blocks per warp)
     const dim3 grid((unsigned)(n < cap ? n : cap)), block(32 * LEV_BVS_WARPS);
-    if (lev_bv_cross_b(a) > 0)  // (final mode only)
+    if (a.cross_b > 0)  // (final mode only)
         lev_launch(lev_bv_short_kernel<TT, W, 0, true>, grid, block, 0, st, a);
     else if (a.mode != LEV_MODE_PREFIX)
         lev_launch(lev_bv_short_kernel<TT, W, 0, false>, grid, block, 0, st, a);

@@ -159,21 +159,16 @@ struct LevParams {
     float mult;  // SM:168-174
     int norm, exclude_last;
     float padding;
-    // FINAL: out[n];  PREFIX: out[i*out_si + n*out_sn];  error counts (lev_launch_counts_dp): int64
-    // (C, S, D, I) of pair n at ((int64_t*)out)[4n .. 4n+3]
-    // ALIGN (the long form of b200lev_error_alignment, lev_align_set below): out holds the int8 ops,
-    // out_si / out_sn their step / pair strides and Hout the steps per pair.  The FINAL-mode
-    // instantiations of K1 with TRACE read these five fields and dbits, umax, Hr and Hr16 with the
-    // alignment's meaning: a new FINAL-mode use of any of them must not reach that path.
+    // FINAL: out[n];  PREFIX: out[i*out_si + n*out_sn]
     float* out;
     int64_t out_si, out_sn;
     int Hout;
     // MASK
     const int32_t* uid;  // [Nref][Rp] rank of ref[j] among the pair's distinct tokens
     const int32_t* ndist;  // [Nref] number of distinct tokens of the reference
-    uint32_t* dbits;     // [Hout][P][Wd]  (ALIGN: the choice trace)
+    uint32_t* dbits;     // [Hout][P][Wd]
     int Wd;
-    int* umax;           // (ALIGN: the insertions of each pair)
+    int* umax;
     int* flags;            // caller's warning flags (may be NULL)
     const int* wide_flag;  // never NULL: workspace state words K0 fills: [0] flags (incl.
                            // B200LEV_FLAG_WIDE_TOKENS), [1], [2] biased token range
@@ -193,32 +188,21 @@ struct LevParams {
     int* gmeta_order;  // same storage viewed as int[P]: pair order of the CTA kernel
     int32_t* raw32;          // [P][Hr]   raw prefix rows (32-bit group path)
     unsigned short* raw16;   // [P][Hr16] same storage, packed path
-    int64_t Hr, Hr16;  // (ALIGN: trace bytes per pair, step slots per strip)
+    int64_t Hr, Hr16;
     int nbins;
+    // b200lev_error_alignment: the cells' choices (short form [row][word][pair] words; long form
+    // trace_pair_bytes per pair, trace_steps step slots per strip), the insertions of each pair
+    // (long form), and the int8 ops the walk writes, step k of pair n at ops[k*ops_sk + n*ops_sn],
+    // k < ops_steps
+    unsigned char* trace;
+    int64_t trace_pair_bytes, trace_steps;
+    int* align_ins;
+    int8_t* ops;
+    int64_t ops_sk, ops_sn;
+    int ops_steps;
+    // b200lev_error_counts: (C, S, D, I) of pair n at counts[4n .. 4n+3]
+    int64_t* counts;
 };
-// Error alignment, long form (lev_launch_align_dp), in the fields final mode leaves unused (so
-// the struct, and every kernel that takes it, stays as it is): lev_warp_kernel's per-cell choices
-// (lev_align_trace, lev_align_pair_bytes per pair, lev_align_ns steps per strip), the insertions
-// of each pair, and the ops the walk writes (int8, step k of pair n at ops[k*sk + n*sn], k < Tout)
-#define lev_align_trace(p) reinterpret_cast<unsigned char*>((p).dbits)
-#define lev_align_ins(p) ((p).umax)
-#define lev_align_pair_bytes_of(p) ((p).Hr)
-#define lev_align_ns(p) ((p).Hr16)
-#define lev_align_ops(p) reinterpret_cast<int8_t*>((p).out)
-#define lev_align_ops_sk(p) ((p).out_si)
-#define lev_align_ops_sn(p) ((p).out_sn)
-#define lev_align_tout(p) ((p).Hout)
-static inline void lev_align_set(LevParams* p, void* trace, int64_t pair_bytes, int64_t ns, int* ins,
-                                 int8_t* ops, int64_t sk, int64_t sn, int tout) {
-    p->dbits = reinterpret_cast<uint32_t*>(trace);
-    p->Hr = pair_bytes;
-    p->Hr16 = ns;
-    p->umax = ins;
-    p->out = reinterpret_cast<float*>(ops);
-    p->out_si = sk;
-    p->out_sn = sn;
-    p->Hout = tout;
-}
 
 
 #if defined(__CUDACC__) || defined(B200LEV_EMU)
@@ -270,20 +254,14 @@ int lev_launch_dp(const LevParams& p, int mode, bool count_mode, bool float_path
 int lev_launch_group(const LevParams& p, int mode, bool count_mode, cudaStream_t st);
 int lev_launch_mask16(const LevParams& p, bool float_path, cudaStream_t st);
 int lev_launch_cta(const LevParams& p, int mode, bool count_mode, bool float_path, cudaStream_t st);
-// b200lev_error_counts: K1 with the insertion channel, after K0 (lev_dp.cu), and the short form
-// for R <= 64 straight from the raw tokens (lev_counts.cuh; `p` supplies the costs)
+// b200lev_error_counts (p.counts) and b200lev_error_alignment (p.ops and p.trace set): K1 with the
+// insertion channel after K0, and for the alignment its choice trace and the walk (lev_dp.cu /
+// lev_align.cuh); and the short form for R <= 64, one launch straight from the raw tokens
+// (lev_counts.cuh; `p` supplies the costs, the flags and the output)
 int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st);
 int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                             const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                            int64_t* out, cudaStream_t st);
-// b200lev_error_alignment: K1 with the choice trace, then the walk (lev_dp.cu / lev_align.cuh),
-// after K0; and the short form with its trace (lev_counts.cuh).  `trace` is the workspace
-// region the layout of kind 3 gives.
-int lev_launch_align_dp(const LevParams& p, bool float_path, cudaStream_t st);
-int lev_align_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                           const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                           uint32_t* trace, int8_t* ops, int64_t ops_sk, int64_t ops_sn,
-                           cudaStream_t st);
+                            cudaStream_t st);
 // lanes per pair if the shapes admit the group kernel (its histogram is then built at
 // pack time), else 0
 int lev_group_eligible(int64_t R, int64_t H, int64_t P);

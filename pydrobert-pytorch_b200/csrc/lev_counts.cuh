@@ -306,10 +306,10 @@ static void lev_counts_launch_tt(const LevAlignArgs& a, bool float_path, bool tr
     }
 }
 
-// the two entry points' launch: `a` carries either the counts' output or the trace and the ops
-static int lev_counts_short_run(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                                const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                                LevAlignArgs& a, cudaStream_t st) {
+// both entry points: the counts to p.counts, or (p.ops set) the choice rows to p.trace and the ops
+int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                            const b200lev_opts_t* o, const LevParams& p, bool float_path,
+                            cudaStream_t st) {
     if (ref->T > 64) {
         lev_set_error("short error-counts form: R = %lld > 64", (long long)ref->T);
         return B200LEV_ERR_ARG;
@@ -319,6 +319,8 @@ static int lev_counts_short_run(const b200lev_tokens_t* ref, const b200lev_token
                       hyp->elem_bytes);
         return B200LEV_ERR_ARG;
     }
+    LevAlignArgs a;
+    memset(&a, 0, sizeof(a));
     a.ref = ref->data;
     a.hyp = hyp->data;
     a.ref_st = ref->stride_t;
@@ -338,39 +340,23 @@ static int lev_counts_short_run(const b200lev_tokens_t* ref, const b200lev_token
     a.del_f = p.del_f;
     a.sub_f = p.sub_f;
     a.flags = p.flags;
+    a.out = p.counts;
+    a.trace = reinterpret_cast<uint32_t*>(p.trace);
+    a.ops = p.ops;
+    a.ops_sk = p.ops_sk;
+    a.ops_sn = p.ops_sn;
+    a.Tout = p.ops_steps;
+    const bool trace = p.ops != nullptr;
     lev_prof_begin(LEV_PROF_DP, st);
     switch (ref->elem_bytes) {
-        case 8: lev_counts_launch_tt<int64_t>(a, float_path, a.trace != nullptr, st); break;
-        case 4: lev_counts_launch_tt<int32_t>(a, float_path, a.trace != nullptr, st); break;
-        case 2: lev_counts_launch_tt<int16_t>(a, float_path, a.trace != nullptr, st); break;
-        case 1: lev_counts_launch_tt<int8_t>(a, float_path, a.trace != nullptr, st); break;
+        case 8: lev_counts_launch_tt<int64_t>(a, float_path, trace, st); break;
+        case 4: lev_counts_launch_tt<int32_t>(a, float_path, trace, st); break;
+        case 2: lev_counts_launch_tt<int16_t>(a, float_path, trace, st); break;
+        case 1: lev_counts_launch_tt<int8_t>(a, float_path, trace, st); break;
         default:
             lev_set_error("token width %d bytes", ref->elem_bytes);
             return B200LEV_ERR_ARG;
     }
     lev_prof_end(LEV_PROF_DP, st);
     return lev_check_cuda("lev_counts_short_kernel");
-}
-
-int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                            const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                            int64_t* out, cudaStream_t st) {
-    LevAlignArgs a;
-    memset(&a, 0, sizeof(a));
-    a.out = out;
-    return lev_counts_short_run(ref, hyp, o, p, float_path, a, st);
-}
-
-int lev_align_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
-                           const b200lev_opts_t* o, const LevParams& p, bool float_path,
-                           uint32_t* trace, int8_t* ops, int64_t ops_sk, int64_t ops_sn,
-                           cudaStream_t st) {
-    LevAlignArgs a;
-    memset(&a, 0, sizeof(a));
-    a.trace = trace;
-    a.ops = ops;
-    a.ops_sk = ops_sk;
-    a.ops_sn = ops_sn;
-    a.Tout = (int)(ref->T + hyp->T);
-    return lev_counts_short_run(ref, hyp, o, p, float_path, a, st);
 }

@@ -215,8 +215,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         }
                         if constexpr (TRACE) {
                             typedef typename LevTraceStrips<C>::Field Field;
-                            reinterpret_cast<Field*>(lev_align_trace(p) + (int64_t)pair * lev_align_pair_bytes_of(p))
-                                [((int64_t)k * lev_align_ns(p) + (s - 1)) * 32 + lane] = (Field)tr;
+                            reinterpret_cast<Field*>(p.trace + (int64_t)pair * p.trace_pair_bytes)
+                                [((int64_t)k * p.trace_steps + (s - 1)) * 32 + lane] = (Field)tr;
                         }
                     } else if (FLT_COST) {
                         // SM:290-293,316-317 in fp32, deletion term by run origin:
@@ -307,11 +307,11 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
         }
         if (OPS && last && lane == 31) {
             if constexpr (TRACE) {
-                lev_align_ins(p)[pair] = ic[C - 1];
+                p.align_ins[pair] = ic[C - 1];
             } else {
                 // m = S + D + I; C + S + D = r and C + S + I = h
                 const int ins = ic[C - 1], del = ins + r - h, sub = (int)m[C - 1] - ins - del;
-                int64_t* __restrict__ o = reinterpret_cast<int64_t*>(p.out) + (int64_t)pair * 4;
+                int64_t* __restrict__ o = p.counts + (int64_t)pair * 4;
                 o[0] = h - sub - ins;
                 o[1] = sub;
                 o[2] = del;
@@ -517,15 +517,6 @@ int lev_launch_dp(const LevParams& p_, int mode, bool count_mode, bool float_pat
     return B200LEV_ERR_ARG;
 }
 
-// b200lev_error_counts, references longer than the short form takes (lev_counts.cuh): K1 with the
-// count cell and the insertion channel, after K0.  No group, CTA or bit-vector kernel: they carry
-// no path.
-int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st) {
-    if (p.P <= 0) return B200LEV_OK;
-    if (!float_path) return lev_launch_variant<int, true, LEV_MODE_FINAL, 10, true>(p, st);
-    return lev_launch_variant<float, true, LEV_MODE_FINAL, 4, true>(p, st);
-}
-
 // b200lev_error_alignment, the long form: K1 with the count cell, the insertion channel and the
 // choice trace at one strip width, then the walk, one thread per pair
 template <typename V, int C>
@@ -538,10 +529,17 @@ static int lev_launch_align_t(const LevParams& p, cudaStream_t st) {
     return lev_check_cuda("lev_align_walk_kernel");
 }
 
-int lev_launch_align_dp(const LevParams& p, bool float_path, cudaStream_t st) {
+// b200lev_error_counts / b200lev_error_alignment, references longer than the short form takes
+// (lev_counts.cuh): K1 with the count cell and the insertion channel, after K0.  No group, CTA or
+// bit-vector kernel: they carry no path.
+int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st) {
     if (p.P <= 0) return B200LEV_OK;
-    if (!float_path) return lev_launch_align_t<int, LEV_ALIGN_C_INT>(p, st);
-    return lev_launch_align_t<float, LEV_ALIGN_C_FLT>(p, st);
+    if (p.ops != nullptr) {
+        if (!float_path) return lev_launch_align_t<int, LEV_ALIGN_C_INT>(p, st);
+        return lev_launch_align_t<float, LEV_ALIGN_C_FLT>(p, st);
+    }
+    if (!float_path) return lev_launch_variant<int, true, LEV_MODE_FINAL, 10, true>(p, st);
+    return lev_launch_variant<float, true, LEV_MODE_FINAL, 4, true>(p, st);
 }
 
 // the short form (R <= 64): one lane per pair from the raw tokens
