@@ -168,6 +168,28 @@ int b200lev_error_alignment(const b200lev_tokens_t *ref, const b200lev_tokens_t 
                             int32_t *flags, void *stream);
 
 /*
+ * Infix edit distance: per pair the cheapest alignment of the whole reference against any
+ * contiguous stretch hyp[s:e] of the hypothesis, leading and trailing hypothesis tokens free.
+ * D is the DP of b200lev_final (same lengths, costs, uniform-cost shortcut and fp32 operation
+ * order) with one change: column 0 is 0 on every row (row 0 keeps D[0][j] = j deletions).
+ *   dist : device float[hyp->N], the minimum over 0 <= i <= h of D[i][r]; opts->norm divides it
+ *          by r as b200lev_final does (an empty reference has distance 0, and raises
+ *          B200LEV_FLAG_EMPTY_REF under norm).
+ *   start, end : device int64[hyp->N], both NULL (distances only) or both set.  end is the
+ *          smallest row reaching the minimum, start the start row of the optimal path into
+ *          (end, r): leaving column 0 at row s starts at s, and at each cell the largest start
+ *          among the predecessors (diagonal, up, deletion run origin) reaching its value wins.
+ *          The match is hyp[start:end].  Not with opts->norm.
+ * opts: has_eos, eos, include_eos, the costs and norm as for b200lev_final; ref_group must be 1;
+ * exclude_last, padding and return_mistakes are ignored.  Free ends on the reference side
+ * instead: swap ref and hyp, and ins_cost and del_cost.
+ * Workspace: b200lev_workspace_bytes(ref, hyp, B200LEV_WS_FINAL, 0).
+ */
+int b200lev_infix(const b200lev_tokens_t *ref, const b200lev_tokens_t *hyp,
+                  const b200lev_opts_t *opts, float *dist, int64_t *start, int64_t *end,
+                  void *workspace, size_t workspace_bytes, int32_t *flags, void *stream);
+
+/*
  * optimal_completion (SM:464-517), two phases around the one host read the
  * reference also needs (SM:511: U = counts.max().item()).
  *   phase 1 runs the DP in mask mode (SM:271-278, 319-339, 347-355), leaves the

@@ -68,6 +68,7 @@ SIGNATURES = {
     "b200lev_mbr": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "b200lev_error_counts": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_error_alignment": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_i64, c_i64, c_vp, c_sz, c_vp, c_vp]),
+    "b200lev_infix": (ctypes.c_int, [_PT, _PT, _PO, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp, c_vp]),
     "b200lev_after_eos_mask": (ctypes.c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp]),
     "b200lev_ragged_to_padded": (ctypes.c_int, [c_vp, c_i32, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64,
                                                 c_vp, c_vp]),

@@ -264,6 +264,46 @@ def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost):
 
 
 # ---------------------------------------------------------------------------------------
+# infix: the cheapest match of each reference anywhere inside its hypothesis
+# ---------------------------------------------------------------------------------------
+def infix_impl(ref: Tensor, hyp: Tensor, eos: Optional[int], include_eos: bool, batch_first: bool,
+               ins_cost: float, del_cost: float, sub_cost: float, norm: bool, spans: bool
+               ) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """One ``b200lev_infix`` call, ``(dist, start, end, flags)``: fp32 ``(N,)``, the int64 ``(N,)``
+    match bounds (``(0,)`` unless ``spans``) and the int32[1] warning flags, on the device of
+    ``ref``."""
+    _, _, n = _shapes(ref, hyp, batch_first, 1)
+    ref, hyp = _as_tokens(ref), _as_tokens(hyp)
+    pl = _host.Placement(ref, hyp)
+    ref, hyp, dev = pl.to_dev(ref), pl.to_dev(hyp), pl.dev
+    L = _abi.lib()
+    with _DeviceGuard(dev):
+        rt, ht = _tok_struct(ref, batch_first), _tok_struct(hyp, batch_first)
+        o = _opts(eos, include_eos, ins_cost, del_cost, sub_cost, norm, False, 0, False, 1)
+        flags = torch.zeros(1, dtype=torch.int32, device=dev)
+        nbytes = L.b200lev_workspace_bytes(ctypes.byref(rt), ctypes.byref(ht), 0, 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        dist = torch.empty(n, dtype=torch.float32, device=dev)
+        start = torch.empty(n if spans else 0, dtype=torch.long, device=dev)
+        end = torch.empty(n if spans else 0, dtype=torch.long, device=dev)
+        _abi.check(L.b200lev_infix(ctypes.byref(rt), ctypes.byref(ht), ctypes.byref(o), dist.data_ptr(),
+                                   start.data_ptr() if spans else None, end.data_ptr() if spans else None,
+                                   ws.data_ptr(), nbytes, flags.data_ptr(), _stream(dev)))
+    return pl.back(dist), pl.back(start), pl.back(end), pl.back(flags)
+
+
+infix = torch.library.custom_op("b200lev::infix", infix_impl, mutates_args=())
+
+
+@infix.register_fake
+def _(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, norm, spans):
+    n = hyp.shape[0] if batch_first else hyp.shape[1]
+    m = n if spans else 0
+    return (ref.new_empty((n,), dtype=torch.float32), ref.new_empty((m,), dtype=torch.long),
+            ref.new_empty((m,), dtype=torch.long), ref.new_empty((1,), dtype=torch.int32))
+
+
+# ---------------------------------------------------------------------------------------
 # pairwise: every reference of a group against every hypothesis of it; minimum Bayes risk
 # ---------------------------------------------------------------------------------------
 def _pairwise_shapes(ref: Tensor, hyp: Tensor, batch_first: bool) -> Tuple[int, int, int]:

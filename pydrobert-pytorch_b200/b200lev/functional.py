@@ -34,6 +34,8 @@ __all__ = [
     "error_rate",
     "fill_after_eos",
     "hard_optimal_completion_distillation_loss",
+    "infix_edit_distance",
+    "infix_matches",
     "minimum_bayes_risk",
     "minimum_error_rate_loss",
     "optimal_completion",
@@ -298,6 +300,88 @@ def error_alignment(
     ``warn=False``).  :func:`alignment_positions` maps the steps to token positions."""
     return _error_path(ref, hyp, eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn,
                        True)
+
+
+def _infix(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int],
+    include_eos: bool,
+    norm: bool,
+    batch_first: bool,
+    ins_cost: float,
+    del_cost: float,
+    sub_cost: float,
+    warn: bool,
+    spans: bool,
+) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """:func:`infix_matches` if ``spans`` else :func:`infix_edit_distance` (empty bounds)."""
+    if ref.dim() != 2 or hyp.dim() != 2:
+        raise RuntimeError("ref and hyp must be 2 dimensional")
+    if not torch.jit.is_scripting():
+        if not _ops.needs_dispatcher():
+            dist, start, end, flags = _ops.infix_impl(ref, hyp, eos, include_eos, batch_first, float(ins_cost),
+                                                      float(del_cost), float(sub_cost), norm, spans)
+            if warn:
+                _warn_flags(flags, eos, include_eos, norm, False)
+            return dist, start, end
+    dist, start, end, flags = torch.ops.b200lev.infix(ref, hyp, eos, include_eos, batch_first, ins_cost,
+                                                      del_cost, sub_cost, norm, spans)
+    if warn:
+        _warn_flags(flags, eos, include_eos, norm, False)
+    return dist, start, end
+
+
+@script
+def infix_edit_distance(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    norm: bool = False,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> torch.Tensor:
+    """The cheapest alignment of each whole reference against any contiguous stretch
+    ``hyp[s:e]`` of its hypothesis: fp32 ``(N,)``.  Leading and trailing hypothesis tokens cost
+    nothing (edlib's "HW" mode).
+
+    The value is the minimum over ``0 <= s <= e <= h`` of :func:`edit_distance` of the reference
+    against ``hyp[s:e]``, bit for bit.  Arguments, lengths, costs and warnings are those of
+    :func:`edit_distance`; ``norm`` divides by the reference length as it does there, and an
+    empty reference has distance 0.  For free ends on the reference side instead, swap ``ref``
+    and ``hyp`` and swap ``ins_cost`` with ``del_cost``.  The output's shape depends on the input
+    shapes only, so the call reads nothing back to the host (with ``warn=False``)."""
+    return _infix(ref, hyp, eos, include_eos, norm, batch_first, ins_cost, del_cost, sub_cost, warn,
+                  False)[0]
+
+
+@script
+def infix_matches(
+    ref: torch.Tensor,
+    hyp: torch.Tensor,
+    eos: Optional[int] = None,
+    include_eos: bool = False,
+    batch_first: bool = False,
+    ins_cost: float = config.DEFT_INS_COST,
+    del_cost: float = config.DEFT_DEL_COST,
+    sub_cost: float = config.DEFT_SUB_COST,
+    warn: bool = True,
+) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Where each reference matches inside its hypothesis: ``(dist, start, end)``, fp32 and two
+    int64 ``(N,)``.
+
+    ``dist`` is :func:`infix_edit_distance` (``norm=False``) and the match is
+    ``hyp[start:end]``: :func:`edit_distance` of the reference against it equals ``dist``.
+    ``end`` is the first hypothesis position at which the minimum is reached and ``start`` the
+    latest start of an optimal alignment ending there.  An empty reference gives ``(0, 0, 0)``,
+    an empty hypothesis ``(r * del_cost, 0, 0)``.  Arguments, lengths and warnings are those of
+    :func:`infix_edit_distance`."""
+    return _infix(ref, hyp, eos, include_eos, False, batch_first, ins_cost, del_cost, sub_cost, warn,
+                  True)
 
 
 @script

@@ -21,6 +21,8 @@ __all__ = [
     "ErrorRate",
     "FillAfterEndOfSequence",
     "HardOptimalCompletionDistillationLoss",
+    "InfixEditDistance",
+    "InfixMatches",
     "MinimumBayesRisk",
     "MinimumErrorRateLoss",
     "OptimalCompletion",
@@ -140,6 +142,40 @@ class ErrorCounts(_StringMatching):
     def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
         return F.error_counts(ref, hyp, self.eos, self.include_eos, self.batch_first, self.ins_cost,
                               self.del_cost, self.sub_cost, self.warn)
+
+
+class InfixEditDistance(_StringMatching):
+    """The cheapest match of each reference anywhere inside its hypothesis: fp32 ``(N,)`` (see
+    :func:`b200lev.functional.infix_edit_distance`)"""
+
+    __constants__ = EditDistance.__constants__
+    norm: bool
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, norm: bool = False,
+                 batch_first: bool = False, ins_cost: float = config.DEFT_INS_COST,
+                 del_cost: float = config.DEFT_DEL_COST, sub_cost: float = config.DEFT_SUB_COST,
+                 warn: bool = True):
+        norm = argcheck.is_bool(norm, "norm")
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+        self.norm = norm
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> torch.Tensor:
+        return F.infix_edit_distance(ref, hyp, self.eos, self.include_eos, self.norm, self.batch_first,
+                                     self.ins_cost, self.del_cost, self.sub_cost, self.warn)
+
+
+class InfixMatches(_StringMatching):
+    """Where each reference matches inside its hypothesis: ``(dist, start, end)`` (see
+    :func:`b200lev.functional.infix_matches`)"""
+
+    def __init__(self, eos: Optional[int] = None, include_eos: bool = False, batch_first: bool = False,
+                 ins_cost: float = config.DEFT_INS_COST, del_cost: float = config.DEFT_DEL_COST,
+                 sub_cost: float = config.DEFT_SUB_COST, warn: bool = True):
+        super().__init__(eos, include_eos, batch_first, ins_cost, del_cost, sub_cost, warn)
+
+    def forward(self, ref: torch.Tensor, hyp: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        return F.infix_matches(ref, hyp, self.eos, self.include_eos, self.batch_first, self.ins_cost,
+                               self.del_cost, self.sub_cost, self.warn)
 
 
 class ErrorRate(_StringMatching):

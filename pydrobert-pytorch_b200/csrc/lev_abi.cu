@@ -607,6 +607,49 @@ extern "C" int b200lev_error_alignment(const b200lev_tokens_t* ref, const b200le
                           workspace_bytes, flags, stream);
 }
 
+// b200lev_infix: per pair the minimum of D[i][r] over the rows of the DP whose column 0 is 0 on every
+// row, and with `start` / `end` the match hyp[start:end].  Distance-only calls that the bit-vector
+// route sends to Ks run its infix kind straight from the raw tokens; everything else runs K0 + K1 with
+// the pinned column (and the start channel for spans).
+extern "C" int b200lev_infix(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
+                             const b200lev_opts_t* opts, float* dist, int64_t* start, int64_t* end,
+                             void* workspace, size_t workspace_bytes, int32_t* flags, void* stream) {
+    const bool spans = start != nullptr;
+    if ((start == nullptr) != (end == nullptr)) {
+        lev_set_error("infix: start and end must both be NULL or both be set");
+        return B200LEV_ERR_ARG;
+    }
+    if (opts && opts->ref_group != 1) {
+        lev_set_error("infix: ref_group must be 1, got %d", opts->ref_group);
+        return B200LEV_ERR_ARG;
+    }
+    if (opts && spans && opts->norm) {
+        lev_set_error("infix: norm applies to distances only, not with start and end");
+        return B200LEV_ERR_ARG;
+    }
+    LevCall c;
+    int rc = lev_begin(ref, hyp, opts, B200LEV_WS_FINAL, dist, workspace, workspace_bytes, flags, &c,
+                       [](b200lev_opts_t* o) { o->return_mistakes = 0; });
+    if (rc) return rc == LEV_EMPTY ? B200LEV_OK : rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    LevParams& p = c.p;
+    p.out = dist;
+    p.infix_start = start;
+    p.infix_end = end;
+    const bool short_form =
+        !spans && lev_bitvec_route(ref, hyp, LEV_MODE_FINAL, p, c.count_mode, c.float_path) == LEV_BV_SHORT;
+    if (getenv("B200LEV_TRACE"))
+        fprintf(stderr, "b200lev: infix, %s, R=%lld H=%lld P=%lld %s\n",
+                short_form ? "lev_bv_short_kernel (infix kind)"
+                           : (spans ? "pack + lev_warp_kernel (infix, spans)" : "pack + lev_warp_kernel (infix)"),
+                (long long)c.L.R, (long long)c.L.H, (long long)c.L.P, c.float_path ? "fp32" : "int32");
+    if (short_form)
+        return lev_bitvec_launch(LEV_BV_SHORT, ref, hyp, &c.o, LEV_MODE_INFIX, c.L, c.ws, p, st, nullptr, nullptr);
+    rc = lev_pack_tokens(ref, hyp, &c.o, c.L, c.ws, flags, 0, st);
+    if (rc == B200LEV_OK) rc = lev_launch_infix_dp(p, c.float_path, spans, st);
+    return rc;
+}
+
 extern "C" int b200lev_completion_count(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                                         const b200lev_opts_t* opts, void* workspace,
                                         size_t workspace_bytes, int32_t* umax, int32_t* flags,

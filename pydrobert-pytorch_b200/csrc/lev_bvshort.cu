@@ -52,7 +52,9 @@ __device__ __forceinline__ unsigned lev_bvs_neq16(const unsigned (&half)[16], un
     return acc0 + acc1 * 256u;
 }
 
-template <int W>
+// PH0: the horizontal delta shifted in at column 0 -- 1 where D[i][0] = i, 0 for the infix form
+// (D[i][0] = 0)
+template <int W, unsigned PH0 = 1u>
 __device__ __forceinline__ void lev_bvs_step(const unsigned (&eq)[W], unsigned (&pv)[W],
                                              unsigned (&mv)[W], unsigned (&ph)[W], unsigned (&mh)[W]) {
     unsigned t[W], sum[W];
@@ -67,7 +69,7 @@ __device__ __forceinline__ void lev_bvs_step(const unsigned (&eq)[W], unsigned (
     }
 #pragma unroll
     for (int w = W - 1; w >= 0; --w) {
-        const unsigned phs = w ? __funnelshift_l(ph[w - 1], ph[w], 1) : ((ph[0] << 1) | 1u);
+        const unsigned phs = w ? __funnelshift_l(ph[w - 1], ph[w], 1) : ((ph[0] << 1) | PH0);
         const unsigned mhs = w ? __funnelshift_l(mh[w - 1], mh[w], 1) : (mh[0] << 1);
         const unsigned xv = eq[w] | mv[w];
         pv[w] = mhs | ~(xv | phs);
@@ -75,7 +77,9 @@ __device__ __forceinline__ void lev_bvs_step(const unsigned (&eq)[W], unsigned (
     }
 }
 
-// KIND: 0 = final value, 1 = prefix rows, 2 = prefix rows with exclude_last.
+// KIND: 0 = final value, 1 = prefix rows, 2 = prefix rows with exclude_last, 3 = infix minimum
+// (b200lev_infix: column 0 is 0 on every row, the score at bit r - 1 is tracked as in the prefix
+// kinds and its minimum over the counted rows, row 0 included, is the value).
 // command_line.py:1135-1147: the totals of the bulk-scoring command, folded into the kernel that
 // produced the values (fp64 sums; of integers when the values are counts, so exact in any order);
 // three atomics per CTA.  Kept out of line: inlined, it costs the DP loop above it 18 registers.
@@ -97,7 +101,7 @@ __device__ __forceinline__ void lev_bvs_totals(double sum_out, int sum_len, doub
 // per pair; the lanes of a warp then read at most B distinct hypothesis columns per row.
 template <typename TT, int W, int KIND, bool CROSS>
 __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_short_kernel(const LevBvArgs a) {
-    constexpr bool PREFIX = KIND != 0, EXCL = KIND == 2;
+    constexpr bool PREFIX = KIND == 1 || KIND == 2, EXCL = KIND == 2, INFIX = KIND == 3;
     constexpr int CH = 4;
     const int lane = threadIdx.x & 31;
     const int64_t nblocks = ((int64_t)a.P + 31) / 32;
@@ -109,7 +113,7 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
     // thread), not in registers carried through the DP loop
     __shared__ double sums[LEV_BVS_WARPS * 32];
     __shared__ int lens[LEV_BVS_WARPS * 32];
-    if (!PREFIX) {
+    if (KIND == 0) {
         sums[threadIdx.x] = 0.0;
         lens[threadIdx.x] = 0;
     }
@@ -211,7 +215,7 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
         const int top = rlen > 0 ? rlen - 1 : 0;
         const int top_sh = top & 31;
         const bool top_hi = W > 1 && top >= 32;
-        const unsigned empty_up = rlen == 0 ? 1u : 0u;
+        const unsigned empty_up = (!INFIX && rlen == 0) ? 1u : 0u;
 
         unsigned pv[W], mv[W];
 #pragma unroll
@@ -220,6 +224,8 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
             mv[w] = 0u;
         }
         float scoref = (float)rlen;
+        float smin = scoref;  // INFIX: the minimum over the counted rows
+        int eos_seen = 0;     // INFIX: an eos among the hypothesis tokens (rows past H clear live_m too)
         int live_m = -1, prev_m = -1, nin = 0;
         float prev_val = PREFIX ? value_of(scoref, 0.0f) : 0.0f;
         float* __restrict__ orow = a.out + pc;
@@ -250,6 +256,7 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
             if (sizeof(TT) == 8) e |= hi ^ eos_hi;
             const int eos_m = e == 0 ? haseos_m : 0;
             const int has_tok = t < H ? -1 : 0;  // (warp-uniform)
+            if (INFIX) eos_seen |= eos_m & has_tok;
             const int in_m = live_m & (incl_m | ~eos_m) & has_tok;
             live_m &= ~eos_m & has_tok;
             nin -= in_m;
@@ -289,13 +296,14 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
                         if ((int64_t)rsrc[(int64_t)(32 * w + jj) * rst] == x) eq[w] |= 1u << jj;
             }
             unsigned ph[W], mh[W];
-            if (PREFIX) {
-                lev_bvs_step<W>(eq, pv, mv, ph, mh);
+            if (PREFIX || INFIX) {
+                lev_bvs_step<W, INFIX ? 0u : 1u>(eq, pv, mv, ph, mh);
                 const unsigned up = (((top_hi ? ph[W - 1] : ph[0]) >> top_sh) & 1u) | empty_up;
                 const unsigned down = ((top_hi ? mh[W - 1] : mh[0]) >> top_sh) & 1u & ~empty_up;
                 scoref += __int_as_float((int)(up * 0x3f800000u));
                 scoref -= __int_as_float((int)(down * 0x3f800000u));
-                prev_val = value_of(scoref, bias);
+                if (PREFIX) prev_val = value_of(scoref, bias);
+                if (INFIX) smin = (in_m != 0 && scoref < smin) ? scoref : smin;
             } else {
                 // FINAL: no score is carried.  The column state (the vertical deltas) freezes at the
                 // lane's last counted token, and D[r][h] = h + #(+1 deltas) - #(-1 deltas) among the
@@ -407,8 +415,9 @@ __global__ void __launch_bounds__(32 * LEV_BVS_WARPS, W == 1 ? 5 : 4) lev_bv_sho
             }
         }
         const int hlen = nin;
-        if (a.has_eos && a.include_eos && live_m != 0) myflags |= B200LEV_FLAG_HYP_NO_EOS;
-        if (!PREFIX) {  // SM:390-405
+        if (a.has_eos && a.include_eos && (INFIX ? eos_seen == 0 : live_m != 0)) myflags |= B200LEV_FLAG_HYP_NO_EOS;
+        if (INFIX) a.out[pc] = value_of(rlen > 0 ? smin : 0.0f, 0.0f);  // (an empty reference: 0)
+        if (KIND == 0) {  // SM:390-405
             int score = hlen;
 #pragma unroll
             for (int w = 0; w < W; ++w) {
@@ -455,6 +464,8 @@ static void lev_bvs_launch_w(const LevBvArgs& a, cudaStream_t st) {
     const dim3 grid((unsigned)(n < cap ? n : cap)), block(32 * LEV_BVS_WARPS);
     if (a.cross_b > 0)  // (final mode only)
         lev_launch(lev_bv_short_kernel<TT, W, 0, true>, grid, block, 0, st, a);
+    else if (a.mode == LEV_MODE_INFIX)
+        lev_launch(lev_bv_short_kernel<TT, W, 3, false>, grid, block, 0, st, a);
     else if (a.mode != LEV_MODE_PREFIX)
         lev_launch(lev_bv_short_kernel<TT, W, 0, false>, grid, block, 0, st, a);
     else if (!a.exclude_last)

@@ -6,7 +6,8 @@
 
 #include "../../include/b200lev.h"
 
-enum LevMode { LEV_MODE_FINAL = 0, LEV_MODE_PREFIX = 1, LEV_MODE_MASK = 2 };
+// INFIX: b200lev_infix's distance-only form on the short bit-vector kernel (lev_bvshort.cu)
+enum LevMode { LEV_MODE_FINAL = 0, LEV_MODE_PREFIX = 1, LEV_MODE_MASK = 2, LEV_MODE_INFIX = 3 };
 
 // "Infinity" for the int32 DP: virtual columns left of column 0 hold it so that
 // column 0 needs no special case.  Costs are bounded on the host so that BIG plus
@@ -202,6 +203,9 @@ struct LevParams {
     int ops_steps;
     // b200lev_error_counts: (C, S, D, I) of pair n at counts[4n .. 4n+3]
     int64_t* counts;
+    // b200lev_infix with spans: the start and end rows of pair n's match
+    int64_t* infix_start;
+    int64_t* infix_end;
 };
 
 
@@ -262,6 +266,9 @@ int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st);
 int lev_counts_short_launch(const b200lev_tokens_t* ref, const b200lev_tokens_t* hyp,
                             const b200lev_opts_t* o, const LevParams& p, bool float_path,
                             cudaStream_t st);
+// b200lev_infix (p.out the distances; p.infix_start / p.infix_end with `spans`): K1 with column 0
+// pinned to 0, after K0 (lev_dp.cu)
+int lev_launch_infix_dp(const LevParams& p, bool float_path, bool spans, cudaStream_t st);
 // lanes per pair if the shapes admit the group kernel (its histogram is then built at
 // pack time), else 0
 int lev_group_eligible(int64_t R, int64_t H, int64_t P);

@@ -32,11 +32,13 @@
 #include "lev_align.cuh"
 
 // number of per-warp shared-memory columns (boundary channels + row minima)
-template <typename V, bool COUNT, int MODE, bool OPS = false>
+template <typename V, bool COUNT, int MODE, bool OPS = false, bool SPAN = false>
 struct LevBufs {
     static constexpr bool FLT_COST = !std::is_same<V, int>::value && !COUNT;
-    // MASK: + row minima + the chained bitmap word handed from strip to strip; OPS: + insertions
-    static constexpr int NB = (COUNT ? 2 : (FLT_COST ? 3 : 1)) + (MODE == LEV_MODE_MASK ? 2 : 0) + (OPS ? 1 : 0);
+    // MASK: + row minima + the chained bitmap word handed from strip to strip; OPS: + insertions;
+    // SPAN: + start rows of the cells (and, fp32, of the run origins)
+    static constexpr int NB = (COUNT ? 2 : (FLT_COST ? 3 : 1)) + (MODE == LEV_MODE_MASK ? 2 : 0) + (OPS ? 1 : 0) +
+                              (SPAN ? (FLT_COST ? 2 : 1) : 0);
 };
 
 // One pair on one warp.  PASS: 0 = the only pass (FINAL/PREFIX) or the row-minimum
@@ -51,6 +53,13 @@ struct LevBufs {
 // TRACE (on top of OPS; b200lev_error_alignment, C = 8 or 4): every row's C choices of a lane as
 // one uint16 / byte of 2-bit op codes (lev_align.cuh) into the pair's trace, and the epilogue
 // writes the insertion count alone.
+// INFIX (FINAL, cost cell; b200lev_infix): column 0 holds 0 on every row, so a path may leave it at
+// any row; the owner of column r keeps the minimum of D[i][r] over the rows (row 0 included) and the
+// first row reaching it, and the epilogue writes that minimum instead of D[h][r].
+// SPAN (on top of INFIX): one more int32 channel, the start row of each cell's path (row i for column
+// 0 of row i), carried like the insertions of OPS; among the predecessors that reach a cell's value
+// exactly (diagonal, up, deletion run origin) the largest start wins.  The epilogue writes the start
+// and end rows of the match.
 // tokens that do not fit in int32 (B200LEV_FLAG_WIDE_TOKENS): read the caller's tensors
 // directly and compare in 64 bits.  Slow (strided gathers) but exact; uniform per launch.
 __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes, int64_t idx) {
@@ -62,7 +71,14 @@ __device__ __forceinline__ int64_t lev_load_raw(const void* base, int elem_bytes
     }
 }
 
-template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE, bool OPS, bool TRACE = false>
+// the start of a cell whose value min(a, b) comes from candidates with starts sa, sb (SPAN)
+template <typename V>
+__device__ __forceinline__ int lev_span_pick(V a, int sa, V b, int sb) {
+    return a < b ? sa : (b < a ? sb : (sa > sb ? sa : sb));
+}
+
+template <typename V, bool COUNT, int MODE, int C, int PASS, bool WIDE, bool OPS, bool TRACE = false,
+          bool INFIX = false, bool SPAN = false>
 __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair, const int r,
                                               const int h, const int steps,
                                               const int* __restrict__ hyp_s_,
@@ -89,7 +105,13 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
     V* __restrict__ rowmin = bufs + (LevBufs<V, COUNT, MODE>::NB - 2) * Hs;  // MASK only
     unsigned* __restrict__ bitcol = reinterpret_cast<unsigned*>(bufs + (LevBufs<V, COUNT, MODE>::NB - 1) * Hs);
     int* __restrict__ bnd_i = reinterpret_cast<int*>(bufs + 2 * Hs);  // OPS: insertions
-    (void)bnd_a; (void)bnd_b; (void)rowmin; (void)bitcol; (void)bnd_i;
+    int* __restrict__ bnd_s = reinterpret_cast<int*>(bufs + (FLT_COST ? 3 : 1) * Hs);  // SPAN: starts
+    int* __restrict__ bnd_os = reinterpret_cast<int*>(bufs + 4 * Hs);  // SPAN, fp32: run-origin starts
+    (void)bnd_a; (void)bnd_b; (void)rowmin; (void)bitcol; (void)bnd_i; (void)bnd_s; (void)bnd_os;
+    // INFIX: the minimum over the rows of column r, the first row reaching it and (SPAN) its start
+    V best = (V)0;
+    int best_end = 0, best_start = 0;
+    (void)best; (void)best_end; (void)best_start;
 
     for (int k = 0; k < S; ++k) {
         const bool first = (k == 0), last = (k == S - 1);
@@ -98,6 +120,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
         V v[C];
         V m[C];     // COUNT: mistake counts
         int ic[C];  // OPS: insertions
+        int sc[C];  // SPAN: start rows
         V jd[C];    // FLT_COST: fl(j * del), SM:258-263
         Tok rt[C];  // reference token of column j (ref position j-1)
         int ud[C];  // EQ: distinct-token rank of ref position j, or -1
@@ -107,6 +130,7 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
             v[c] = (j >= 0) ? (V)j * delc : BIG;
             m[c] = (V)(j >= 0 ? j : 0);  // SM:260
             ic[c] = 0;                   // row 0: deletions only
+            sc[c] = 0;
             jd[c] = (j >= 0) ? (V)j * delc : (V)0;
             if (WIDE)
                 rt[c] = (j >= 1) ? (Tok)lev_load_raw(p.ref_raw, p.ref_eb,
@@ -119,18 +143,22 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
             // EQC: the bit of this column's token (ranks < 32), 0 for columns that are no target
             if (EQC) ud[c] = (j >= 0 && j < r) ? (int)(1u << (p.uid[(int64_t)refcol * p.Rp + j] & 31)) : 0;
         }
-        (void)m; (void)jd; (void)ud; (void)ic;
+        (void)m; (void)jd; (void)ud; (void)ic; (void)sc;
+        if (INFIX && last) best = v[C - 1];  // D[0][r] (lane 31)
+        const int zc = -j0;  // INFIX: this lane's column c that is column 0, if any
+        (void)zc;
         unsigned bitrun = 0u;  // EQC chain register
         (void)bitrun;
         // chain registers: what this lane publishes to lane+1 at the next step
         V ob = BIG, oj = (V)0, rmrun = BIG;
-        (void)ob; (void)oj; (void)rmrun;
+        int os = 0;  // SPAN, fp32: start of the run origin
+        (void)ob; (void)oj; (void)rmrun; (void)os;
         // previous step's hand-in (the diagonal); lane 0 starts from row 0 of the
         // boundary column, the other lanes pick it up from the shuffle at step l
         V pl_v = first ? BIG : (V)jb * delc;
         V pl_m = (V)(first ? 0 : jb);
-        int pl_i = 0;
-        (void)pl_m; (void)pl_i;
+        int pl_i = 0, pl_s = 0;
+        (void)pl_m; (void)pl_i; (void)pl_s;
         if (steps > 0) {
             const int nsteps = steps + 31;
             for (int s = 1; s <= nsteps; ++s) {
@@ -154,6 +182,18 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                     pl_i = in_i;
                 }
                 (void)in_i; (void)diag_i;
+                int in_s = 0, diag_s = 0, in_os = 0;
+                if constexpr (SPAN) {
+                    const int sh_s = __shfl_up_sync(LEV_FULL_MASK, sc[C - 1], 1);
+                    in_s = (lane == 0) ? (first ? 0 : bnd_s[32 + s]) : sh_s;
+                    diag_s = pl_s;
+                    pl_s = in_s;
+                    if (FLT_COST) {
+                        const int sh_os = __shfl_up_sync(LEV_FULL_MASK, os, 1);
+                        in_os = (lane == 0) ? (first ? 0 : bnd_os[32 + s]) : sh_os;
+                    }
+                }
+                (void)in_s; (void)diag_s; (void)in_os;
                 if (FLT_COST) {
                     const V sh_ob = __shfl_up_sync(LEV_FULL_MASK, ob, 1);
                     const V sh_oj = __shfl_up_sync(LEV_FULL_MASK, oj, 1);
@@ -222,6 +262,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         // SM:290-293,316-317 in fp32, deletion term by run origin:
                         // new[j] = min(t[j], t[k*] + (fl(j*d) - fl(k* * d)))
                         V dg = diag_v, obr = in_ob, ojr = in_oj;
+                        int sdg = diag_s, sob = in_os;
+                        (void)sdg; (void)sob;
 #pragma unroll
                         for (int c = 0; c < C; ++c) {
                             const V up = v[c];
@@ -233,10 +275,23 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                             v[c] = fresh ? t : cand;
                             obr = fresh ? t : obr;
                             ojr = fresh ? jd[c] : ojr;
+                            if constexpr (SPAN) {
+                                const int ns = lev_span_pick(cand, sob, t, lev_span_pick(a, sc[c], sb, sdg));
+                                sdg = sc[c];
+                                sc[c] = ns;
+                                sob = fresh ? ns : sob;
+                            }
+                            if (INFIX && c == zc) {  // column 0: a match may start at this row
+                                v[c] = (V)0;
+                                obr = (V)0;
+                                ojr = jd[c];
+                                if (SPAN) sc[c] = sob = i;
+                            }
                             dg = up;
                         }
                         ob = obr;
                         oj = ojr;
+                        os = sob;
                     } else {
                         // integer costs: 4 INT32 instructions per cell
                         int dg = (int)diag_v, lf = (int)in_v;
@@ -245,13 +300,28 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         // keep the compare)
                         const unsigned nht = 0u - (unsigned)ht;
                         (void)nht;
+                        int sdg = diag_s, slf = in_s;
+                        (void)sdg; (void)slf;
 #pragma unroll
                         for (int c = 0; c < C; ++c) {
                             const int up = (int)v[c];
                             const int sb = WIDE ? dg + ((rt[c] != ht) ? (int)subc : 0)
                                                 : dg + (int)(__viaddmin_u32((unsigned)rt[c], nht, 1u) * (unsigned)subc);
                             const int t = __viaddmin_s32(up, (int)insc, sb);
-                            lf = __viaddmin_s32(lf, (int)delc, t);
+                            if constexpr (SPAN) {
+                                const int st = lev_span_pick(up + (int)insc, sc[c], sb, sdg);
+                                const int l = lf + (int)delc;
+                                slf = lev_span_pick(l, slf, t, st);
+                                sdg = sc[c];
+                                lf = l < t ? l : t;
+                            } else {
+                                lf = __viaddmin_s32(lf, (int)delc, t);
+                            }
+                            if (INFIX && c == zc) {  // column 0: a match may start at this row
+                                lf = 0;
+                                if (SPAN) slf = i;
+                            }
+                            if (SPAN) sc[c] = slf;
                             dg = up;
                             v[c] = (V)lf;
                         }
@@ -292,6 +362,8 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                             bnd_v[32 + i] = v[C - 1];
                             if (COUNT) bnd_a[32 + i] = m[C - 1];
                             if (OPS) bnd_i[32 + i] = ic[C - 1];
+                            if (SPAN) bnd_s[32 + i] = sc[C - 1];
+                            if (SPAN && FLT_COST) bnd_os[32 + i] = os;
                             if (FLT_COST) {
                                 bnd_a[32 + i] = ob;
                                 bnd_b[32 + i] = oj;
@@ -299,6 +371,10 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                         } else if (MODE == LEV_MODE_PREFIX) {  // SM:340-346
                             p.out[(int64_t)i * p.out_si + (int64_t)pair * p.out_sn] =
                                 lev_finalize((float)(COUNT ? m[C - 1] : v[C - 1]), p, r, true);
+                        } else if (INFIX && v[C - 1] < best) {  // the first row reaching the minimum
+                            best = v[C - 1];
+                            best_end = i;
+                            if (SPAN) best_start = sc[C - 1];
                         }
                         if (RMIN) rowmin[32 + i] = rmrun;
                     }
@@ -317,6 +393,12 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
                 o[2] = del;
                 o[3] = ins;
             }
+        } else if (INFIX && last && lane == 31) {  // an empty reference matches the empty stretch: 0
+            p.out[pair] = lev_finalize((float)best, p, r, false);
+            if (SPAN) {
+                p.infix_start[pair] = best_start;
+                p.infix_end[pair] = best_end;
+            }
         } else if (MODE == LEV_MODE_FINAL && last && lane == 31) {  // SM:390-405
             p.out[pair] = lev_finalize((float)(COUNT ? m[C - 1] : v[C - 1]), p, r, h > 0);
         }
@@ -327,11 +409,12 @@ __device__ __forceinline__ int lev_warp_pair(const LevParams& p, const int pair,
 
 // Returns -1 when the largest target set still has to be counted from the bitmaps in global
 // memory (atomic pass), else that size as lane 31 saw it (chained pass).
-template <typename V, bool COUNT, int MODE, int C, bool WIDE = false, bool OPS = false, bool TRACE = false>
+template <typename V, bool COUNT, int MODE, int C, bool WIDE = false, bool OPS = false, bool TRACE = false,
+          bool INFIX = false, bool SPAN = false>
 __device__ __forceinline__ int lev_warp_pair_all(const LevParams& p, int pair, int r, int h,
                                                  int steps, const int* hyp_s, V* bufs, int Hs,
                                                  bool one_word) {
-    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs);
+    lev_warp_pair<V, COUNT, MODE, C, 0, WIDE, OPS, TRACE, INFIX, SPAN>(p, pair, r, h, steps, hyp_s, bufs, Hs);
     if (MODE == LEV_MODE_MASK) {
         if (one_word) return lev_warp_pair<V, COUNT, MODE, C, 2, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
         lev_warp_pair<V, COUNT, MODE, C, 1, WIDE, false>(p, pair, r, h, steps, hyp_s, bufs, Hs);
@@ -342,8 +425,10 @@ __device__ __forceinline__ int lev_warp_pair_all(const LevParams& p, int pair, i
 // CMASK: bit c set => the kernel carries a C = 2^c variant (1, 2, 4, 8); each pair
 // takes the smallest variant whose single strip covers its r + 1 columns, the largest
 // one (multi-strip) otherwise.  OPS: the error-counts epilogue (FINAL, COUNT).  TRACE: the
-// error-alignment trace (with OPS; one C only, CMASK 8 or 4).
-template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false>
+// error-alignment trace (with OPS; one C only, CMASK 8 or 4).  INFIX / SPAN: b200lev_infix (FINAL,
+// cost cell).
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false, bool INFIX = false,
+          bool SPAN = false>
 __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     LEV_DYN_SMEM(int, smem);
     const int lane = threadIdx.x & 31;
@@ -351,7 +436,7 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     const int wpc = blockDim.x >> 5;
     // (even: every warp's slice starts 8-byte aligned, the 64-bit-token path stores int64)
     const int Hs = (p.H + 65) & ~1;
-    constexpr int NB = LevBufs<V, COUNT, MODE, OPS>::NB;
+    constexpr int NB = LevBufs<V, COUNT, MODE, OPS, SPAN>::NB;
     int* hyp_s = smem + (size_t)warp * (2 + NB) * Hs;  // 2*Hs ints: room for int64 tokens
     V* bufs = reinterpret_cast<V*>(hyp_s + 2 * Hs);
     const bool wide = (*p.wide_flag & B200LEV_FLAG_WIDE_TOKENS) != 0;
@@ -379,16 +464,16 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
         const bool one_word = MODE == LEV_MODE_MASK && p.ndist[pair / p.ref_group] <= 32;
         int set_max = -1;
         if (wide)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true, OPS, TRACE>(
+            set_max = lev_warp_pair_all<V, COUNT, MODE, (CMASK & 8) ? 8 : ((CMASK & 4) ? 4 : ((CMASK & 2) ? 2 : 1)), true, OPS, TRACE, INFIX, SPAN>(
                 p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 1) && (cols <= 32 || !(CMASK & 14)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 1, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 1, false, OPS, TRACE, INFIX, SPAN>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 2) && (cols <= 64 || !(CMASK & 12)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 2, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 2, false, OPS, TRACE, INFIX, SPAN>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if ((CMASK & 4) && (cols <= 128 || !(CMASK & 8)))
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 4, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 4, false, OPS, TRACE, INFIX, SPAN>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
         else if (CMASK & 8)
-            set_max = lev_warp_pair_all<V, COUNT, MODE, 8, false, OPS, TRACE>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
+            set_max = lev_warp_pair_all<V, COUNT, MODE, 8, false, OPS, TRACE, INFIX, SPAN>(p, pair, r, h, steps, hyp_s, bufs, Hs, one_word);
 
         if (MODE == LEV_MODE_PREFIX) {
             // SM:279-285 (row 0) and SM:379-386 (tail := padding)
@@ -432,9 +517,10 @@ __global__ void __launch_bounds__(256) lev_warp_kernel(const LevParams p) {
     }
 }
 
-template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false>
+template <typename V, bool COUNT, int MODE, int CMASK, bool OPS = false, bool TRACE = false, bool INFIX = false,
+          bool SPAN = false>
 static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
-    constexpr int NB = LevBufs<V, COUNT, MODE, OPS>::NB;
+    constexpr int NB = LevBufs<V, COUNT, MODE, OPS, SPAN>::NB;
     const size_t per_warp = (size_t)(2 + NB) * (size_t)((p.H + 65) & ~1) * sizeof(int);
     const size_t budget = 200 * 1024;
     if (per_warp > budget) {
@@ -447,7 +533,7 @@ static int lev_launch_variant(const LevParams& p, cudaStream_t st) {
     // keep at least two CTAs per SM resident when the rows are short
     while (wpc > 1 && per_warp * wpc > 100 * 1024) --wpc;
     const size_t smem = per_warp * wpc;
-    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK, OPS, TRACE>;
+    auto kern = lev_warp_kernel<V, COUNT, MODE, CMASK, OPS, TRACE, INFIX, SPAN>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)smem);
@@ -540,6 +626,18 @@ int lev_launch_counts_dp(const LevParams& p, bool float_path, cudaStream_t st) {
     }
     if (!float_path) return lev_launch_variant<int, true, LEV_MODE_FINAL, 10, true>(p, st);
     return lev_launch_variant<float, true, LEV_MODE_FINAL, 4, true>(p, st);
+}
+
+// b200lev_infix, everything but the distance-only calls Ks serves: K1 with column 0 pinned to 0 and
+// the minimum over the rows of column r, after K0; `spans` adds the start channel.  No group, CTA or
+// bit-vector kernel: none of them has the pinned column.
+int lev_launch_infix_dp(const LevParams& p, bool float_path, bool spans, cudaStream_t st) {
+    if (p.P <= 0) return B200LEV_OK;
+    if (!float_path)
+        return spans ? lev_launch_variant<int, false, LEV_MODE_FINAL, 15, false, false, true, true>(p, st)
+                     : lev_launch_variant<int, false, LEV_MODE_FINAL, 15, false, false, true, false>(p, st);
+    return spans ? lev_launch_variant<float, false, LEV_MODE_FINAL, 4, false, false, true, true>(p, st)
+                 : lev_launch_variant<float, false, LEV_MODE_FINAL, 4, false, false, true, false>(p, st);
 }
 
 // the short form (R <= 64): one lane per pair from the raw tokens
